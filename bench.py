@@ -2,6 +2,7 @@
 """Benchmark of the fused trajectory rollout (BASELINE.json metric: particle-steps/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision f16x3|tf32x3|fp32|tf32|bf16]
+                    [--dump-outputs DIR]
 
 The headline number is measured in the fp32-grade mode f16x3 (drift network, mixture logits AND mixture-score
 contractions on tcgen05 tensor cores with the 3-pass fp16 (hi, lo) split of power-of-two scaled operands; parity-tested to
@@ -260,6 +261,10 @@ def run_ours(args):
     kern_ms_each = [round(a.elapsed_time(b), 3) for a, b, _ in ev]
     ms_per_step = max_over_ranks(step_ms) / args.steps
     value = world * B * K_STEPS / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path receives from its last step: x_T [B, 50] and rnd [B, 1] in float32 (13.4 MB),
+        # the 8 merged estimator partials in float64
+        dump_outputs(args.dump_outputs, {"x_T": x, "rnd": rnd, "estimator_partials": last})
 
     # ---- reduced-precision fast mode, reported separately ------------------------------------------------------
     fast = None
@@ -382,6 +387,15 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as <out_dir>/<name>.npy in the dtype it was computed in, so that two builds of the project run
+    with the same arguments (hence the same seeded inputs) can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy())
+
+
 def other_workloads(dev, precision, flush):
     """Device-resident kernel time of the other BASELINE.json shapes (production mode, in-kernel noise): 2 warm-ups,
     3 timed launches each with the L2 flushed in between; tensor-roof fraction from BASELINE.md's FLOP counts."""
@@ -466,7 +480,13 @@ def main():
     ap.add_argument("--no-fast-mode", action="store_true", help=argparse.SUPPRESS)  # accepted for older command lines
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-workloads", action="store_true", help="skip the other BASELINE shapes (single-GPU runs time them too)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's x_T, rnd and estimator partials (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -6,7 +6,8 @@ tmp=$(mktemp -d)
 ncu -i $rep --page raw --csv > $tmp/raw.csv 2>/dev/null
 ncu -i $rep --page source --csv > $tmp/src.csv 2>/dev/null
 python tools/ncu_summary.py $tmp/raw.csv "$(basename $rep)"
-(cd $tmp && cuobjdump -xelf all /root/repo/sde_sampler_lrds_b200/csrc/liblrds_b200.so >/dev/null 2>&1)
+lib=$(cd "$(dirname "$0")/.." && pwd)/sde_sampler_lrds_b200/csrc/liblrds_b200.so
+(cd $tmp && cuobjdump -xelf all "$lib" >/dev/null 2>&1)
 echo
 echo '```'
 python tools/ncu_by_line.py $tmp/src.csv $tmp/$unit.sm_100a.cubin "$kname" $top

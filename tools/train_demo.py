@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """End-to-end training through the fused rollout: make_model(...) over TwoModes d=2, 200 Adam steps (batch 512, lr 3e-3,
 K=50) per solver, evaluation log-variance / ELBO before and after, wall time per step:   python tools/train_demo.py"""
-import sys, math, time; sys.path.insert(0, "/root/repo")
+import os, sys, math, time; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from sde_sampler_lrds_b200 import benchmark_utils as BU
 
