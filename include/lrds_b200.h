@@ -17,7 +17,7 @@
 extern "C" {
 #endif
 
-#define LRDS_ABI_VERSION 8
+#define LRDS_ABI_VERSION 9 /* 9: lrds_gmm.layout (full-covariance Gaussian / mixture references) */
 #define LRDS_CHANNELS 64 /* FourierMLP / TimeEmbed width, conf/model/base/fouriermlp.yaml:4 */
 #define LRDS_MAX_DIM_PAD 1024 /* largest d_pad the operand packers accept */
 
@@ -65,7 +65,7 @@ typedef enum {
 
 typedef enum {
   LRDS_DISTR_NONE = 0,
-  LRDS_DISTR_GMM = 1,   /* diagonal Gaussian / mixture: distr/gauss.py:67-73, 97-107, 124-126, 202-221 */
+  LRDS_DISTR_GMM = 1,   /* Gaussian / mixture, diagonal (distr/gauss.py:67-73, 97-107, 124-126, 202-221) or full (gmm.layout) */
   LRDS_DISTR_PHI4 = 2,  /* PhiFour U / grad_U, distr/phi_four.py:45-96 (dim_phys=1, Dirichlet-0) */
   LRDS_DISTR_LOGREG = 3 /* LogisticRegression.posterior_log_prob + its autograd score, distr/logistic_regression.py:41-61 */
 } lrds_distr_kind;
@@ -120,12 +120,24 @@ typedef struct {
   const void* tc_image; /* weight image written by lrds_pack_mlp_tc for spec.precision (tensor-core precisions only) */
 } lrds_mlp;
 
-/* Diagonal Gaussian mixture with M >= 1 components.  `step_stride_*` = 0 for a static distribution; for the
+/* Storage layout of a lrds_gmm block. */
+typedef enum {
+  LRDS_GMM_DIAG = 0, /* diagonal covariances: logc, mu, ivar, sn (and optionally mix_tc) as described below */
+  LRDS_GMM_FULL = 1  /* full covariances (eq/sdes.py:232-239, distr/gauss.py:76-121): logc and mu as below, and
+                      * sn = the precision matrices [M][d_pad][d_pad] (row-major, zero in the padded rows and columns,
+                      * step_stride_sn = M d_pad^2 for a per-step block); ivar and mix_tc are unused (NULL).
+                      * logc_m = log w_m - d/2 log(2 pi) - 1/2 log det(Sigma_m).  Accepted as spec.ref_t / spec.ref_0 of
+                      * the LINEAR and EUBO_LINEAR kinds and by lrds_distr_eval; LRDS_ERR_UNSUPPORTED everywhere else
+                      * (targets, CMCD / DIS priors, lrds_mala, lrds_score_cot_sums). */
+} lrds_gmm_layout;
+
+/* Gaussian mixture with M >= 1 components.  `step_stride_*` = 0 for a static distribution; for the
  * time-marginal reference p_t^ref (eq/sdes.py:208-248, 281-345) the arrays hold one block per step and the
- * strides are the element distance between consecutive steps. */
+ * strides are the element distance between consecutive steps.  The fields below describe the diagonal layout
+ * (layout = LRDS_GMM_DIAG); see lrds_gmm_layout for the full one. */
 typedef struct {
   int32_t M;
-  int32_t reserved;
+  int32_t layout; /* lrds_gmm_layout; 0 (a zero-initialised block) = diagonal */
   const float* logc; /* [4 ceil(M/4)]  log w_m - d/2 log(2 pi) - 1/2 sum_j log var_mj (w normalised); padding = -inf; 16-byte aligned */
   const float* mu;   /* [M][d_pad]  rows padded with 0 to d_pad = 8 ceil(d / 8) floats, 16-byte aligned */
   const float* ivar; /* [M][d_pad]  1 / var, padded with 0 */

@@ -19,7 +19,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.environ.get("LRDS_B200_LIB") or os.path.join(CSRC, "liblrds_b200.so")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 
-ABI_VERSION = 8
+ABI_VERSION = 9
 CHANNELS = 64
 STEP_STRIDE = 80
 (STEP_A, STEP_B, STEP_C, STEP_DT, STEP_SQRT_DT, STEP_W_COST, STEP_W_ITO, STEP_GAMMA, STEP_FRAC, STEP_SIGU,
@@ -31,6 +31,7 @@ UPDATE_AXPY, UPDATE_EM = range(2)
 ITO_NONE, ITO_SCALED, ITO_EM, ITO_DDS = range(4)
 CTRL_CLIPPED, CTRL_SCORE, CTRL_CANCEL_DRIFT, CTRL_LERP = range(4)
 DISTR_NONE, DISTR_GMM, DISTR_PHI4, DISTR_LOGREG = range(4)
+GMM_DIAG, GMM_FULL = range(2)
 MCMC_MALA, MCMC_RWMH = 0, 1
 PRECISION_FP32_SIMT, PRECISION_TF32X3, PRECISION_BF16, PRECISION_TF32, PRECISION_F16X3 = range(5)
 PRECISIONS = {"fp32": PRECISION_FP32_SIMT, "tf32x3": PRECISION_TF32X3, "bf16": PRECISION_BF16, "tf32": PRECISION_TF32,
@@ -45,7 +46,7 @@ class Mlp(C.Structure):
 
 
 class Gmm(C.Structure):
-    _fields_ = [("M", C.c_int32), ("reserved", C.c_int32), ("logc", FP), ("mu", FP), ("ivar", FP), ("sn", FP),
+    _fields_ = [("M", C.c_int32), ("layout", C.c_int32), ("logc", FP), ("mu", FP), ("ivar", FP), ("sn", FP),
                 ("step_stride_logc", C.c_int64), ("step_stride_param", C.c_int64), ("step_stride_sn", C.c_int64),
                 ("mix_tc", FP), ("step_stride_mix_tc", C.c_int64)]
 

@@ -198,11 +198,12 @@ def mcmc_sample(device, target, x_init, mcmc_type="mala", step_size=1e-3, n_chai
 def fit_gmm(n_components, dataset, means_init=None, em_type="diag", max_iter=1000):
     """experiments/benchmark_utils.py:336-365: sklearn's EM over the MCMC data set (host library code in the reference
     as well), tried over the reference's ladder of ``reg_covar`` values.  Returns (weights, means, variances) as the
-    ``*_ref`` entries of ``solver_details``; only diagonal covariances feed a kernel (full ones: SURVEY.md 8f item 2)."""
+    ``*_ref`` entries of ``solver_details``: variances [M][d] for em_type='diag', covariance matrices [M][d][d] for
+    em_type='full' (the full-covariance reference, GMMFull)."""
     from sklearn.mixture import GaussianMixture
-    if em_type != "diag":
-        raise NotImplementedError("full-covariance references have no kernel (SURVEY.md 8f item 2)")
-    from .distr.gauss import GMM
+    if em_type not in ("diag", "full"):
+        raise NotImplementedError(f"em_type {em_type!r}: the references are built for 'diag' and 'full' covariances")
+    from .distr.gauss import GMM, GMMFull
     for reg_covar in [1e-6, 5e-5, 1e-5, 5e-4, 1e-4, 5e-3, 1e-3, 5e-2, 1e-2]:
         try:
             dim = dataset.shape[-1]
@@ -213,7 +214,10 @@ def fit_gmm(n_components, dataset, means_init=None, em_type="diag", max_iter=100
             weights = torch.from_numpy(gmm.weights_).float()
             means = torch.from_numpy(gmm.means_).float()
             variances = torch.from_numpy(gmm.covariances_).float()
-            GMM(dim=dim, loc=means, scale=variances.sqrt(), mixture_weights=weights)
+            if em_type == "full":
+                GMMFull(dim=dim, loc=means, covariance_matrix=variances, mixture_weights=weights)
+            else:
+                GMM(dim=dim, loc=means, scale=variances.sqrt(), mixture_weights=weights)
             return weights, means, variances
         except Exception:  # noqa: BLE001  (the reference retries on any failure with the next regularisation)
             continue

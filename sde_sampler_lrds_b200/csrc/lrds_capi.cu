@@ -44,7 +44,19 @@ int pick_threads(int floats_per_particle, int smem_cap) {
 }
 
 int validate_gmm(const lrds_gmm& g, const char* name) {
+  if (g.layout == LRDS_GMM_FULL) {  // logc, mu, sn = precision matrices; no ivar / tensor-core image
+    if (g.M < 1 || !g.logc || !g.mu || !g.sn) return fail(LRDS_ERR_INVALID, "%s: incomplete full-covariance block", name);
+    if (g.mix_tc) return fail(LRDS_ERR_INVALID, "%s: a full-covariance block has no mix_tc image", name);
+    return LRDS_OK;
+  }
+  if (g.layout != LRDS_GMM_DIAG) return fail(LRDS_ERR_INVALID, "%s: unknown lrds_gmm layout", name);
   if (g.M < 1 || !g.logc || !g.mu || !g.ivar || !g.sn) return fail(LRDS_ERR_INVALID, "%s: incomplete mixture block", name);
+  return LRDS_OK;
+}
+// the entry points that evaluate only diagonal blocks
+int refuse_full(const lrds_gmm& g, const char* where) {
+  if (g.layout == LRDS_GMM_FULL) return fail(LRDS_ERR_UNSUPPORTED, "%s: full-covariance blocks are built for the LINEAR / EUBO_LINEAR "
+                                             "reference (ref_t, ref_0) and lrds_distr_eval only", where);
   return LRDS_OK;
 }
 
@@ -58,11 +70,12 @@ int validate_spec(const lrds_spec* s, bool need_steps) {
     return fail(LRDS_ERR_INVALID, "mlp weight pointers missing");
   if (need_steps && !s->steps) return fail(LRDS_ERR_INVALID, "per-step table missing");
   if (s->ctrl_kind < LRDS_CTRL_CLIPPED || s->ctrl_kind > LRDS_CTRL_LERP) return fail(LRDS_ERR_INVALID, "unknown ctrl_kind");
-  if (s->ctrl_kind == LRDS_CTRL_LERP && (s->ref_0.M != 1 || !s->ref_0.mu || !s->ref_0.ivar))
+  if (s->ctrl_kind == LRDS_CTRL_LERP && (s->ref_0.M != 1 || s->ref_0.layout != LRDS_GMM_DIAG || !s->ref_0.mu || !s->ref_0.ivar))
     return fail(LRDS_ERR_INVALID, "LerpCtrl needs the diagonal Gaussian prior in ref_0");
   switch (s->target.kind) {
     case LRDS_DISTR_GMM:
       if (int r = validate_gmm(s->target.gmm, "target")) return r;
+      if (int r = refuse_full(s->target.gmm, "target")) return r;
       break;
     case LRDS_DISTR_PHI4:
       break;
@@ -376,6 +389,14 @@ __global__ void __launch_bounds__(128) distr_eval_kernel(const lrds_spec s, cons
   const GmmView tv0 = gmm_at(s.target.gmm, 0);
   const int d = s.d, dp = s.mlp.d_pad;
   for (int j = 0; j < dp; ++j) P.x(j) = (j < d) ? __ldg(x + (int64_t)b * d + j) : 0.f;
+  if (s.target.kind == LRDS_DISTR_GMM && s.target.gmm.layout == LRDS_GMM_FULL) {  // score column P.rr, scratch P.rh
+    const GmmFullView g = gmm_full_at(s.target.gmm, 0);
+    const float lp = score_out ? gmm_full_pass<true>(g, d, dp, P.x, P.rr, P.rh) : gmm_full_pass<false>(g, d, dp, P.x, P.rr, P.rh);
+    if (live && logp_out) logp_out[b] = lp + s.rnd_offset;
+    if (live && score_out)
+      for (int j = 0; j < d; ++j) score_out[(int64_t)b * d + j] = P.rr(j);
+    return;
+  }
   const float lp = target_pass1<false>(s, s.target.kind, tv0, P, logp_out != nullptr);
   if (live && logp_out) logp_out[b] = lp + s.rnd_offset;
   if (!score_out) return;
@@ -739,6 +760,7 @@ int distr_spec(const lrds_distr* distr, int32_t d, int32_t B, lrds_spec* out) {
   s.precision = LRDS_PRECISION_F16X3;  // column layout without the fp32 network's activation columns (no network here)
   if (distr->kind == LRDS_DISTR_GMM) {
     if (int r = validate_gmm(distr->gmm, "distr")) return r;
+    if (int r = refuse_full(distr->gmm, "score_cot_sums")) return r;
   } else if (distr->kind == LRDS_DISTR_LOGREG) {
     if (distr->logreg.p + 1 != d) return fail(LRDS_ERR_INVALID, "logreg: d must be p + 1");
   } else if (distr->kind != LRDS_DISTR_PHI4) {
@@ -812,7 +834,10 @@ int lrds_rollout(const lrds_spec* spec, const float* x0, const float* noise, uin
     return fail(LRDS_ERR_UNSUPPORTED, "CancelDriftCtrl / LerpCtrl are built for the LINEAR simulate loop (DIS) only");
   if (linear && s.has_ref_ctrl)
     if (int r = validate_gmm(s.ref_t, "ref_t")) return r;
-  if (!linear && s.ref_0.M != 1) return fail(LRDS_ERR_UNSUPPORTED, "CMCD needs a diagonal Gaussian prior");
+  if (!linear && (s.ref_0.M != 1 || s.ref_0.layout != LRDS_GMM_DIAG))
+    return fail(LRDS_ERR_UNSUPPORTED, "CMCD needs a diagonal Gaussian prior");
+  if (s.init_cost)
+    if (int r = refuse_full(s.ref_0, "the DIS prior (init_cost)")) return r;
   if (!linear && s.target.kind == LRDS_DISTR_NONE) return fail(LRDS_ERR_INVALID, "CMCD needs a target");
   cudaStream_t st = (cudaStream_t)stream;
   lrds::RolloutArgs a{s, x0, noise, seed, particle_offset, x_out, rnd_out, traj_out};
@@ -866,6 +891,7 @@ int64_t lrds_gmm_mix_tc_bytes(int32_t M, int32_t d_pad) {
 }
 
 int lrds_pack_gmm_mix_tc(const lrds_gmm* gmm, int32_t d, int32_t d_pad, int32_t steps, void* image_out, void* stream) {
+  if (gmm && gmm->layout != LRDS_GMM_DIAG) return fail(LRDS_ERR_UNSUPPORTED, "pack_gmm_mix_tc: diagonal blocks only");
   if (!gmm || !image_out || !gmm->mu || !gmm->ivar || !gmm->logc || gmm->M < 2 || gmm->M > 64 || d < 1 || d > d_pad || d_pad < 8 ||
       d_pad % 8 != 0 || d_pad > LRDS_MAX_DIM_PAD || steps < 1)
     return fail(LRDS_ERR_INVALID, "pack_gmm_mix_tc: bad arguments");
@@ -992,6 +1018,7 @@ int lrds_mala(const lrds_distr* target, int32_t d, int32_t C, int32_t n_warmup, 
   s.kind = LRDS_ROLLOUT_CMCD;  // column layout with the three extra per-chain vectors (current state, two scores)
   if (target->kind == LRDS_DISTR_GMM) {
     if (int r = validate_gmm(target->gmm, "target")) return r;
+    if (int r = refuse_full(target->gmm, "mala")) return r;
   } else if (target->kind == LRDS_DISTR_LOGREG) {
     if (target->logreg.p + 1 != d) return fail(LRDS_ERR_INVALID, "logreg: d must be p + 1");
   } else if (target->kind != LRDS_DISTR_PHI4) {

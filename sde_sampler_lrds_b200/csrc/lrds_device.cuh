@@ -452,6 +452,107 @@ __device__ __forceinline__ void gmm_score_chunk(const GmmViewT<SH>& g, int d, in
 }
 
 // ---------------------------------------------------------------------------------------------------
+// full-covariance Gaussian mixture (lrds_gmm.layout == LRDS_GMM_FULL), distr/gauss.py:76-121
+// ---------------------------------------------------------------------------------------------------
+// Per mode m: h_m = prec_m (x - mu_m), q_m = (x - mu_m) . h_m, logit_m = logc_m - q_m / 2.  The precision rows are
+// warp-uniform 16-byte loads through L1 (one broadcast load feeds 32 particles); a per-step block is M d_pad^2 floats,
+// far beyond the TMA step stage at the sizes this layout is for, so nothing is staged.  The arithmetic is fp32 in
+// every network precision.
+struct GmmFullView {
+  int M;
+  const float* logc;
+  const float* mu;    // [M][dp]
+  const float* prec;  // [M][dp][dp]
+};
+__device__ __forceinline__ GmmFullView gmm_full_at(const lrds_gmm& g, int step) {
+  return GmmFullView{g.M, g.logc + (int64_t)step * g.step_stride_logc, g.mu + (int64_t)step * g.step_stride_param,
+                     g.sn + (int64_t)step * g.step_stride_sn};
+}
+
+// q_m of mode m; with STORE, h_m goes to column h (zero in the padded dims: the padded precision rows are zero).
+// Eight rows of prec at a time, so that one read of (x - mu) from the particle column feeds 32 FMA.
+template <bool STORE>
+__device__ __forceinline__ float gmm_full_mode(const GmmFullView& g, int m, int d, int dp, const Col4& x, const Col4& h) {
+  const float* P = g.prec + (int64_t)m * dp * dp;
+  const float4* mu4 = reinterpret_cast<const float4*>(g.mu + (int64_t)m * dp);
+  const int nq = (d + 3) >> 2;
+  float q = 0.f;
+  for (int i0 = 0; i0 < d; i0 += JC) {
+    float acc[JC];
+#pragma unroll
+    for (int r = 0; r < JC; ++r) acc[r] = 0.f;
+    const float4* row = reinterpret_cast<const float4*>(P + (int64_t)i0 * dp);
+    const int rq = dp >> 2;  // float4 per row
+#pragma unroll 2
+    for (int c = 0; c < nq; ++c) {
+      const float4 xv = x.ld4(c), mv = __ldg(mu4 + c);
+      const float y0 = xv.x - mv.x, y1 = xv.y - mv.y, y2 = xv.z - mv.z, y3 = xv.w - mv.w;
+#pragma unroll
+      for (int r = 0; r < JC; ++r) {
+        const float4 p = __ldg(row + r * rq + c);
+        acc[r] = fmaf(p.x, y0, acc[r]);
+        acc[r] = fmaf(p.y, y1, acc[r]);
+        acc[r] = fmaf(p.z, y2, acc[r]);
+        acc[r] = fmaf(p.w, y3, acc[r]);
+      }
+    }
+    const float4 xa = x.ld4(i0 >> 2), xb = x.ld4((i0 >> 2) + 1);
+    const float4 ma = __ldg(mu4 + (i0 >> 2)), mb = __ldg(mu4 + (i0 >> 2) + 1);
+    q = fmaf(xa.x - ma.x, acc[0], q); q = fmaf(xa.y - ma.y, acc[1], q);
+    q = fmaf(xa.z - ma.z, acc[2], q); q = fmaf(xa.w - ma.w, acc[3], q);
+    q = fmaf(xb.x - mb.x, acc[4], q); q = fmaf(xb.y - mb.y, acc[5], q);
+    q = fmaf(xb.z - mb.z, acc[6], q); q = fmaf(xb.w - mb.w, acc[7], q);
+    if constexpr (STORE) {
+      h.st4(i0 >> 2, make_float4(acc[0], acc[1], acc[2], acc[3]));
+      h.st4((i0 >> 2) + 1, make_float4(acc[4], acc[5], acc[6], acc[7]));
+    }
+  }
+  return q;
+}
+
+// log sum_m exp(logit_m) (the mixture log-density) in one pass over the modes with a running maximum.  With a score
+// column `sc` (SCORE), also sc = -sum_m r_m h_m, r = softmax_m(logit_m), accumulated online: sc holds
+// sum_m exp(logit_m - running max) h_m and is rescaled whenever the maximum moves; `h` is the per-mode scratch column.
+template <bool SCORE>
+__device__ __forceinline__ float gmm_full_pass(const GmmFullView& g, int d, int dp, const Col4& x, const Col4& sc,
+                                               const Col4& h) {
+  float mx = -INFINITY, s = 0.f;
+  const int nq = dp >> 2;
+  for (int m = 0; m < g.M; ++m) {
+    const float l = __ldg(g.logc + m) - 0.5f * gmm_full_mode<SCORE>(g, m, d, dp, x, h);
+    float w, scale;
+    if (l > mx) {
+      scale = __expf(mx - l);  // 0 for the first mode
+      w = 1.f;
+      mx = l;
+    } else {
+      scale = 1.f;
+      w = __expf(l - mx);
+    }
+    s = fmaf(s, scale, w);
+    if constexpr (SCORE) {
+      if (m == 0) {
+        for (int c = 0; c < nq; ++c) sc.st4(c, h.ld4(c));
+      } else {
+        for (int c = 0; c < nq; ++c) {
+          const float4 a = sc.ld4(c), b = h.ld4(c);
+          sc.st4(c, make_float4(fmaf(a.x, scale, w * b.x), fmaf(a.y, scale, w * b.y), fmaf(a.z, scale, w * b.z),
+                                fmaf(a.w, scale, w * b.w)));
+        }
+      }
+    }
+  }
+  if constexpr (SCORE) {
+    const float inv = -1.0f / s;
+    for (int c = 0; c < nq; ++c) {
+      const float4 a = sc.ld4(c);
+      sc.st4(c, make_float4(a.x * inv, a.y * inv, a.z * inv, a.w * inv));
+    }
+  }
+  return mx + __logf(s);
+}
+
+// ---------------------------------------------------------------------------------------------------
 // PhiFour (1-D lattice, Dirichlet-0)
 // ---------------------------------------------------------------------------------------------------
 // score_j = -beta * [ (b - x_j (1 - x_j^2)) / coef + coef (2 x_j - x_{j+1} - x_{j-1}) ]

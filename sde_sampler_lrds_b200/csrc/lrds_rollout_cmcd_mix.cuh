@@ -24,7 +24,7 @@ constexpr int CMX_MAX_WARPS = 8;  // two tiles: x and s in shared memory (448 B 
 constexpr uint32_t CMX_TILE_COLS = 192, CMX_DB_COL = 128;
 
 __host__ __device__ inline bool cmcd_mix_applicable(const lrds_spec& s) {
-  return s.precision == LRDS_PRECISION_F16X3 && s.kind == LRDS_ROLLOUT_CMCD && s.ctrl_kind <= LRDS_CTRL_SCORE &&
+  return s.precision == LRDS_PRECISION_F16X3 && s.kind == LRDS_ROLLOUT_CMCD && s.ctrl_kind <= LRDS_CTRL_SCORE && !gmm_full_on_path(s) &&
          s.target.kind == LRDS_DISTR_GMM && s.target.gmm.M > 1 && s.target.gmm.M <= MIX_MAX_M && s.target.gmm.mix_tc != nullptr &&
          s.ref_0.M == 1 && s.mlp.d_pad <= 56 && !s.init_cost;
 }

@@ -59,7 +59,7 @@ __host__ __device__ inline bool cmcd_tc_applicable(const lrds_spec& s) {
   const bool cmcd = s.kind == LRDS_ROLLOUT_CMCD || s.kind == LRDS_ROLLOUT_EUBO_CMCD;
   const bool lin = s.kind == LRDS_ROLLOUT_LINEAR && !s.has_ref_ctrl && s.ctrl_kind == LRDS_CTRL_SCORE;
   if (!(s.precision == LRDS_PRECISION_F16X3 && (cmcd || lin) && s.target.kind == LRDS_DISTR_LOGREG &&
-        s.target.logreg.x_tc != nullptr && s.ref_0.M == 1 && s.mlp.d_pad <= 64))
+        s.target.logreg.x_tc != nullptr && s.ref_0.M == 1 && s.mlp.d_pad <= 64 && !gmm_full_on_path(s)))
     return false;
   return cmcd_tc_layout(s).cols <= 512;
 }

@@ -18,6 +18,7 @@ namespace lrds {
 
 __host__ __device__ inline bool lin_tc_applicable(const lrds_spec& s) {
   return s.precision == LRDS_PRECISION_F16X3 && s.kind == LRDS_ROLLOUT_LINEAR && !s.has_ref_ctrl && s.ctrl_kind <= LRDS_CTRL_SCORE &&
+         !gmm_full_on_path(s) &&
          (s.target.kind == LRDS_DISTR_PHI4 || s.target.kind == LRDS_DISTR_NONE ||
           (s.target.kind == LRDS_DISTR_GMM && s.ctrl_kind == LRDS_CTRL_CLIPPED && s.target.gmm.M == 1));
 }

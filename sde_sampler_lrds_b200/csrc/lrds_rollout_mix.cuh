@@ -60,7 +60,7 @@ using MixBench = MixCfg<false, 1, 2, false>;  // the benchmark configuration
 
 // index of the configuration that serves `s` (see launch_mix_f16x3), or -1
 __host__ __device__ inline int mix_tc_config(const lrds_spec& s) {
-  if (s.precision != LRDS_PRECISION_F16X3 || s.mlp.d_pad > 128) return -1;
+  if (s.precision != LRDS_PRECISION_F16X3 || s.mlp.d_pad > 128 || gmm_full_on_path(s)) return -1;
   const bool tmix = s.ctrl_kind == LRDS_CTRL_SCORE && s.target.kind == LRDS_DISTR_GMM && s.target.gmm.M > 1 &&
                     s.target.gmm.M <= MIX_MAX_M && s.target.gmm.mix_tc != nullptr;
   const bool tdis = s.ctrl_kind >= LRDS_CTRL_CANCEL_DRIFT && s.target.kind == LRDS_DISTR_GMM && s.target.gmm.M > 1 &&

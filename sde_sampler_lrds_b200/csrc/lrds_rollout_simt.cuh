@@ -35,8 +35,14 @@ __device__ __forceinline__ void report_status(const lrds_spec& s, bool live, boo
 
 // shared-memory floats per particle for a spec (host + device agree through this one function)
 struct ColLayout {
-  int x, act, rt, rr, g, us, tsd, db, total;
+  int x, act, rt, rr, rh, g, us, tsd, db, total;
 };
+
+// a full-covariance reference (lrds_gmm.layout) on the time-marginal path resp. as the terminal term
+__host__ __device__ inline bool ref_t_full(const lrds_spec& s) { return s.has_ref_ctrl && s.ref_t.layout == LRDS_GMM_FULL; }
+__host__ __device__ inline bool gmm_full_on_path(const lrds_spec& s) {
+  return ref_t_full(s) || s.ref_0.layout == LRDS_GMM_FULL || (s.target.kind == LRDS_DISTR_GMM && s.target.gmm.layout == LRDS_GMM_FULL);
+}
 
 // mix_tc: the mixture-score contractions run on the tensor core (lrds_rollout_mix.cuh): responsibilities live in
 // registers / TMEM, not in shared-memory columns
@@ -48,12 +54,18 @@ __host__ __device__ inline ColLayout col_layout(const lrds_spec& s, bool mix_tc 
   L.act = off;
   if (s.precision == LRDS_PRECISION_FP32_SIMT) off += C;  // hidden activations: tensor-core backends keep them in TMEM
   L.rt = off;
-  if (!mix_tc && s.target.kind == LRDS_DISTR_GMM && s.target.gmm.M > 1) off += (s.target.gmm.M + 3) / 4 * 4;
+  const bool tfull = s.target.kind == LRDS_DISTR_GMM && s.target.gmm.layout == LRDS_GMM_FULL;  // lrds_distr_eval only
+  if (!mix_tc && !tfull && s.target.kind == LRDS_DISTR_GMM && s.target.gmm.M > 1) off += (s.target.gmm.M + 3) / 4 * 4;
   L.rr = off;
-  if (!mix_tc) {
+  L.rh = off;
+  if (ref_t_full(s) || tfull) {  // full-covariance reference: its score (rr) and the per-mode scratch h (rh), d_pad floats each
+    L.rh = off + dp;
+    off += 2 * dp;
+    if (s.ref_0.layout != LRDS_GMM_FULL && s.ref_0.M > 1 && s.ref_0.M > 2 * dp) off += (s.ref_0.M + 3) / 4 * 4 - 2 * dp;
+  } else if (!mix_tc) {
     int m = 0;
     if (s.has_ref_ctrl && s.ref_t.M > 1) m = s.ref_t.M;
-    if (s.ref_0.M > 1 && s.ref_0.M > m) m = s.ref_0.M;
+    if (s.ref_0.layout != LRDS_GMM_FULL && s.ref_0.M > 1 && s.ref_0.M > m) m = s.ref_0.M;
     off += (m + 3) / 4 * 4;
   }
   L.g = off;
@@ -72,7 +84,7 @@ __host__ __device__ inline ColLayout col_layout(const lrds_spec& s, bool mix_tc 
 
 // x, rt, rr are float4-grouped columns (their layout offsets are multiples of 4); the rest are scalar columns
 struct Particle {
-  Col4 x, rt, rr;
+  Col4 x, rt, rr, rh;
   Col g, us, tsd, db;
 };
 
@@ -81,6 +93,7 @@ __device__ __forceinline__ Particle make_particle(float* smem, const ColLayout& 
   P.x = Col4{smem + L.x * NT + 4 * tid, 4 * NT};
   P.rt = Col4{smem + L.rt * NT + 4 * tid, 4 * NT};
   P.rr = Col4{smem + L.rr * NT + 4 * tid, 4 * NT};
+  P.rh = Col4{smem + L.rh * NT + 4 * tid, 4 * NT};
   P.g = Col{smem + L.g * NT + tid, NT};
   P.us = Col{smem + L.us * NT + tid, NT};
   P.tsd = Col{smem + L.tsd * NT + tid, NT};
@@ -119,7 +132,7 @@ __host__ __device__ inline StageLayout stage_layout(const lrds_spec& s, int leve
     if (mix_tc) L.tgt_mix_bytes = gmm_mix_tc_bytes(s.target.gmm.M, s.mlp.d_pad);
     L.tgt_bytes = L.tgt_logc_bytes + L.tgt_param_bytes + L.tgt_mix_bytes;
   }
-  if (s.has_ref_ctrl && s.ref_t.M > 1) {  // single Gaussians are read from global memory
+  if (s.has_ref_ctrl && s.ref_t.M > 1 && !ref_t_full(s)) {  // single Gaussians (and full blocks) are read from global memory
     L.ref_logc_bytes = (uint32_t)((s.ref_t.M + 3) / 4 * 4) * 4u;
     L.ref_param_bytes = (uint32_t)((s.ref_t.M + 3) / 4) * dp * 32u;
     if (mix_tc) L.ref_mix_bytes = gmm_mix_tc_bytes(s.ref_t.M, s.mlp.d_pad);
@@ -167,16 +180,19 @@ struct LinearTraits {
   static constexpr int kIto = ITO;        // lrds_ito_form
   static constexpr int kTarget = TARGET;  // lrds_distr_kind
   static constexpr int kScore = SCORE;    // 1 = ScoreCtrl, 0 = ClippedCtrl
-  static constexpr int kRef = REF;        // 0 = no reference control, 1 = Gaussian (M == 1), 2 = mixture (M > 1)
+  static constexpr int kRef = REF;        // 0 = no reference control, 1 = Gaussian (M == 1), 2 = mixture (M > 1), 3 = full (ref_class)
 };
 using RuntimeTraits = LinearTraits<>;
-__host__ __device__ inline int ref_class(const lrds_spec& s) { return !s.has_ref_ctrl ? 0 : (s.ref_t.M > 1 ? 2 : 1); }
+// 3 = full-covariance reference (any M): only the run-time-switched kernels serve it
+__host__ __device__ inline int ref_class(const lrds_spec& s) {
+  return !s.has_ref_ctrl ? 0 : (ref_t_full(s) ? 3 : (s.ref_t.M > 1 ? 2 : 1));
+}
 template <class TR>
 __host__ __device__ inline bool traits_match(const lrds_spec& s) {
   return (TR::kUpdate < 0 || TR::kUpdate == s.update_form) && (TR::kIto < 0 || TR::kIto == s.ito_form) &&
          (TR::kTarget < 0 || TR::kTarget == s.target.kind) &&
          (TR::kScore < 0 || (s.ctrl_kind <= LRDS_CTRL_SCORE && TR::kScore == (s.ctrl_kind == LRDS_CTRL_SCORE))) &&
-         (TR::kRef < 0 || TR::kRef == ref_class(s)) &&
+         (TR::kRef < 0 || TR::kRef == ref_class(s)) && (TR::kRef < 0 || !gmm_full_on_path(s)) &&
          (!TR::kMix || ((s.target.kind != LRDS_DISTR_GMM || s.target.gmm.M > 1) && (!s.has_ref_ctrl || s.ref_t.M > 1)));
 }
 
@@ -326,6 +342,13 @@ __device__ __forceinline__ float langevin_drift(const lrds_spec& s, float ts, fl
   return clipf(dr, s.cmcd_clip);
 }
 
+// reference_log_prob(x) of the terminal term: ref_0 in either layout (full: h is not stored, the score column untouched)
+template <bool PIPE>
+__device__ __forceinline__ float ref0_log_prob(const lrds_spec& s, const Particle& P) {
+  if (s.ref_0.layout == LRDS_GMM_FULL) return gmm_full_pass<false>(gmm_full_at(s.ref_0, 0), s.d, s.mlp.d_pad, P.x, P.rr, P.rh);
+  return gmm_pass1<PIPE>(gmm_at(s.ref_0, 0), s.d, s.mlp.d_pad, P.x, P.rr);
+}
+
 // `smem` = this CTA's column area (col_layout(s).total * blockDim.x floats); every thread of the CTA runs the body
 // with uniform control flow (idle lanes shadow the last particle), which the tensor-core policy relies on.
 // STAGE > 0 (LINEAR kind): `stage` is a stage_layout(s, STAGE).total-byte shared-memory area; the time-marginal
@@ -356,6 +379,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
   const int update_form = TR::kUpdate >= 0 ? TR::kUpdate : s.update_form;
   const int ito_form = TR::kIto >= 0 ? TR::kIto : s.ito_form;
   const bool need_nbr = tkind == LRDS_DISTR_PHI4;  // lattice stencil reads x_{j0-1}, x_{j0+8}
+  const bool rfull = TR::kRef < 0 && has_ref && s.ref_t.layout == LRDS_GMM_FULL;  // full reference: score column P.rr
   CtrlConst cc = ctrl_const(s);
   cc.score = score_ctrl;
   const GmmView tv0 = gmm_at(s.target.gmm, 0);  // target mixture in global memory (dereferenced for GMM targets only)
@@ -396,17 +420,18 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
         const uint8_t* buf = stage + SL.off_buf + (k & 1) * SL.buf_bytes;
         row = reinterpret_cast<const float*>(buf);
         rowp = PPtr<true>{ptx::smem_u32(buf)};
-        if (has_ref) rv = staged_view(buf + SL.row_bytes, gmm_at(s.ref_t, k), SL.ref_logc_bytes, SL.ref_param_bytes);
+        if (has_ref && !rfull) rv = staged_view(buf + SL.row_bytes, gmm_at(s.ref_t, k), SL.ref_logc_bytes, SL.ref_param_bytes);
       } else {
         rowp = PPtr<false>{row};
-        if (has_ref) rv = gmm_at(s.ref_t, k);
+        if (has_ref && !rfull) rv = gmm_at(s.ref_t, k);
       }
       const float A = rowp.ld1(LRDS_STEP_A), Bc = rowp.ld1(LRDS_STEP_B), Cc = rowp.ld1(LRDS_STEP_C);
       const float dt = rowp.ld1(LRDS_STEP_DT), sqdt = rowp.ld1(LRDS_STEP_SQRT_DT);
       const float wcost = rowp.ld1(LRDS_STEP_W_COST), wito = rowp.ld1(LRDS_STEP_W_ITO);
       const float gamma = rowp.ld1(LRDS_STEP_GAMMA), sigu = rowp.ld1(LRDS_STEP_SIGU);
       if (score_ctrl) target_pass1<PIPE, TR::kMix>(s, tkind, tv, P, false);
-      if (has_ref && (TR::kRef == 2 || rv.M > 1)) gmm_pass1<PIPE, TR::kMix>(rv, d, dp, P.x, P.rr);
+      if (rfull) gmm_full_pass<true>(gmm_full_at(s.ref_t, k), d, dp, P.x, P.rr, P.rh);
+      else if (has_ref && (TR::kRef == 2 || rv.M > 1)) gmm_pass1<PIPE, TR::kMix>(rv, d, dp, P.x, P.rr);
       mlp.template hidden<SH>(row + LRDS_STEP_BIAS1, P.x);
       float su2 = 0.f, sito = 0.f, xm = 0.f;
       for (int j0 = 0; j0 < dp; j0 += JC) {
@@ -421,7 +446,8 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
         } else {
           ctrl_chunk(cc, mlp, j0, ts, gamma, u);
         }
-        if (has_ref) gmm_score_chunk<PIPE, TR::kMix>(rv, d, dp, xr, P.rr, j0, rs);
+        if (rfull) load_chunk(P.rr, j0, rs);
+        else if (has_ref) gmm_score_chunk<PIPE, TR::kMix>(rv, d, dp, xr, P.rr, j0, rs);
         noise_chunk(a, k, b, j0, z);
 #pragma unroll
         for (int c = 0; c < JC; ++c) {
@@ -450,7 +476,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
     // terminal cost: rnd += reference_log_prob(x) - terminal_unnorm_log_prob(x)   (oc.py:290, 505, 645, 1389);
     // init_cost (DIS): the initial cost initial_log_prob(x_0) + rnd_offset, written to rnd_out by lrds_rollout's pre-pass,
     // takes the place of the reference term (oc.py:1164-1168, 1230)
-    const float lref = s.init_cost ? a.rnd_out[b] : gmm_pass1<PIPE>(gmm_at(s.ref_0, 0), d, dp, P.x, P.rr);
+    const float lref = s.init_cost ? a.rnd_out[b] : ref0_log_prob<PIPE>(s, P);
     const float ltgt = clipf(target_pass1<PIPE>(s, tkind, tv, P, true), s.clip_target);
     rnd += lref - ltgt;
   }
@@ -458,7 +484,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
   if constexpr (KIND == LRDS_ROLLOUT_EUBO_LINEAR) {
     {  // rnd = reference_log_prob(x) - terminal_unnorm_log_prob(x)   (oc.py:321, 536); init_cost (the discrete-time
        // DIS loss, oc.py:1000-1033): ref_0 is the prior and enters at the END of the noising rollout instead
-      const float lref = s.init_cost ? 0.f : gmm_pass1<PIPE>(gmm_at(s.ref_0, 0), d, dp, P.x, P.rr);
+      const float lref = s.init_cost ? 0.f : ref0_log_prob<PIPE>(s, P);
       const float ltgt = clipf(target_pass1<PIPE>(s, tkind, tv0, P, true), s.clip_target);
       rnd = lref - ltgt;
     }
@@ -479,7 +505,9 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
       }
       if (score_ctrl) target_pass1<PIPE>(s, tkind, tv0, P, false);
       GmmView rv{};
-      if (has_ref) {
+      if (rfull) {
+        gmm_full_pass<true>(gmm_full_at(s.ref_t, k), d, dp, P.x, P.rr, P.rh);
+      } else if (has_ref) {
         rv = gmm_at(s.ref_t, k);
         if (rv.M > 1) gmm_pass1<PIPE>(rv, d, dp, P.x, P.rr);
       }
@@ -491,7 +519,9 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
         const float xp = (need_nbr && j0 + JC < dp) ? P.x(j0 + JC) : 0.f;
         if (score_ctrl) target_score_chunk<PIPE>(s, tkind, tv0, P, xr, xm, xp, j0, ts);
         ctrl_chunk(cc, mlp, j0, ts, gamma, u);
-        if (has_ref) {
+        if (rfull) {
+          load_chunk(P.rr, j0, rs);
+        } else if (has_ref) {
           gmm_score_chunk<PIPE>(rv, d, dp, xr, P.rr, j0, rs);
         } else {
 #pragma unroll

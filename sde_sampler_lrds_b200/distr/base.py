@@ -119,7 +119,61 @@ def gmm_mix_tc_image(loc: torch.Tensor, var: torch.Tensor, d_pad: int, logc: tor
     return torch.cat(blocks, dim=-1).contiguous()
 
 
+class FullBlock(tuple):
+    """(logc, mu, prec) of a full-covariance block (lrds_gmm.layout = LRDS_GMM_FULL, include/lrds_b200.h)."""
+
+
+def full_eig(cov: torch.Tensor):
+    """(eigenvalues [..][d], eigenvectors [..][d][d]) of symmetric positive-definite covariances, decomposed once in
+    float64 and returned as float32 (the per-step blocks are formed from them in float32)."""
+    c = cov.detach().to("cpu", torch.float64)
+    evals, evecs = torch.linalg.eigh(0.5 * (c + c.transpose(-1, -2)))
+    if not bool((evals > 0).all()):
+        raise ValueError("covariance matrices must be positive definite")
+    return evals.float(), evecs.float()
+
+
+def gmm_full_block(means: torch.Tensor, evals: torch.Tensor, evecs: torch.Tensor, weights: torch.Tensor | None, device,
+                   s: torch.Tensor | None = None, sigma_sq: torch.Tensor | None = None):
+    """Packs the full-covariance mixture N(s mu_m, s^2 (Sigma_m + sigma_sq I)), Sigma_m = P_m diag(D_m) P_m^T, into a
+    FullBlock.  ``s`` / ``sigma_sq`` carry a leading step axis ([S][1][1]) for the time-marginal reference (then every
+    array gets one block per step) and default to 1 / 0 (the distribution itself).  Float32, in the order
+        loc = s mu,  prec = P diag(1 / (D + sigma_sq)) P^T / s^2,
+        logc = log w - d/2 log(2 pi) - 1/2 sum_i log(s^2 (D_i + sigma_sq)),
+    rows padded to d_pad = 8 ceil(d / 8) with zeros (prec in its padded rows and columns too), logc to a multiple of
+    4 entries with -inf."""
+    means = means.detach().to("cpu", torch.float32)
+    D, P = evals.to("cpu", torch.float32), evecs.to("cpu", torch.float32)
+    M, d = means.shape
+    s = torch.ones((1, 1)) if s is None else s.to("cpu", torch.float32)
+    sigma_sq = torch.zeros((1, 1)) if sigma_sq is None else sigma_sq.to("cpu", torch.float32)
+    Ds = D + sigma_sq                                                     # [(S)][M][d]
+    loc = s * means
+    prec = torch.matmul(P * (1.0 / Ds).unsqueeze(-2), P.transpose(-1, -2)) / s.unsqueeze(-1) ** 2
+    logc = -0.5 * d * math.log(2.0 * math.pi) - 0.5 * torch.log(s ** 2 * Ds).sum(dim=-1)
+    if weights is not None:
+        w = weights.detach().to("cpu", torch.float32)
+        logc = logc + torch.log(w / w.sum())
+    pad, mpad = (-d) % 8, (-M) % 4
+    F = torch.nn.functional
+    loc = F.pad(loc, (0, pad))
+    prec = F.pad(prec, (0, pad, 0, pad))
+    logc = F.pad(logc, (0, mpad), value=float("-inf"))
+    return FullBlock(t.contiguous().to(device) for t in (logc, loc, prec))
+
+
 def fill_gmm(g: N.Gmm, block, stepped: bool = False):
+    if isinstance(block, FullBlock):
+        logc, mu, prec = block
+        g.layout = N.GMM_FULL
+        g.M = mu.shape[-2]
+        g.logc, g.mu, g.ivar, g.sn = logc.data_ptr(), mu.data_ptr(), None, prec.data_ptr()
+        g.step_stride_logc = logc.shape[-1] if stepped else 0
+        g.step_stride_param = g.M * mu.shape[-1] if stepped else 0
+        g.step_stride_sn = g.M * mu.shape[-1] ** 2 if stepped else 0
+        g.mix_tc, g.step_stride_mix_tc = None, 0
+        return g
+    g.layout = N.GMM_DIAG
     logc, mu, ivar, sn = block[:4]
     g.M = mu.shape[-2]
     g.logc, g.mu, g.ivar, g.sn = logc.data_ptr(), mu.data_ptr(), ivar.data_ptr(), sn.data_ptr()

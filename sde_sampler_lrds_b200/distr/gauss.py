@@ -1,7 +1,9 @@
 """Diagonal Gaussian / Gaussian-mixture family with the reference's class names and constructors
 (sde_sampler/distr/gauss.py: GMM 138-307, TwoModes 422-453, ManyModes 569-594, Gauss 597-629,
 IsotropicGauss 720-787) and its functional helpers (log_prob_gaussian 67-73, score_mog 97-107,
-score_gauss 124-126).  Densities and scores are evaluated by the CUDA library."""
+score_gauss 124-126), plus the full-covariance Gaussian / mixture of the learned RDS references (GaussFull, GMMFull;
+score_mog_full / log_prob_gaussian_full, distr/gauss.py:76-121).  Densities and scores are evaluated by the CUDA
+library."""
 from __future__ import annotations
 
 import ctypes as C
@@ -9,7 +11,7 @@ import ctypes as C
 import torch
 
 from .. import _native as N
-from .base import Distribution, fill_gmm, gmm_block
+from .base import Distribution, fill_gmm, full_eig, gmm_block, gmm_full_block
 
 
 class _AdHocMixture(Distribution):
@@ -166,3 +168,84 @@ class IsotropicGauss(Gauss):
     def sample(self, shape=None) -> torch.Tensor:
         shape = tuple(shape or ())
         return self.loc[0, 0] + self.scale[0, 0] * torch.randn(*shape, self.dim, device=self.domain.device)
+
+
+class GMMFull(Distribution):
+    """Mixture of Gaussians with full covariance matrices: the learned RDS reference fitted with
+    ``fit_gmm(em_type="full")`` and its time marginals (``MarginalReference.distr_at``).
+
+    The reference names this class but its constructor could not be checked here; the signature below is this
+    project's own.  ``covariance_matrix`` is [M][d][d] (symmetric positive definite), or ``eig`` = (eigenvalues [M][d],
+    eigenvectors [M][d][d]) with Sigma_m = P_m diag(D_m) P_m^T, the form ``OU.marginal_params`` takes.  A matrix is
+    decomposed once in float64.  ``log_prob`` / ``score`` run through lrds_distr_eval (full layout)."""
+
+    def __init__(self, dim: int = 2, loc=None, covariance_matrix=None, mixture_weights=None, eig=None, **kwargs):
+        super().__init__(dim=dim, log_norm_const=0.0, **kwargs)
+        if (covariance_matrix is None) == (eig is None):
+            raise ValueError("give exactly one of covariance_matrix and eig")
+        self.n_mixtures = loc.shape[0]
+        if loc.shape != (self.n_mixtures, dim):
+            raise ValueError("loc must be [M][dim]")
+        evals, evecs = full_eig(covariance_matrix) if eig is None else (eig[0].float(), eig[1].float())
+        evals, evecs = evals.reshape(self.n_mixtures, dim), evecs.reshape(self.n_mixtures, dim, dim)
+        if not bool((evals > 0).all()):
+            raise ValueError("covariance matrices must be positive definite")
+        if mixture_weights is None and self.n_mixtures > 1:
+            raise ValueError("Require mixture weights.")
+        self.register_buffer("loc", loc, persistent=False)
+        self.register_buffer("eigenvalues", evals.to(loc.device), persistent=False)
+        self.register_buffer("eigenvectors", evecs.to(loc.device), persistent=False)
+        self.register_buffer("mixture_weights", mixture_weights, persistent=False)
+        self._marginal = None  # (means_init, s, sigma_sq): packed in the time-marginal operation order
+
+    @classmethod
+    def marginal(cls, means, evals, evecs, weights, s, sigma_sq, device):
+        """N(s mu_m, s^2 (Sigma_m + sigma_sq I)), packed with the arithmetic of the reference blocks (gmm_full_block)."""
+        means, s, sigma_sq = means.float(), torch.as_tensor(s).float().reshape(1, 1), torch.as_tensor(sigma_sq).float().reshape(1, 1)
+        out = cls.__new__(cls)
+        GMMFull.__init__(out, dim=means.shape[-1], loc=(s * means).to(device), eig=(s ** 2 * (evals + sigma_sq), evecs),
+                         mixture_weights=None if weights is None else weights.to(device))
+        out._marginal = (means, evals, evecs, s, sigma_sq)
+        return out
+
+    @property
+    def covariance_matrix(self):
+        return (self.eigenvectors * self.eigenvalues.unsqueeze(-2)) @ self.eigenvectors.transpose(-1, -2)
+
+    def block(self, device):
+        if self._marginal is not None:
+            means, evals, evecs, s, sigma_sq = self._marginal
+            return gmm_full_block(means, evals, evecs, self.mixture_weights, device, s=s, sigma_sq=sigma_sq)
+        return gmm_full_block(self.loc, self.eigenvalues, self.eigenvectors, self.mixture_weights, device)
+
+    def _lrds_pack(self, device):
+        d = N.Distr()
+        d.kind = N.DISTR_GMM
+        block = self.block(device)
+        fill_gmm(d.gmm, block)
+        return d, block
+
+    def sample(self, shape=None) -> torch.Tensor:
+        shape = tuple(shape or ())
+        n = int(torch.tensor(shape).prod()) if shape else 1
+        if self.mixture_weights is None:
+            comp = torch.zeros(n, dtype=torch.long, device=self.loc.device)
+        else:
+            comp = torch.multinomial(self.mixture_weights / self.mixture_weights.sum(), n, replacement=True)
+        z = torch.randn(n, self.dim, device=self.loc.device) * self.eigenvalues[comp].sqrt()
+        x = self.loc[comp] + (self.eigenvectors[comp] @ z.unsqueeze(-1)).squeeze(-1)
+        return x.reshape(*shape, self.dim)
+
+    def has_entropy(self):
+        return self.n_mixtures > 1
+
+
+class GaussFull(GMMFull):
+    """Gaussian with a full covariance matrix ``covariance_matrix`` [d][d] (or ``eig`` = (eigenvalues [d], eigenvectors
+    [d][d])).  Constructor signature: this project's own, as for GMMFull."""
+
+    def __init__(self, dim: int = 1, loc=0.0, covariance_matrix=None, eig=None, **kwargs):
+        loc = Gauss._prepare_input(loc, dim)
+        if covariance_matrix is not None:
+            covariance_matrix = torch.as_tensor(covariance_matrix).reshape(1, dim, dim)
+        super().__init__(dim=dim, loc=loc, covariance_matrix=covariance_matrix, eig=eig, **kwargs)

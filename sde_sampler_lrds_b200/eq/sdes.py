@@ -17,8 +17,8 @@ import torch
 from torch.nn import Module
 
 from .. import _native as N
-from ..distr.base import Distribution, fill_gmm, gmm_block
-from ..distr.gauss import GMM, Gauss
+from ..distr.base import Distribution, fill_gmm, full_eig, gmm_block, gmm_full_block
+from ..distr.gauss import GMM, Gauss, GaussFull, GMMFull
 
 _noise_calls = itertools.count()
 
@@ -155,10 +155,13 @@ class OU(TorchSDE):
         a = self.s(t)
         return torch.log(torch.square(a) / (torch.square(a) * self.sigma_sq(t)))
 
-    # ---- reference marginals p_t^ref (diagonal covariances) ----------------------------------------------
+    # ---- reference marginals p_t^ref ---------------------------------------------------------------------
     def marginal_params(self, t, x_init, var_init=None, is_mixture: bool = False):
+        """(loc, var) of the marginal at t.  Full covariances (a matrix per component, or its eigen form (D, P)) come back
+        in eigen form: (loc, (s^2 (D + sigma_sq), P)) (eq/sdes.py:232-239)."""
         if isinstance(var_init, tuple) or (var_init is not None and var_init.dim() > x_init.dim()):
-            raise NotImplementedError("full-covariance references are a later row (SURVEY.md 8f item 2)")
+            evals, evecs = var_init if isinstance(var_init, tuple) else full_eig(var_init)
+            return self.s(t) * x_init, (self.s(t) ** 2 * (evals + self.sigma_sq(t)), evecs)
         loc = self.s(t) * x_init
         var = self.s(t) ** 2 * self.sigma_sq(t)
         if var_init is not None:
@@ -375,15 +378,20 @@ class PinnedBM(OU):
 
 class MarginalReference:
     """The time-marginal reference score nabla log p_t^ref(x) of RDS (solver/oc.py:513-592) as an object the
-    rollout can introspect: a diagonal Gaussian (``gaussian``/``default``) or mixture (``gmm``) pushed through
-    the OU marginals (eq/sdes.py:208-248, 265-279, 329-345)."""
+    rollout can introspect: a Gaussian (``gaussian``/``default``) or mixture (``gmm``) pushed through the OU marginals
+    (eq/sdes.py:208-248, 265-279, 329-345).  Covariances are diagonal ([d] / [M][d]) or full: a matrix ([d][d] /
+    [M][d][d]) or the eigen form (eigenvalues [(M)][d], eigenvectors [(M)][d][d]); a matrix is decomposed once (fp64).
+    The full kind packs LRDS_GMM_FULL blocks: per step the precision matrices P diag(1 / (D + sigma_sq)) P^T / s^2."""
 
     def __init__(self, sde: OU, kind: str, x_init=None, var_init=None, means_init=None, variances_init=None,
                  weights_init=None):
         self.sde, self.kind = sde, kind
+        full_g = False
         if kind == "gaussian":
             self.means = x_init.reshape(1, -1)
-            self.variances = None if var_init is None else var_init.reshape(1, -1)
+            full_g = isinstance(var_init, tuple) or (var_init is not None and var_init.dim() == 2 and
+                                                        var_init.shape[0] == var_init.shape[1] == self.means.shape[-1] > 1)
+            self.variances = var_init if full_g or var_init is None else var_init.reshape(1, -1)
             self.weights = None
         elif kind == "gmm":
             self.means, self.variances, self.weights = means_init, variances_init, weights_init
@@ -391,15 +399,35 @@ class MarginalReference:
                 self.weights = torch.ones(means_init.shape[0]) / means_init.shape[0]
         else:
             raise NotImplementedError(f"reference type {kind!r} has no B200 kernel")
-        if isinstance(self.variances, tuple) or (self.variances is not None and self.variances.dim() != 2):
-            raise NotImplementedError("full-covariance references are a later row (SURVEY.md 8f item 2)")
+        M, d = self.means.shape
+        self.full = isinstance(self.variances, tuple) or (self.variances is not None and self.variances.dim() == 3) or \
+            (kind == "gaussian" and full_g)
+        if self.full:
+            if isinstance(self.variances, tuple):
+                evals, evecs = self.variances
+            else:
+                evals, evecs = full_eig(self.variances.reshape(M, d, d))
+            # tensors of the object key the cached rollout plans (losses/oc.py, _state)
+            self.eigenvalues = evals.detach().to("cpu", torch.float32).reshape(M, d)
+            self.eigenvectors = evecs.detach().to("cpu", torch.float32).reshape(M, d, d)
+            if not bool((self.eigenvalues > 0).all()):
+                raise ValueError("reference covariances must be positive definite")
+        elif self.variances is not None and self.variances.dim() != 2:
+            raise NotImplementedError("diagonal reference variances must be [M][d]")
 
     @property
     def dim(self):
         return self.means.shape[-1]
 
+    def _s_sigma_sq(self, taus):
+        h = self.sde.host()
+        taus = taus.detach().to("cpu", torch.float32).reshape(-1, 1, 1)
+        return h.s(taus), h.sigma_sq(taus)
+
     def params_at(self, taus: torch.Tensor):
-        """(loc[S][M][d], var[S][M][d]) on the host for a 1-D tensor of times."""
+        """(loc[S][M][d], var[S][M][d]) on the host for a 1-D tensor of times (diagonal kinds)."""
+        if self.full:
+            raise ValueError("params_at is the diagonal form; a full-covariance reference packs with block_at")
         h = self.sde.host()
         taus = taus.detach().to("cpu", torch.float32).reshape(-1, 1, 1)
         means = self.means.detach().to("cpu", torch.float32).unsqueeze(0)
@@ -411,10 +439,18 @@ class MarginalReference:
         return loc, var.expand_as(loc)
 
     def block_at(self, taus, device):
+        if self.full:
+            s, sig2 = self._s_sigma_sq(taus)
+            return gmm_full_block(self.means, self.eigenvalues, self.eigenvectors, self.weights, device, s=s, sigma_sq=sig2)
         loc, var = self.params_at(taus)
         return gmm_block(loc, var, self.weights, device)
 
     def distr_at(self, t, device) -> Distribution:
+        if self.full:
+            s, sig2 = self._s_sigma_sq(torch.as_tensor(t).reshape(1))
+            cls = GaussFull if self.kind == "gaussian" else GMMFull
+            return cls.marginal(self.means.detach().cpu().float(), self.eigenvalues, self.eigenvectors,
+                                None if self.weights is None else self.weights.detach().cpu().float(), s, sig2, device)
         loc, var = self.params_at(torch.as_tensor(t).reshape(1))
         if self.kind == "gaussian":
             return Gauss(dim=self.dim, loc=loc[0].to(device), scale=var[0].sqrt().to(device), domain_tol=None)

@@ -14,7 +14,7 @@ import torch
 
 from . import _native as N
 from .distr.base import Distribution, fill_gmm, gmm_block
-from .distr.gauss import GMM
+from .distr.gauss import GMM, GMMFull
 from .models.mlp import FourierMLP, TimeEmbed
 from .models.reparam import CancelDriftCtrl, ClippedCtrl, LerpCtrl, ScoreCtrl
 
@@ -224,7 +224,11 @@ def _scalar_rows(ts: torch.Tensor):
 
 
 def gauss_block_from(distr: Distribution, device):
-    """(logc, mu, ivar) block of a diagonal Gaussian / mixture Distribution (for ref_0 / the CMCD prior)."""
+    """(logc, mu, ivar) block of a diagonal Gaussian / mixture Distribution (for ref_0 / the CMCD prior), or the
+    FullBlock of a full-covariance one (GaussFull / GMMFull: the RDS reference term ref_0; the CMCD / DIS priors and
+    LerpCtrl are refused for it by the library)."""
+    if isinstance(distr, GMMFull):
+        return distr.block(device)
     if not isinstance(distr, GMM):
         raise NotImplementedError(f"{type(distr).__name__} cannot serve as a Gaussian reference / prior here")
     return gmm_block(distr.loc, torch.square(distr.scale), distr.mixture_weights, device)

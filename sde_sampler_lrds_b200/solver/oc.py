@@ -312,8 +312,9 @@ class RDS(TrainableDiff):
     def change_reference_type(self, ref_type="default", net=None, eps=None, mean=None, var=None, means=None,
                               variances=None, weights=None):
         """Reference distribution and its time marginals (solver/oc.py:513-588): 'default' (from prior and SDE),
-        'gaussian' (mean, diagonal var), 'gmm' (means, diagonal variances, weights).  'nn' and full covariances are
-        later rows (SURVEY.md 8f items 2-3)."""
+        'gaussian' (mean, var = diagonal [d], full [d][d] or the eigen form (eigenvalues, eigenvectors)), 'gmm' (means,
+        variances = diagonal [M][d], full [M][d][d] or the eigen form, weights).  'nn' is a later row (SURVEY.md 8f
+        item 3)."""
         if ref_type == "default":
             loc = self.prior.loc.detach().flatten().cpu()
             if isinstance(self.sde, VP):
@@ -326,14 +327,12 @@ class RDS(TrainableDiff):
             self.reference_distr_utils = {"x_init": loc, "var_init": var0}
             self.reference_score_t = MarginalReference(self.sde, "gaussian", x_init=loc, var_init=var0)
         elif ref_type == "gaussian":
-            if isinstance(var, tuple) or var.ndim == 2:
-                raise NotImplementedError("full-covariance references are a later row (SURVEY.md 8f item 2)")
-            self.reference_distr_utils = {"x_init": mean.float().cpu(), "var_init": var.float().cpu()}
+            var = tuple(v.float().cpu() for v in var) if isinstance(var, tuple) else var.float().cpu()
+            self.reference_distr_utils = {"x_init": mean.float().cpu(), "var_init": var}
             self.reference_score_t = MarginalReference(self.sde, "gaussian", **self.reference_distr_utils)
         elif ref_type == "gmm":
-            if isinstance(variances, tuple) or variances.ndim == 3:
-                raise NotImplementedError("full-covariance references are a later row (SURVEY.md 8f item 2)")
-            self.reference_distr_utils = {"means_init": means.float().cpu(), "variances_init": variances.float().cpu(),
+            variances = tuple(v.float().cpu() for v in variances) if isinstance(variances, tuple) else variances.float().cpu()
+            self.reference_distr_utils = {"means_init": means.float().cpu(), "variances_init": variances,
                                           "weights_init": weights.float().cpu()}
             self.reference_score_t = MarginalReference(self.sde, "gmm", **self.reference_distr_utils)
         elif ref_type == "nn":
