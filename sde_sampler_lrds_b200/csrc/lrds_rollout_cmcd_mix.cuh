@@ -38,48 +38,24 @@ rollout_cmcd_mix_kernel(const RolloutArgs a, const uint8_t* __restrict__ image, 
   const int tid = threadIdx.x;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int nwarps = blockDim.x >> 5, NT = blockDim.x;
-  uint8_t* img = smem_raw;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + TL.bytes);  // [0] image + target block, [1 + t] MMAs of tile t done
-  uint32_t* slot = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 48);
   uint32_t* cnts = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + TC_TAIL_BYTES);
   uint8_t* stage = smem_raw + TL.bytes + TC_TAIL_BYTES + MIX_TAIL_BYTES;  // the static target mixture: logc | sn | tensor-core images
   const StageLayout SL = stage_layout(s, 2, true);
   float* cols = reinterpret_cast<float*>(stage + ((SL.off_buf + 15u) & ~15u));
   const int d = s.d, dp = s.mlp.d_pad, K = s.K;
   const uint32_t mix_off_t = SL.tgt_logc_bytes + SL.tgt_param_bytes;
-  if (warp == 0) ptx::tmem_alloc(slot, tmem_cols);
-  if (tid == 0) {
-    for (int i = 0; i < 3; ++i) ptx::mbar_init(bars + i, 1);
-    for (int i = 0; i < 4; ++i) cnts[i] = 0u;
-    ptx::fence_mbar_init();
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  if (tid == 0) {  // drift weights and the target mixture, staged once per CTA by the TMA engine
-    ptx::mbar_expect_tx(bars, TL.bytes + SL.tgt_bytes);
-    ptx::bulk_g2s(img, image, TL.bytes, bars);
+  auto target = [&]() {  // the target mixture, staged once per CTA with the drift weights
     stage_gmm(stage + SL.off_tgt, gmm_at(s.target.gmm, 0), SL.tgt_logc_bytes, SL.tgt_param_bytes, bars);
     ptx::bulk_g2s(stage + SL.off_tgt + mix_off_t, static_cast<const uint8_t*>(s.target.gmm.mix_tc), SL.tgt_mix_bytes, bars);
-  }
-  ptx::mbar_wait(bars, 0);
-  const uint32_t tmem = __shfl_sync(0xffffffffu, *slot, 0);
+  };
+  const uint32_t tmem =
+      __shfl_sync(0xffffffffu, tc_cta_begin(smem_raw, TL, image, tmem_cols, warp, 3, nullptr, 0, cnts, 4, SL.tgt_bytes, target), 0);
   const int tile = warp >> 2;
   const int tile_warps = min(4, nwarps - 4 * tile);
   MixTc<PREC> mlp;
-  mlp.L = TL;
-  mlp.img = img;
-  mlp.img_s = ptx::smem_u32(img);
-  mlp.tm_tile = tmem + (uint32_t)tile * CMX_TILE_COLS;
-  mlp.tm_lane = mlp.tm_tile + ((uint32_t)((warp & 3) * 32) << 16);
-  mlp.bar = bars + 1 + tile;
-  mlp.phase = 0;
-  mlp.cnt = cnts + tile;
-  mlp.tile_warps = (uint32_t)tile_warps;
-  mlp.target = 0u;
-  mlp.hand = 0u;
-  mlp.issue_mask = ((warp & 3) == tile_warps - 1 ? 1u : 0u) | ((warp & 3) == max(tile_warps - 2, 0) ? 2u : 0u);
-  mlp.dp = dp;
+  mlp.init(TL, smem_raw, tmem + (uint32_t)tile * CMX_TILE_COLS, warp, bars + 1 + tile, cnts + tile, (uint32_t)tile_warps,
+           ((warp & 3) == tile_warps - 1 ? 1u : 0u) | ((warp & 3) == max(tile_warps - 2, 0) ? 2u : 0u), dp);
   const int Mt = s.target.gmm.M;
   const uint32_t contr_bytes = gmm_mix_contr_bytes(Mt, dp), lg_part = gmm_mix_logit_part_bytes(Mt, dp);
   mlp.lbo = (uint32_t)(2 * dp) * 16u;
@@ -268,9 +244,7 @@ rollout_cmcd_mix_kernel(const RolloutArgs a, const uint8_t* __restrict__ image, 
       }
   }
   report_status(s, live, mlp.saturated(), !isfinite(rnd + xsum));
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 0) ptx::tmem_dealloc(tmem, tmem_cols);
+  tc_cta_end(warp, tmem, tmem_cols);
 }
 
 // shared memory: [weight image | barriers | counters | target mixture | x and s columns]
@@ -285,16 +259,11 @@ inline bool plan_rollout_cmcd_mix(const lrds_spec& s, int smem_cap, int sms, TcP
   int wmax = (int)(((size_t)smem_cap - fixed) / per_warp);
   wmax = wmax < CMX_MAX_WARPS ? wmax : CMX_MAX_WARPS;
   const int need = (s.B + 31) / 32;
-  const int waves = (need + sms * wmax - 1) / (sms * wmax);
-  int w = (need + sms * waves - 1) / (sms * waves);
-  w = w < 1 ? 1 : (w > wmax ? wmax : w);
-  const int tiles = (w + 3) / 4;
-  uint32_t cols = 32;
-  while (cols < (uint32_t)tiles * CMX_TILE_COLS) cols <<= 1;
+  const int w = plan_warps(need, sms, wmax);
   out->warps = w;
   out->grid = (need + w - 1) / w;
   out->staged = 2;
-  out->tmem_cols = cols;
+  out->tmem_cols = plan_tmem_cols((w + 3) / 4 * (int)CMX_TILE_COLS);
   out->smem = fixed + per_warp * w;
   return true;
 }

@@ -114,64 +114,29 @@ struct CmcdTc : TcMlp<LRDS_PRECISION_F16X3> {
   const uint8_t* ximg;   // the same, generic
   float usx;             // its un-scale
 
-  // D[dcol] (+)= A (hi at a_hi, lo at a_lo; 8 packed columns per K step) . B (hi image at b, lo at b + part), 3 passes
-  __device__ __forceinline__ void mma_x3(uint32_t dcol, uint32_t a_hi, uint32_t a_lo, uint32_t a_step, uint32_t b, uint32_t b_part,
-                                         uint32_t b_step, uint32_t lbo, uint32_t sbo, int ksteps, uint32_t idesc) {
-    uint32_t acc = 0;
-#pragma unroll 1
-    for (int pass = 0; pass < 3; ++pass) {  // small terms first: lo.hi, hi.lo, hi.hi
-      const uint32_t a = pass == 0 ? a_lo : a_hi;
-      const uint32_t bb = b + (pass == 1 ? b_part : 0u);
-      for (int ks = 0; ks < ksteps; ++ks) {
-        ptx::mma_bf16_ts(dcol, a + (uint32_t)ks * a_step, ptx::make_smem_desc(bb + (uint32_t)ks * b_step, lbo, sbo), idesc, acc);
-        acc = 1;
-      }
-    }
-  }
-
   // x -> A; first drift-network layer AND the logit GEMM (N16 may exceed the 256-column MMA limit: split)
   __device__ __forceinline__ void issue_first(const Col4& x) {
-    for (int c0 = 8 * half; c0 < L.Kin / 2; c0 += 16) {  // this thread's 16-dim groups -> 8 packed columns each
-      float v[16];
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const int j0 = 2 * c0 + 8 * h;
-        float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
-        if (j0 < dp) {
-          a = x.ld4(j0 >> 2);
-          b = x.ld4((j0 >> 2) + 1);
-        }
-        v[8 * h + 0] = a.x; v[8 * h + 1] = a.y; v[8 * h + 2] = a.z; v[8 * h + 3] = a.w;
-        v[8 * h + 4] = b.x; v[8 * h + 5] = b.y; v[8 * h + 6] = b.z; v[8 * h + 7] = b.w;
-      }
-      store16_half(c0, v);
-    }
-    const bool mine = handoff();
-    if (mine && ptx::elect_one()) {
+    store_x(x, half, 2);  // this thread's 16-dim groups
+    arrive_issue([&]() {
       const uint32_t a_hi = tm_tile + a_col(0), a_lo = tm_tile + a_col(1);
-      mma_x3(tm_tile + d_col(), a_hi, a_lo, 8u, img_s + L.off_in, L.part_bytes, 2u * (uint32_t)C * 16u, (uint32_t)C * 16u, 128u,
-             L.Kin / 16, ptx::make_idesc_f16(128, C));
+      mma_passes<true, false>(tm_tile + d_col(), a_hi, a_lo, 8u, img_s + L.off_in, L.part_bytes, 2u * (uint32_t)C * 16u,
+                              (uint32_t)C * 16u, 128u, L.Kin / 16, ptx::make_idesc_f16(128, C));
       const int nsplit = (CL.N16 + 255) / 256;
       const int per = ((CL.N16 / 16 + nsplit - 1) / nsplit) * 16;
       for (int n0 = 0; n0 < CL.N16; n0 += per) {
         const int nn = min(per, CL.N16 - n0);
-        mma_x3(tm_tile + CL.z_col + (uint32_t)n0, a_hi, a_lo, 8u, ximg_s + (uint32_t)n0 * 16u, CL.part_bytes,
-               2u * (uint32_t)CL.N16 * 16u, (uint32_t)CL.N16 * 16u, 128u, CL.K16 / 16, ptx::make_idesc_f16(128, nn));
+        mma_passes<true, false>(tm_tile + CL.z_col + (uint32_t)n0, a_hi, a_lo, 8u, ximg_s + (uint32_t)n0 * 16u, CL.part_bytes,
+                                2u * (uint32_t)CL.N16 * 16u, (uint32_t)CL.N16 * 16u, 128u, CL.K16 / 16, ptx::make_idesc_f16(128, nn));
       }
-      ptx::mma_commit(bar);
-    }
-    if (mine) __syncwarp();
+    });
   }
   // gradient GEMM: A = g (hi | lo per 16 data, in place of the logits), B = the data image read MN-major
   __device__ __forceinline__ void issue_gradient() {
-    const bool mine = handoff();
-    if (mine && ptx::elect_one()) {
+    arrive_issue([&]() {
       const uint32_t zc = tm_tile + CL.z_col;
-      mma_x3(tm_tile + CL.t_col, zc, zc + 8u, 16u, ximg_s, CL.part_bytes, 256u, 128u, (uint32_t)CL.N16 * 16u, CL.N16 / 16,
-             ptx::make_idesc_f16(128, CL.K16) | (1u << 16));
-      ptx::mma_commit(bar);
-    }
-    if (mine) __syncwarp();
+      mma_passes<true, false>(tm_tile + CL.t_col, zc, zc + 8u, 16u, ximg_s, CL.part_bytes, 256u, 128u, (uint32_t)CL.N16 * 16u,
+                              CL.N16 / 16, ptx::make_idesc_f16(128, CL.K16) | (1u << 16));
+    });
   }
 
   // logits of data [16 t0, 16 t1) -> g = m (y - sigma(z)), m = [eps <= sigma <= 1 - eps] (and >= threshold), as fp16
@@ -272,43 +237,16 @@ rollout_cmcd_tc_kernel(const RolloutArgs a, const uint8_t* __restrict__ image, c
   const int tid = threadIdx.x, warp = tid >> 5;
   constexpr int NT = 128;                          // particles per CTA; 256 threads = two per particle
   const int pt = tid & (NT - 1), half = tid >> 7;  // particle slot and which of its two threads
-  uint8_t* img = smem_raw;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + TL.bytes);
-  uint32_t* slot = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 48);
+  uint32_t* cnt = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 64);  // the tile's hand-off counter
   uint8_t* ximg = smem_raw + TL.bytes + TC_TAIL_BYTES;
   float* dimtab = reinterpret_cast<float*>(ximg + ((CL.img_bytes + 15u) & ~15u));  // [4][dp] per-dim constants
   float* cols = dimtab + cmcd_tab_floats(a.s.mlp.d_pad);
-  if (warp == 0) ptx::tmem_alloc(slot, tmem_cols);
-  if (tid == 0) {
-    for (int i = 0; i < 2; ++i) ptx::mbar_init(bars + i, 1);
-    *reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 64) = 0u;  // the tile's hand-off counter
-    ptx::fence_mbar_init();
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  if (tid == 0) {  // drift weights and the data image, staged once per CTA by the TMA engine
-    ptx::mbar_expect_tx(bars, TL.bytes + CL.img_bytes);
-    ptx::bulk_g2s(img, image, TL.bytes, bars);
-    ptx::bulk_g2s(ximg, LR.x_tc, CL.img_bytes, bars);
-  }
-  ptx::mbar_wait(bars, 0);
-  const uint32_t tmem = *slot;
+  auto data = [&]() { ptx::bulk_g2s(ximg, LR.x_tc, CL.img_bytes, bars); };  // the data image, staged with the drift weights
+  const uint32_t tmem = tc_cta_begin(smem_raw, TL, image, tmem_cols, warp, 2, nullptr, 0, cnt, 1, CL.img_bytes, data);
   CmcdTc mlp;
-  mlp.L = TL;
-  mlp.img = img;
-  mlp.img_s = ptx::smem_u32(img);
-  mlp.tm_tile = tmem;
-  mlp.tm_lane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-  mlp.bar = bars + 1;
-  mlp.phase = 0;
-  mlp.bar_id = 1;
-  mlp.bar_threads = 2 * NT;
-  mlp.issuer = warp == 0;  // (warp-uniform)
-  mlp.hand_cnt = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 64);
-  mlp.hand_warps = (uint32_t)(2 * NT / 32);
+  mlp.init(TL, smem_raw, tmem, warp, bars + 1, cnt, (uint32_t)(2 * NT / 32), warp == 0 ? 3u : 0u, s.mlp.d_pad);  // warp 0 issues
   mlp.half = half;
-  mlp.dp = s.mlp.d_pad;
   mlp.CL = CL;
   mlp.ximg = ximg;
   mlp.ximg_s = ptx::smem_u32(ximg);
@@ -521,9 +459,7 @@ rollout_cmcd_tc_kernel(const RolloutArgs a, const uint8_t* __restrict__ image, c
   if (live && a.x_out != nullptr)
     for (int j = half; j < d; j += 2) a.x_out[(int64_t)b * d + j] = X(j);
   report_status(s, live, mlp.saturated(), !half && !isfinite(rnd));
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 0) ptx::tmem_dealloc(tmem, tmem_cols);
+  tc_cta_end(warp, tmem, tmem_cols);
 }
 
 inline bool plan_rollout_cmcd_tc(const lrds_spec& s, int smem_cap, TcPlan* out) {

@@ -33,40 +33,16 @@ rollout_lin_kernel(const RolloutArgs a, const uint8_t* __restrict__ image, const
   const int tid = threadIdx.x, warp = tid >> 5;
   const int nwarps = blockDim.x >> 6, NT = blockDim.x >> 1;  // warps / threads that own particles (a multiple of 4 / 128)
   const int half = tid >= NT, ptid = tid - half * NT, pwarp = warp - half * nwarps;  // the particle's two threads
-  uint8_t* img = smem_raw;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + TL.bytes);  // [0] image, [1 + t] tile t
-  uint32_t* slot = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 48);
+  uint32_t* cnts = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 64);  // [t] hand-offs of tile t
   float* cols = reinterpret_cast<float*>(smem_raw + TL.bytes + TC_TAIL_BYTES);
-  if (warp == 0) ptx::tmem_alloc(slot, tmem_cols);
-  if (tid == 0) {
-    for (int i = 0; i < 5; ++i) ptx::mbar_init(bars + i, 1);
-    for (int i = 0; i < 4; ++i) reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 64)[i] = 0u;
-    ptx::fence_mbar_init();
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  if (tid == 0) {
-    ptx::mbar_expect_tx(bars, TL.bytes);
-    ptx::bulk_g2s(img, image, TL.bytes, bars);
-  }
-  ptx::mbar_wait(bars, 0);
-  const uint32_t tmem = *slot;
+  const uint32_t tmem = tc_cta_begin(smem_raw, TL, image, tmem_cols, warp, 5, nullptr, 0, cnts, 4, 0u, []() {});
   const int tile = pwarp >> 2;
+  const int bar_id = 1 + tile;  // the tile's named barrier: 4 warps x 2 threads per particle (full tiles only)
   TcMlp<PREC> mlp;
-  mlp.L = TL;
-  mlp.img = img;
-  mlp.img_s = ptx::smem_u32(img);
-  mlp.tm_tile = tmem + (uint32_t)(tile * TL.tile_cols);
-  mlp.tm_lane = mlp.tm_tile + ((uint32_t)((warp & 3) * 32) << 16);
-  mlp.bar = bars + 1 + tile;
-  mlp.phase = 0;
-  mlp.bar_id = 1 + tile;
-  mlp.bar_threads = 256;  // full tiles only: 4 warps x 2 threads per particle
-  mlp.issuer = half == 0 && (pwarp & 3) == 3;  // one warp of the tile (warp-uniform)
-  mlp.hand_cnt = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 64) + tile;
-  mlp.hand_warps = 8u;  // 4 warps x 2 threads per particle
-  mlp.dp = s.mlp.d_pad;
+  // one warp of the tile issues every hand-off of its 4 x 2 warps
+  mlp.init(TL, smem_raw, tmem + (uint32_t)(tile * TL.tile_cols), warp, bars + 1 + tile, cnts + tile, 8u,
+           half == 0 && (pwarp & 3) == 3 ? 3u : 0u, s.mlp.d_pad);
 
   const int b_raw = blockIdx.x * NT + ptid;
   const bool live = b_raw < s.B;
@@ -103,27 +79,13 @@ rollout_lin_kernel(const RolloutArgs a, const uint8_t* __restrict__ image, const
     // update as x' = xa x + xu u + xz z:  AXPY (A, B, C);  EM x + (-(f x) + sigma u) dt + sigma (z sqrt dt)
     const u64 xa2 = f2::pk(EM ? 1.0f - A * dt : A), xu2 = f2::pk(EM ? Bc * dt : Bc), xz2 = f2::pk(EM ? Bc * sqdt : Cc);
     const u64 gs2 = f2::pk(cc.scale_score * gamma);
-    ptx::bar_sync(mlp.bar_id, 256);  // the pair's writes of x (previous chunk loop / initial load) are visible to both
+    ptx::bar_sync(bar_id, 256);  // the pair's writes of x (previous chunk loop / initial load) are visible to both
     // the lattice sites next to this thread's range, before anybody updates them (the barriers of the network's GEMMs
     // separate these reads from the chunk loops)
     float xm = (PHI4 && c_begin > 0) ? X(c_begin * JC - 1) : 0.f;
     const float x_after = (PHI4 && c_end * JC < dp) ? X(c_end * JC) : 0.f;
     {  // the drift network with the operand columns and the epilogue halves split between the pair
-      for (int c0 = 8 * half; c0 < mlp.L.Kin / 2; c0 += 16) {
-        float v[16];
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int j0 = 2 * c0 + 8 * h;
-          float4 va = make_float4(0.f, 0.f, 0.f, 0.f), vb = va;
-          if (j0 < dp) {
-            va = X.ld4(j0 >> 2);
-            vb = X.ld4((j0 >> 2) + 1);
-          }
-          v[8 * h + 0] = va.x; v[8 * h + 1] = va.y; v[8 * h + 2] = va.z; v[8 * h + 3] = va.w;
-          v[8 * h + 4] = vb.x; v[8 * h + 5] = vb.y; v[8 * h + 6] = vb.z; v[8 * h + 7] = vb.w;
-        }
-        mlp.store16_half(c0, v);
-      }
+      mlp.store_x(X, half, 2);
       mlp.issue(mlp.L.off_in, mlp.L.Kin, C);
       const float* bh = reinterpret_cast<const float*>(mlp.img + mlp.L.off_bhid);
       for (int l = 0; l <= mlp.L.nh; ++l) {
@@ -215,9 +177,7 @@ rollout_lin_kernel(const RolloutArgs a, const uint8_t* __restrict__ image, const
       a.x_out[(int64_t)b * d + j] = v;
     }
   report_status(s, live, mlp.saturated(), !isfinite(half ? xsum : rnd + xsum) && !half);  // non-finite: counted once per particle
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 0) ptx::tmem_dealloc(tmem, tmem_cols);
+  tc_cta_end(warp, tmem, tmem_cols);
 }
 
 inline bool plan_rollout_lin(const lrds_spec& s, int smem_cap, int sms, TcPlan* out) {
@@ -231,12 +191,10 @@ inline bool plan_rollout_lin(const lrds_spec& s, int smem_cap, int sms, TcPlan* 
   const bool two = 2 * TL.tile_cols <= 512 && fixed + 2 * per_tile <= (size_t)smem_cap && s.B > 128 * sms;
   const int w = two ? 8 : 4;
   const int need = (s.B + 31) / 32;
-  uint32_t cols = 32;
-  while ((int)cols < (w / 4) * TL.tile_cols) cols <<= 1;
   out->warps = 2 * w;  // launched warps: two threads per particle
   out->grid = (need + w - 1) / w;
   out->staged = 0;
-  out->tmem_cols = cols;
+  out->tmem_cols = plan_tmem_cols((w / 4) * TL.tile_cols);
   out->smem = fixed + per_tile * (w / 4);
   return true;
 }

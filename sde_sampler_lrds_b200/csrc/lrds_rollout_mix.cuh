@@ -225,84 +225,15 @@ template <int PREC>
 struct MixTc : TcMlp<PREC> {
   using Base = TcMlp<PREC>;
   static constexpr uint32_t kRCol = 0, kDCol = 32;
-  uint32_t* cnt;        // the tile's hand-off counter: one increment per warp and hand-off
-  uint32_t target;      // its value once every warp of the tile has arrived for the current hand-off
-  uint32_t tile_warps;
-  uint32_t issue_mask;  // bit (n & 1): this warp issues the tile's hand-offs n with that parity (warp-uniform)
-  uint32_t hand;        // hand-offs so far
   uint32_t lbo, part_bytes;  // contraction image: bytes between the K chunks (modes 0-7 | 8-15), bytes of one (hi | lo) part
   uint32_t lg_part;          // logit image: bytes of one (hi | lo) part
   MixTm tm;
 
-  // This warp's part of the tile's next batch is in place (A rows stored / accumulator rows read).  Every warp
-  // increments the tile's counter (release, no round trip) and goes on; the hand-off's issuer warp - the tile's last
-  // two warps take turns; in a full tile they sit on the two SM sub-partitions that carry three particle warps instead
-  // of four and therefore have slack - polls the counter, issues the batch `f` from warp-uniform registers and
-  // commits it to the tile's mbarrier.  A partial last tile (whose warps all sit on the loaded sub-partitions) has
-  // issue_mask = 0: its batches are issued by the CTA's auxiliary warp (mix_aux_issuer).
-  // `done` = the mbarrier the batch commits to (default: the tile's; a batch that completes while the tile already
-  // works on the next one needs its own, or the tile's barrier would run two phases ahead of a waiter)
-  template <class F>
-  __device__ __forceinline__ void arrive_issue(F&& f, uint64_t* done = nullptr) {
-    ptx::tmem_wait_st();
-    ptx::tc_fence_before();
-    __syncwarp();
-    if ((threadIdx.x & 31) == 0) ptx::red_add_release(cnt, 1u);
-    const bool mine = (issue_mask >> (hand & 1u)) & 1u;
-    ++hand;
-    if (mine) issue_when_ready(f, done);
-    else target += tile_warps;
-  }
-  // polls the tile's counter until every warp has arrived for the next hand-off, then issues and commits its batch
-  template <class F>
-  __device__ __forceinline__ void issue_when_ready(F&& f, uint64_t* done = nullptr) {
-    target += tile_warps;
-    while ((int32_t)(ptx::ld_acquire(cnt) - target) < 0) {
-    }
-    ptx::tc_fence_after();
-    if (ptx::elect_one()) {
-      f();
-      ptx::mma_commit(done ? done : this->bar);
-    }
-    __syncwarp();
-  }
-
-  // one layer of the network: D = A . W^T as three passes of fp16 (hi, lo) products, small terms first
-  __device__ __forceinline__ void gemm(uint32_t b_off, int K, int N) const {
-    const uint32_t idesc = ptx::make_idesc_f16(128, N);
-    const uint32_t dcol = this->tm_tile + this->d_col();
-    const int ksteps = K / this->L.kstep;
-    const uint32_t kbytes = 2u * (uint32_t)N * 16u;  // one MMA consumes two 16-byte K chunks
-    uint32_t acc = 0;
-#pragma unroll
-    for (int pass = 0; pass < 3; ++pass) {
-      const int a_part = pass == 0 ? 1 : 0, b_part = pass == 1 ? 1 : 0;
-      const uint32_t abase = this->tm_tile + this->a_col(a_part);
-      const uint32_t bbase = this->img_s + (uint32_t)b_part * this->L.part_bytes + b_off;
-      for (int ks = 0; ks < ksteps; ++ks) {
-        const uint64_t bdesc = ptx::make_smem_desc(bbase + (uint32_t)ks * kbytes, (uint32_t)N * 16u, 128u);
-        ptx::mma_bf16_ts(dcol, abase + ks * 8, bdesc, idesc, acc);
-        acc = 1;
-      }
-    }
-  }
   // logits of mixture `which` (0 target, 1 reference): accumulator columns [16 which, 16 which + 16) <- x . wc^T
   __device__ __forceinline__ void logit(int which, uint32_t img, int col = -1) const {
-    const uint32_t idesc = ptx::make_idesc_f16(128, MIX_MAX_M);
     const uint32_t dcol = this->tm_tile + (col < 0 ? this->d_col() : (uint32_t)col) + (uint32_t)which * MIX_MAX_M;
-    const int ksteps = this->L.Kin / 16;
-    uint32_t acc = 0;
-#pragma unroll
-    for (int pass = 0; pass < 3; ++pass) {
-      const int a_part = pass == 0 ? 1 : 0, b_part = pass == 1 ? 1 : 0;
-      const uint32_t abase = this->tm_tile + this->a_col(a_part);
-      const uint32_t bbase = img + (uint32_t)b_part * lg_part;
-      for (int ks = 0; ks < ksteps; ++ks) {
-        const uint64_t bdesc = ptx::make_smem_desc(bbase + (uint32_t)ks * (2u * MIX_MAX_M * 16u), MIX_MAX_M * 16u, 128u);
-        ptx::mma_bf16_ts(dcol, abase + ks * 8, bdesc, idesc, acc);
-        acc = 1;
-      }
-    }
+    mma_passes<true, true>(dcol, this->tm_tile + this->a_col(0), this->tm_tile + this->a_col(1), 8u, img, lg_part,
+                           2u * MIX_MAX_M * 16u, MIX_MAX_M * 16u, 128u, this->L.Kin / 16, ptx::make_idesc_f16(128, MIX_MAX_M));
   }
   // chunk c of the contractions -> columns [32, 64) of the tile; images = shared-window addresses of the (hi | lo) blocks
   template <bool TGT, bool REF>
@@ -380,7 +311,7 @@ struct MixTc : TcMlp<PREC> {
   template <bool BIAS_SH, class S0, class S1>
   __device__ __forceinline__ void hidden_ws(const float* __restrict__ bias1, S0&& slot0, S1&& slot1) {
     const TcLayout& L = this->L;
-    arrive_issue([&]() { gemm(L.off_in, L.Kin, C); });
+    this->issue(L.off_in, L.Kin, C);
     tm.mark(1);
     slot0();
     tm.mark(2);
@@ -395,8 +326,8 @@ struct MixTc : TcMlp<PREC> {
       tm.mark(l == 0 ? 3 : l == 1 ? 6 : 8);
       if (l == 0) this->template epilogue_f16<!BIAS_SH>(bias1, 0);
       else this->template epilogue_f16<false>(bh + (l - 1) * C, l);
-      if (l < nh) arrive_issue([&]() { gemm(L.off_hid + (uint32_t)(l * C * C * L.es), C, C); });
-      else arrive_issue([&]() { gemm(L.off_out, C, L.Nout); });
+      if (l < nh) this->issue(L.off_hid + (uint32_t)(l * C * C * L.es), C, C);
+      else this->issue(L.off_out, C, L.Nout);
       tm.mark(l == 0 ? 4 : 7);
     }
     if (nh == 0) slot1();
@@ -404,6 +335,26 @@ struct MixTc : TcMlp<PREC> {
     tm.mark(8);
   }
 };
+
+// Operands of step k -> step buffer k & 1, completion on its mbarrier (one thread): table row | reference mixture block |
+// its tensor-core images; step 0 also stages the static target mixture (whether or not the control uses its score:
+// the terminal cost does).  Stage layout: [step-buffer mbarriers | target | buffers] (stage_layout).
+template <bool RMIX>
+__device__ __forceinline__ void mix_load_step(const lrds_spec& s, const StageLayout& SL, uint8_t* stage, int k) {
+  uint64_t* sbar = reinterpret_cast<uint64_t*>(stage) + (k & 1);
+  uint8_t* dst = stage + SL.off_buf + (k & 1) * SL.buf_bytes;
+  const bool tgt = k == 0 && SL.tgt_bytes;
+  ptx::mbar_expect_tx(sbar, SL.buf_bytes + (tgt ? SL.tgt_bytes : 0u));
+  if (tgt) {
+    stage_gmm(stage + SL.off_tgt, gmm_at(s.target.gmm, 0), SL.tgt_logc_bytes, SL.tgt_param_bytes, sbar);
+    ptx::bulk_g2s(stage + SL.off_tgt + SL.tgt_logc_bytes + SL.tgt_param_bytes, static_cast<const uint8_t*>(s.target.gmm.mix_tc),
+                  SL.tgt_mix_bytes, sbar);
+  }
+  stage_step(dst, s, SL, k, sbar);
+  if constexpr (RMIX)
+    ptx::bulk_g2s(dst + SL.row_bytes + SL.ref_logc_bytes + SL.ref_param_bytes,
+                  static_cast<const uint8_t*>(s.ref_t.mix_tc) + (int64_t)k * s.ref_t.step_stride_mix_tc, SL.ref_mix_bytes, sbar);
+}
 
 // ---- the loop ------------------------------------------------------------------------------------------------------
 // EUBO: the noising rollout of compute_eubo (losses/oc.py:512-568): per step x <- mean x + std z first, then the
@@ -431,19 +382,12 @@ __device__ __forceinline__ void rollout_body_mix(const RolloutArgs& a, float* sm
   const GmmView tv0 = gmm_at(s.target.gmm, 0);
   const StageLayout SL = stage_layout(s, 2, true);
   uint64_t* sbar = reinterpret_cast<uint64_t*>(stage);  // [i]: step buffer i filled (TMA transaction bytes)
-  const uint8_t* rmix_g = static_cast<const uint8_t*>(s.ref_t.mix_tc);
   const uint32_t mix_off_t = SL.tgt_logc_bytes + SL.tgt_param_bytes;                // inside the target area
   const uint32_t mix_off_r = SL.row_bytes + SL.ref_logc_bytes + SL.ref_param_bytes;  // inside a step buffer
   // a block of mix_tc: [contraction hi | lo | 16 B][logit hi | lo][c_m | 16 B]  (gmm_mix_tc_bytes)
   const int Mt = TMIX ? s.target.gmm.M : s.ref_t.M;  // both are padded to 16 modes: equal block geometry
   const uint32_t contr_bytes = gmm_mix_contr_bytes(Mt, dp), lg_part = gmm_mix_logit_part_bytes(Mt, dp);
   const uint32_t lg_tail_off = contr_bytes + 2u * lg_part;
-  auto load_step = [&](int k) {  // table row | reference mixture block | its tensor-core images -> buffer k & 1 (one thread)
-    uint8_t* dst = stage + SL.off_buf + (k & 1) * SL.buf_bytes;
-    ptx::mbar_expect_tx(sbar + (k & 1), SL.buf_bytes);
-    stage_step(dst, s, SL, k, sbar + (k & 1));
-    if constexpr (RMIX) ptx::bulk_g2s(dst + mix_off_r, rmix_g + (int64_t)k * s.ref_t.step_stride_mix_tc, SL.ref_mix_bytes, sbar + (k & 1));
-  };
   const GmmViewT<true> tv = staged_view(stage + SL.off_tgt, tv0, SL.tgt_logc_bytes, SL.tgt_param_bytes);
   const uint32_t tgt_img = ptx::smem_u32(stage + SL.off_tgt + mix_off_t);
   mlp.lbo = (uint32_t)(2 * dp) * 16u;
@@ -705,7 +649,7 @@ __device__ __forceinline__ void rollout_body_mix(const RolloutArgs& a, float* sm
     __syncwarp();
     if ((tid & 31) == 0) {
       const uint32_t old = ptx::atom_add_acq_rel(step_cnt + (k & 1), 1u);
-      if (old == (uint32_t)((k >> 1) * nwarps + nwarps - 1) && k + 2 < K) load_step(k + 2);
+      if (old == (uint32_t)((k >> 1) * nwarps + nwarps - 1) && k + 2 < K) mix_load_step<RMIX>(s, SL, stage, k + 2);
     }
     mlp.tm.mark(13);
   }
@@ -775,71 +719,32 @@ __global__ void __launch_bounds__(MIX_MAX_WARPS * 32, 1)
 rollout_mix_kernel(const RolloutArgs a, const uint8_t* __restrict__ image, const uint32_t tmem_cols, const int nwarps) {
   // nwarps = particle warps; blockDim.x / 32 = nwarps + 1 when the last tile is partial (the auxiliary issuer warp)
   extern __shared__ __align__(128) uint8_t smem_raw[];
-  constexpr bool TMIX = CFG::kTgt == 1, RMIX = CFG::kRef == 2;
+  constexpr bool RMIX = CFG::kRef == 2;
   const lrds_spec& s = a.s;
   const TcLayout TL = tc_layout(s.d, s.mlp.num_hidden, PREC);
   const int tid = threadIdx.x;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);  // warp-uniform for the compiler as well
   const bool has_aux = (int)(blockDim.x >> 5) > nwarps;
-  uint8_t* img = smem_raw;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + TL.bytes);  // [0] image, [1 + t] MMAs of tile t done
-  uint32_t* slot = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 48);
   uint32_t* cnts = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + TC_TAIL_BYTES);  // [t] tile hand-offs, [4 + i] step buffer i released
   uint8_t* stage = smem_raw + TL.bytes + TC_TAIL_BYTES + MIX_TAIL_BYTES;
   const StageLayout SL = stage_layout(s, 2, true);
   float* cols = reinterpret_cast<float*>(stage + ((SL.total + 15u) & ~15u));
-  if (warp == 0) ptx::tmem_alloc(slot, tmem_cols);
-  if (tid == 0) {
-    uint64_t* sbar = reinterpret_cast<uint64_t*>(stage);
-    for (int i = 0; i < 5; ++i) ptx::mbar_init(bars + i, 1);
-    ptx::mbar_init(sbar, 1);
-    ptx::mbar_init(sbar + 1, 1);
-    for (int i = 0; i < 6; ++i) cnts[i] = 0u;
-    ptx::fence_mbar_init();
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  if (tid == 0) {  // drift weights staged once per CTA by the TMA engine; the static target mixture and steps 0, 1
-    ptx::mbar_expect_tx(bars, TL.bytes);
-    ptx::bulk_g2s(img, image, TL.bytes, bars);
-    uint64_t* sbar = reinterpret_cast<uint64_t*>(stage);
-    const uint32_t mix_off_t = SL.tgt_logc_bytes + SL.tgt_param_bytes;
-    const uint32_t mix_off_r = SL.row_bytes + SL.ref_logc_bytes + SL.ref_param_bytes;
-    const uint8_t* rmix_g = static_cast<const uint8_t*>(s.ref_t.mix_tc);
-    for (int k = 0; k < 2 && k < s.K; ++k) {
-      uint8_t* dst = stage + SL.off_buf + k * SL.buf_bytes;
-      ptx::mbar_expect_tx(sbar + k, SL.buf_bytes + (k == 0 ? SL.tgt_bytes : 0u));
-      if (k == 0 && SL.tgt_bytes) {  // a mixture target is staged whether or not the control uses its score (terminal cost)
-        stage_gmm(stage + SL.off_tgt, gmm_at(s.target.gmm, 0), SL.tgt_logc_bytes, SL.tgt_param_bytes, sbar);
-        ptx::bulk_g2s(stage + SL.off_tgt + mix_off_t, static_cast<const uint8_t*>(s.target.gmm.mix_tc), SL.tgt_mix_bytes, sbar);
-      }
-      stage_step(dst, s, SL, k, sbar + k);
-      if constexpr (RMIX) ptx::bulk_g2s(dst + mix_off_r, rmix_g + (int64_t)k * s.ref_t.step_stride_mix_tc, SL.ref_mix_bytes, sbar + k);
-    }
-  }
-  ptx::mbar_wait(bars, 0);
-  const uint32_t tmem = __shfl_sync(0xffffffffu, *slot, 0);
+  auto steps01 = [&]() {  // the static target mixture and steps 0, 1, staged with the drift weights
+    for (int k = 0; k < 2 && k < s.K; ++k) mix_load_step<RMIX>(s, SL, stage, k);
+  };
+  const uint32_t tmem = __shfl_sync(
+      0xffffffffu, tc_cta_begin(smem_raw, TL, image, tmem_cols, warp, 5, reinterpret_cast<uint64_t*>(stage), 2, cnts, 6, 0u, steps01), 0);
   const bool aux = warp == nwarps;              // the auxiliary issuer serves the partial last tile
   const int tile = aux ? (nwarps - 1) >> 2 : warp >> 2;
   const int tile_warps = min(4, nwarps - 4 * tile);
-  MixTc<PREC> mlp;
-  mlp.L = TL;
-  mlp.img = img;
-  mlp.img_s = ptx::smem_u32(img);
-  mlp.tm_tile = tmem + (uint32_t)(tile * TL.tile_cols);
-  mlp.tm_lane = mlp.tm_tile + ((uint32_t)((warp & 3) * 32) << 16);
-  mlp.bar = bars + 1 + tile;
-  mlp.phase = 0;
-  mlp.cnt = cnts + tile;
-  mlp.tile_warps = (uint32_t)tile_warps;
-  mlp.target = 0u;
-  mlp.hand = 0u;
   // even hand-offs: the tile's last warp; odd ones: the one before it (the same warp in a one-warp tile); none in a
   // partial tile served by the auxiliary warp
-  mlp.issue_mask = ((warp & 3) == tile_warps - 1 ? 1u : 0u) | ((warp & 3) == max(tile_warps - 2, 0) ? 2u : 0u);
-  if (has_aux && tile_warps < 4) mlp.issue_mask = 0u;
-  mlp.dp = s.mlp.d_pad;
+  uint32_t issue_mask = ((warp & 3) == tile_warps - 1 ? 1u : 0u) | ((warp & 3) == max(tile_warps - 2, 0) ? 2u : 0u);
+  if (has_aux && tile_warps < 4) issue_mask = 0u;
+  MixTc<PREC> mlp;
+  mlp.init(TL, smem_raw, tmem + (uint32_t)(tile * TL.tile_cols), warp, bars + 1 + tile, cnts + tile, (uint32_t)tile_warps, issue_mask,
+           s.mlp.d_pad);
 #ifdef LRDS_MIX_TIMING
   unsigned long long* tmw = reinterpret_cast<unsigned long long*>(cols + (size_t)col_layout(s, true).total * 32 * nwarps) + warp * 16;
   if ((tid & 31) < 16) tmw[tid & 31] = 0;
@@ -853,13 +758,10 @@ rollout_mix_kernel(const RolloutArgs a, const uint8_t* __restrict__ image, const
   if ((blockIdx.x == 0 || blockIdx.x == gridDim.x / 2) && (tid & 31) < 16)
     g_mix_timing[((blockIdx.x ? 1 : 0) * 16 + warp) * 16 + (tid & 31)] = tmw[tid & 31];
 #endif
-  (void)TMIX;
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 0) ptx::tmem_dealloc(tmem, tmem_cols);
+  tc_cta_end(warp, tmem, tmem_cols);
 }
 
-// Launch shape of the mix kernel: one CTA per SM, as few waves as possible, then as few idle lanes as possible.
+// Launch shape of the mix kernel: one CTA per SM, warps per CTA as plan_warps picks them.
 inline bool plan_rollout_mix(const lrds_spec& s, int smem_cap, int sms, TcPlan* out) {
   if (!mix_tc_applicable(s)) return false;
   const TcLayout TL = tc_layout(s.d, s.mlp.num_hidden, s.precision);
@@ -875,18 +777,21 @@ inline bool plan_rollout_mix(const lrds_spec& s, int smem_cap, int sms, TcPlan* 
   wmax = wmax < MIX_MAX_WARPS ? wmax : MIX_MAX_WARPS;
   wmax = wmax < 4 * (512 / TL.tile_cols) ? wmax : 4 * (512 / TL.tile_cols);
   const int need = (s.B + 31) / 32;
-  const int waves = (need + sms * wmax - 1) / (sms * wmax);
-  int w = (need + sms * waves - 1) / (sms * waves);
-  w = w < 1 ? 1 : (w > wmax ? wmax : w);
-  const int tiles = (w + 3) / 4;
-  uint32_t cols = 32;
-  while ((int)cols < tiles * TL.tile_cols) cols <<= 1;
+  const int w = plan_warps(need, sms, wmax);
   out->warps = w;
   out->grid = (need + w - 1) / w;
   out->staged = 2;
-  out->tmem_cols = cols;
+  out->tmem_cols = plan_tmem_cols((w + 3) / 4 * TL.tile_cols);
   out->smem = fixed + per_warp * w;
   return true;
+}
+
+template <class CFG>
+int launch_mix_cfg(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
+  // a partial last tile gets the auxiliary issuer warp when the CTA has room for it
+  const int aux = (p.warps % 4 != 0 && p.warps < MIX_MAX_WARPS) ? 1 : 0;
+  return launch_tc(rollout_mix_kernel<LRDS_PRECISION_F16X3, CFG>, "mixture tensor-core rollout", a, p, (p.warps + aux) * 32, st, err, n,
+                   p.tmem_cols, p.warps);
 }
 
 }  // namespace lrds

@@ -44,9 +44,7 @@ rollout_mix_small_kernel(const RolloutArgs a, const uint8_t* __restrict__ image)
   const int sub = warp >> 2;   // which of the particle's four threads
   const int ptid = tid & 127;  // particle within the tile = TMEM lane
   constexpr int NT = 128;
-  uint8_t* img = smem_raw;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + TL.bytes);  // [0] image, [1] MMAs of the tile done, [2] the logits of a step, [3] the first contraction chunk of every thread
-  uint32_t* slot = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 48);
   uint32_t* cnts = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + TC_TAIL_BYTES);  // [0] hand-offs, [4 + i] step buffer i released
   uint8_t* stage = smem_raw + TL.bytes + TC_TAIL_BYTES + MIX_TAIL_BYTES;
   const StageLayout SL = stage_layout(s, 2, true);
@@ -56,53 +54,15 @@ rollout_mix_small_kernel(const RolloutArgs a, const uint8_t* __restrict__ image)
   uint64_t* sbar = reinterpret_cast<uint64_t*>(stage);
   const uint32_t mix_off_t = SL.tgt_logc_bytes + SL.tgt_param_bytes;
   const uint32_t mix_off_r = SL.row_bytes + SL.ref_logc_bytes + SL.ref_param_bytes;
-  const uint8_t* rmix_g = static_cast<const uint8_t*>(s.ref_t.mix_tc);
-  auto load_step = [&](int k) {
-    uint8_t* dst = stage + SL.off_buf + (k & 1) * SL.buf_bytes;
-    ptx::mbar_expect_tx(sbar + (k & 1), SL.buf_bytes + (k == 0 ? SL.tgt_bytes : 0u));
-    if (k == 0) {
-      stage_gmm(stage + SL.off_tgt, gmm_at(s.target.gmm, 0), SL.tgt_logc_bytes, SL.tgt_param_bytes, sbar);
-      ptx::bulk_g2s(stage + SL.off_tgt + mix_off_t, static_cast<const uint8_t*>(s.target.gmm.mix_tc), SL.tgt_mix_bytes, sbar);
-    }
-    stage_step(dst, s, SL, k, sbar + (k & 1));
-    ptx::bulk_g2s(dst + mix_off_r, rmix_g + (int64_t)k * s.ref_t.step_stride_mix_tc, SL.ref_mix_bytes, sbar + (k & 1));
+  auto steps01 = [&]() {
+    mix_load_step<true>(s, SL, stage, 0);
+    if (K > 1) mix_load_step<true>(s, SL, stage, 1);
   };
-  if (warp == 0) ptx::tmem_alloc(slot, 512);
-  if (tid == 0) {
-    ptx::mbar_init(bars, 1);
-    ptx::mbar_init(bars + 1, 1);
-    ptx::mbar_init(bars + 2, 1);
-    ptx::mbar_init(bars + 3, 1);
-    ptx::mbar_init(sbar, 1);
-    ptx::mbar_init(sbar + 1, 1);
-    for (int i = 0; i < 6; ++i) cnts[i] = 0u;
-    ptx::fence_mbar_init();
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  if (tid == 0) {
-    ptx::mbar_expect_tx(bars, TL.bytes);
-    ptx::bulk_g2s(img, image, TL.bytes, bars);
-    load_step(0);
-    if (K > 1) load_step(1);
-  }
-  ptx::mbar_wait(bars, 0);
-  const uint32_t tmem = __shfl_sync(0xffffffffu, *slot, 0);
+  const uint32_t tmem =
+      __shfl_sync(0xffffffffu, tc_cta_begin(smem_raw, TL, image, 512u, warp, 4, sbar, 2, cnts, 6, 0u, steps01), 0);
   MixTc<PREC> mlp;
-  mlp.L = TL;
-  mlp.img = img;
-  mlp.img_s = ptx::smem_u32(img);
-  mlp.tm_tile = tmem;
-  mlp.tm_lane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-  mlp.bar = bars + 1;
-  mlp.phase = 0;
-  mlp.cnt = cnts;
-  mlp.tile_warps = 16u;
-  mlp.target = 0u;
-  mlp.hand = 0u;
-  mlp.issue_mask = (warp == 15 ? 1u : 0u) | (warp == 14 ? 2u : 0u);  // the threads without a mixture to evaluate have slack
-  mlp.dp = dp;
+  // hand-offs: the threads without a mixture to evaluate have slack
+  mlp.init(TL, smem_raw, tmem, warp, bars + 1, cnts, 16u, (warp == 15 ? 1u : 0u) | (warp == 14 ? 2u : 0u), dp);
   const int Mt = s.target.gmm.M;
   const uint32_t contr_bytes = gmm_mix_contr_bytes(Mt, dp), lg_part = gmm_mix_logit_part_bytes(Mt, dp);
   const uint32_t lg_tail_off = contr_bytes + 2u * lg_part;
@@ -147,7 +107,6 @@ rollout_mix_small_kernel(const RolloutArgs a, const uint8_t* __restrict__ image)
     const float gamma = rowp.ld1(LRDS_STEP_GAMMA);
     const float ust = *reinterpret_cast<const float*>(stage + SL.off_tgt + mix_off_t + contr_bytes - 16u);
     const float usr = *reinterpret_cast<const float*>(buf + mix_off_r + contr_bytes - 16u);
-    // x -> A operand: the 16-dim group `sub`
     if (16 * sub < TL.Kin) {
       float v[16];
 #pragma unroll
@@ -208,7 +167,7 @@ rollout_mix_small_kernel(const RolloutArgs a, const uint8_t* __restrict__ image)
       for (int i = 0; i < 16; ++i) r_p[i] = ok ? r_p[i] : p[i];
     }
     mlp.tm.mark(6);
-    const float* bh = reinterpret_cast<const float*>(img + TL.off_bhid);
+    const float* bh = reinterpret_cast<const float*>(smem_raw + TL.off_bhid);
     mlp.tm.mark(6);
     float z0[JC], z1[JC];  // the increments of this thread's first two chunks, drawn behind the hidden GEMMs
     const bool two = sub + MIXS_TP < nchunk;
@@ -219,10 +178,10 @@ rollout_mix_small_kernel(const RolloutArgs a, const uint8_t* __restrict__ image)
       }
       mlp.wait();  // l == 0: the first GEMM, issued behind the logits
       mlp.tm.mark(7);
-      if (l == 0) mlp.template epilogue_f16_16<false>(row + LRDS_STEP_BIAS1, 0, 16 * sub);
-      else mlp.template epilogue_f16_16<false>(bh + (l - 1) * C, l, 16 * sub);
-      if (l < TL.nh) mlp.arrive_issue([&]() { mlp.gemm(TL.off_hid + (uint32_t)(l * C * C * TL.es), C, C); });
-      else mlp.arrive_issue([&]() { mlp.gemm(TL.off_out, C, TL.Nout); });
+      if (l == 0) mlp.template epilogue_f16<false, 16>(row + LRDS_STEP_BIAS1, 0, 16 * sub, 16 * sub + 16);
+      else mlp.template epilogue_f16<false, 16>(bh + (l - 1) * C, l, 16 * sub, 16 * sub + 16);
+      if (l < TL.nh) mlp.issue(TL.off_hid + (uint32_t)(l * C * C * TL.es), C, C);
+      else mlp.issue(TL.off_out, C, TL.Nout);
       mlp.tm.mark(8);
     }
     if (TL.nh < 1) noise_chunk(a, k, b, sub * JC, z0);  // (fewer hidden GEMMs than chunks per thread: draw what is left now)
@@ -301,7 +260,7 @@ rollout_mix_small_kernel(const RolloutArgs a, const uint8_t* __restrict__ image)
     __syncwarp();
     if ((tid & 31) == 0) {  // the CTA's last warp to finish the step refills its buffer with the operands of step k + 2
       const uint32_t old = ptx::atom_add_acq_rel(cnts + 4 + (k & 1), 1u);
-      if (old == (uint32_t)((k >> 1) * 16 + 15) && k + 2 < K) load_step(k + 2);
+      if (old == (uint32_t)((k >> 1) * 16 + 15) && k + 2 < K) mix_load_step<true>(s, SL, stage, k + 2);
     }
     mlp.tm.mark(12);
   }
@@ -333,9 +292,7 @@ rollout_mix_small_kernel(const RolloutArgs a, const uint8_t* __restrict__ image)
     nonfinite = !isfinite(rnd + xsum);  // (a non-finite coordinate reaches rnd through the terminal log-densities)
   }
   report_status(s, live, mlp.saturated(), nonfinite);
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 0) ptx::tmem_dealloc(tmem, 512);
+  tc_cta_end(warp, tmem, 512u);
 }
 
 // one CTA per tile of 128 particles; shared memory: [weight image | barriers | counters | operand stage | x columns | partial sums]

@@ -20,6 +20,8 @@
 #pragma once
 #include <cuda_fp16.h>
 
+#include <cstdio>
+
 #include "lrds_rollout_simt.cuh"
 #include "lrds_tc_ptx.cuh"
 
@@ -138,6 +140,63 @@ static __global__ void pack_tc_image_kernel(const lrds_mlp w, const TcLayout L, 
     bo[i] = i < w.d_pad ? w.b_out[i] : 0.f;
 }
 
+// ---- the tile protocol ----------------------------------------------------------------------------------------------
+// D[dcol] (+)= A . B on the tensor core: A in TMEM (hi at a_hi, lo at a_lo, a_step columns per K step), B in shared
+// memory (hi image at b, lo image at b + b_part, b_step bytes per K step, K-major descriptors with strides lbo / sbo).
+// X3: three passes of (hi, lo) products, small terms first (lo.hi, hi.lo, hi.hi); otherwise the single hi.hi pass.
+// UNROLL unrolls the pass loop: the issuer's instruction stream of the throughput kernels is on their critical path.
+template <bool X3, bool UNROLL, bool TF32 = false>
+__device__ __forceinline__ void mma_passes(uint32_t dcol, uint32_t a_hi, uint32_t a_lo, uint32_t a_step, uint32_t b, uint32_t b_part,
+                                           uint32_t b_step, uint32_t lbo, uint32_t sbo, int ksteps, uint32_t idesc) {
+  uint32_t acc = 0;
+#pragma unroll(UNROLL ? 3 : 1)
+  for (int pass = X3 ? 0 : 2; pass < 3; ++pass) {
+    const uint32_t a = pass == 0 ? a_lo : a_hi;
+    const uint32_t bb = b + (pass == 1 ? b_part : 0u);
+    for (int ks = 0; ks < ksteps; ++ks) {
+      const uint64_t bdesc = ptx::make_smem_desc(bb + (uint32_t)ks * b_step, lbo, sbo);
+      if (TF32) ptx::mma_tf32_ts(dcol, a + (uint32_t)ks * a_step, bdesc, idesc, acc);
+      else ptx::mma_bf16_ts(dcol, a + (uint32_t)ks * a_step, bdesc, idesc, acc);  // kind::f16 (bf16 or fp16 per idesc)
+      acc = 1;
+    }
+  }
+}
+
+// CTA prologue of the tensor-core kernels.  Warp 0 allocates `tmem_cols` TMEM columns; thread 0 initialises the nbars
+// mbarriers behind the weight image and nsbar more at `sbar` (one arrival each) and zeroes the ncnt hand-off counters
+// at `cnts`.  After the fences and the CTA barrier thread 0 stages the weight image on bars[0], which also expects
+// `extra_bytes` of the kernel's own bulk copies, issued by extra().  Returns the TMEM address once bars[0] completes.
+template <class F>
+__device__ __forceinline__ uint32_t tc_cta_begin(uint8_t* smem, const TcLayout& TL, const uint8_t* image, uint32_t tmem_cols,
+                                                  int warp, int nbars, uint64_t* sbar, int nsbar, uint32_t* cnts, int ncnt,
+                                                  uint32_t extra_bytes, F&& extra) {
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + TL.bytes);
+  uint32_t* slot = reinterpret_cast<uint32_t*>(smem + TL.bytes + 48);
+  if (warp == 0) ptx::tmem_alloc(slot, tmem_cols);
+  if (threadIdx.x == 0) {
+    for (int i = 0; i < nbars; ++i) ptx::mbar_init(bars + i, 1);
+    for (int i = 0; i < nsbar; ++i) ptx::mbar_init(sbar + i, 1);
+    for (int i = 0; i < ncnt; ++i) cnts[i] = 0u;
+    ptx::fence_mbar_init();
+  }
+  ptx::tc_fence_before();
+  __syncthreads();
+  ptx::tc_fence_after();
+  if (threadIdx.x == 0) {  // drift weights staged once per CTA by the TMA engine
+    ptx::mbar_expect_tx(bars, TL.bytes + extra_bytes);
+    ptx::bulk_g2s(smem, image, TL.bytes, bars);
+    extra();
+  }
+  ptx::mbar_wait(bars, 0);
+  return *slot;
+}
+// CTA epilogue: every warp is done with the tensor memory, warp 0 frees it
+__device__ __forceinline__ void tc_cta_end(int warp, uint32_t tmem, uint32_t tmem_cols) {
+  ptx::tc_fence_before();
+  __syncthreads();
+  if (warp == 0) ptx::tmem_dealloc(tmem, tmem_cols);
+}
+
 // ---- the policy --------------------------------------------------------------------------------------------------
 template <int PREC>
 struct TcMlp {
@@ -146,20 +205,39 @@ struct TcMlp {
   static constexpr bool kF16 = PREC == LRDS_PRECISION_F16X3;
   static constexpr bool kPipe = tc_max_warps(PREC) <= 8;  // 255-register kernels prefetch their mixture operands
   TcLayout L;
-  const uint8_t* img;  // weight image in shared memory
-  uint32_t img_s;      // its shared-window address
-  uint32_t tm_tile;    // TMEM address of the tile's column 0 at lane 0 (MMA operands)
-  uint32_t tm_lane;    // the same at this warp's first lane (tcgen05.ld / st)
-  uint64_t* bar;       // the tile's MMA-completion mbarrier
+  const uint8_t* img;   // weight image in shared memory
+  uint32_t img_s;       // its shared-window address
+  uint32_t tm_tile;     // TMEM address of the tile's column 0 at lane 0 (MMA operands)
+  uint32_t tm_lane;     // the same at this warp's first lane (tcgen05.ld / st)
+  uint64_t* bar;        // the tile's MMA-completion mbarrier
   uint32_t phase;
-  int bar_id, bar_threads;  // (named barrier of the tile: only the kernels' own barriers use it now)
-  bool issuer;              // this WARP issues the tile's batches (warp-uniform)
-  uint32_t* hand_cnt;       // the tile's hand-off counter: one increment per warp and hand-off
-  uint32_t hand_target = 0; // its value once every warp of the tile has arrived for the current hand-off
-  uint32_t hand_warps;      // warps that take part in a hand-off
-  int dp;              // columns of x held by the body (d rounded up to 8, zero padded)
+  uint32_t* cnt;        // the tile's hand-off counter: one increment per warp and hand-off
+  uint32_t target;      // its value once every warp of the tile has arrived for the current hand-off
+  uint32_t tile_warps;  // warps that take part in a hand-off
+  uint32_t issue_mask;  // bit (n & 1): this warp issues the tile's hand-offs n with that parity (warp-uniform)
+  uint32_t hand;        // hand-offs so far
+  int dp;               // columns of x held by the body (d rounded up to 8, zero padded)
   float vmax = 0.f, xmax = 0.f;  // F16X3: largest hidden pre-activation / |coordinate| this thread has converted to fp16
   __device__ __forceinline__ bool saturated() const { return kF16 && (vmax > F16X3_MAX_PREACT || xmax > F16X3_MAX_COORD); }
+
+  // The tile's fields: TMEM address of its column 0, this warp, the tile's MMA mbarrier and hand-off counter, the
+  // warps that take part in a hand-off and the hand-offs this warp issues (issue_mask)
+  __device__ __forceinline__ void init(const TcLayout& TL, const uint8_t* smem, uint32_t tmem_tile, int warp, uint64_t* tile_bar,
+                                       uint32_t* tile_cnt, uint32_t warps, uint32_t mask, int d_pad) {
+    L = TL;
+    img = smem;
+    img_s = ptx::smem_u32(smem);
+    tm_tile = tmem_tile;
+    tm_lane = tmem_tile + ((uint32_t)((warp & 3) * 32) << 16);
+    bar = tile_bar;
+    phase = 0;
+    cnt = tile_cnt;
+    target = 0u;
+    tile_warps = warps;
+    issue_mask = mask;
+    hand = 0u;
+    dp = d_pad;
+  }
 
   // (hi, lo) operand bits of an activation.  The 3-pass splits truncate (one LOP3): hi = the top 11 significand bits,
   // lo = v - hi is exact in fp32; the tf32 tensor core drops lo's bits below tf32 itself, the fp16 conversion rounds
@@ -174,53 +252,49 @@ struct TcMlp {
     return reinterpret_cast<const float*>(img + L.off_scale)[8 + layer];
   }
 
-  // This warp's operand rows are stored / its accumulator rows read: increment the tile's counter (release, no round
-  // trip) and go on; returns true in the tile's issuer warp once every warp of the tile has arrived (it polls the
-  // counter): the caller then issues the batch under elect.sync and commits it to the tile's mbarrier.  Nobody else
-  // blocks here - the warps wait for the batch on the mbarrier when they need its result (the named barrier that
-  // round 1 had in front of every batch cost 6 - 11 % of the warps' time in the two-threads-per-particle kernels).
-  __device__ __forceinline__ bool handoff() {
+  // This warp's part of the tile's next batch is in place (A rows stored / accumulator rows read).  Every warp
+  // increments the tile's counter (release, no round trip) and goes on; the hand-off's issuer warp polls the counter,
+  // issues the batch `f` from warp-uniform registers and commits it to the tile's mbarrier.  Nobody else blocks here:
+  // the warps wait for the batch on the mbarrier when they need its result.  Which warps issue is the kernel's choice
+  // (issue_mask): the throughput kernels let the warps of the least loaded SM sub-partitions take turns.
+  // `done` = the mbarrier the batch commits to (default: the tile's; a batch that completes while the tile already
+  // works on the next one needs its own, or the tile's barrier would run two phases ahead of a waiter)
+  template <class F>
+  __device__ __forceinline__ void arrive_issue(F&& f, uint64_t* done = nullptr) {
     ptx::tmem_wait_st();
     ptx::tc_fence_before();
     __syncwarp();
-    hand_target += hand_warps;
-    if ((threadIdx.x & 31) == 0) ptx::red_add_release(hand_cnt, 1u);
-    if (!issuer) return false;
-    while ((int32_t)(ptx::ld_acquire(hand_cnt) - hand_target) < 0) {
+    if ((threadIdx.x & 31) == 0) ptx::red_add_release(cnt, 1u);
+    const bool mine = (issue_mask >> (hand & 1u)) & 1u;
+    ++hand;
+    if (mine) issue_when_ready(f, done);
+    else target += tile_warps;
+  }
+  // polls the tile's counter until every warp has arrived for the next hand-off, then issues and commits its batch
+  template <class F>
+  __device__ __forceinline__ void issue_when_ready(F&& f, uint64_t* done = nullptr) {
+    target += tile_warps;
+    while ((int32_t)(ptx::ld_acquire(cnt) - target) < 0) {
     }
     ptx::tc_fence_after();
-    return true;
+    if (ptx::elect_one()) {
+      f();
+      ptx::mma_commit(done ? done : bar);
+    }
+    __syncwarp();
   }
 
-  // one layer's MMAs, issued by the tile's issuer warp and committed to the tile's mbarrier
+  // one layer of the network: D = A . W^T
+  __device__ __forceinline__ void gemm(uint32_t b_off, int K, int N) const {
+    const uint32_t idesc = PREC == LRDS_PRECISION_BF16 ? ptx::make_idesc_bf16(128, N)
+                           : kF16                      ? ptx::make_idesc_f16(128, N)
+                                                       : ptx::make_idesc_tf32(128, N);
+    mma_passes<kX3, true, !kHalf>(tm_tile + d_col(), tm_tile + a_col(0), tm_tile + a_col(1), 8u, img_s + b_off, L.part_bytes,
+                                  2u * (uint32_t)N * 16u, (uint32_t)N * 16u, 128u, K / L.kstep, idesc);  // two 16-byte K chunks per MMA
+  }
+  // the same at the tile's next hand-off
   __device__ __forceinline__ void issue(uint32_t b_off, int K, int N) {
-    const bool mine = handoff();
-    if (mine && ptx::elect_one()) {
-      const uint32_t idesc = PREC == LRDS_PRECISION_BF16 ? ptx::make_idesc_bf16(128, N)
-                             : kF16                      ? ptx::make_idesc_f16(128, N)
-                                                         : ptx::make_idesc_tf32(128, N);
-      const uint32_t dcol = tm_tile + d_col();
-      const int ksteps = K / L.kstep;
-      const uint32_t kbytes = 2u * (uint32_t)N * 16u;  // one MMA consumes two 16-byte K chunks
-      uint32_t acc = 0;
-      auto pass = [&](int a_part, int b_part) {
-        const uint32_t abase = tm_tile + a_col(a_part);
-        const uint32_t bbase = img_s + (uint32_t)b_part * L.part_bytes + b_off;
-        for (int ks = 0; ks < ksteps; ++ks) {
-          const uint64_t bdesc = ptx::make_smem_desc(bbase + (uint32_t)ks * kbytes, (uint32_t)N * 16u, 128u);
-          if (kHalf) ptx::mma_bf16_ts(dcol, abase + ks * 8, bdesc, idesc, acc);  // kind::f16 (bf16 or fp16 per idesc)
-          else ptx::mma_tf32_ts(dcol, abase + ks * 8, bdesc, idesc, acc);
-          acc = 1;
-        }
-      };
-      if (kX3) {  // small terms first
-        pass(1, 0);
-        pass(0, 1);
-      }
-      pass(0, 0);
-      ptx::mma_commit(bar);
-    }
-    if (mine) __syncwarp();
+    arrive_issue([&]() { gemm(b_off, K, N); });
   }
   __device__ __forceinline__ void wait() {
     ptx::mbar_wait(bar, phase);
@@ -266,9 +340,11 @@ struct TcMlp {
     }
   }
 
-  __device__ __forceinline__ void store_x(const Col4& x) {
+  // A operand <- x: this thread's groups g0, g0 + gstep, ... of 8 columns (16 dims packed in the 16-bit kinds, 8 dims in
+  // the tf32 kinds, where Kin == dp); the default stores all of x
+  __device__ __forceinline__ void store_x(const Col4& x, int g0 = 0, int gstep = 1) {
     if (kHalf) {
-      for (int c0 = 0; c0 < L.Kin / 2; c0 += 8) {  // 16 dims -> 8 packed columns
+      for (int c0 = 8 * g0; c0 < L.Kin / 2; c0 += 8 * gstep) {
         float v[16];
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
@@ -284,7 +360,7 @@ struct TcMlp {
         store16_half(c0, v);
       }
     } else {
-      for (int c0 = 0; c0 < L.Kin; c0 += 8) {  // Kin == dp for the tf32 kinds
+      for (int c0 = 8 * g0; c0 < L.Kin; c0 += 8 * gstep) {
         const float4 a = x.ld4(c0 >> 2), b = x.ld4((c0 >> 2) + 1);
         const float v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
         store8(c0, v);
@@ -292,19 +368,22 @@ struct TcMlp {
     }
   }
 
-  // F16X3: the whole epilogue on packed fp32x2 arithmetic
-  template <bool GLOBAL_BIAS>
+  // F16X3: accumulator columns [c_begin, c_end), W (32 or 16) at a time, * un-scale + bias -> GELU -> A operand of the
+  // next layer, on packed fp32x2 arithmetic
+  template <bool GLOBAL_BIAS, int W = 32>
   __device__ __forceinline__ void epilogue_f16(const float* __restrict__ bias, int layer, int c_begin = 0, int c_end = C) {
+    static_assert(W == 32 || W == 16, "tcgen05.ld / st widths");
     const u64 us2 = f2::pk(unscale(layer));
 #pragma unroll 1
-    for (int c0 = c_begin; c0 < c_end; c0 += 32) {
-      uint32_t r[32];
-      ptx::tmem_ld32(tm_lane + d_col() + c0, r);
+    for (int c0 = c_begin; c0 < c_end; c0 += W) {
+      uint32_t r[W];
+      if constexpr (W == 32) ptx::tmem_ld32(tm_lane + d_col() + c0, r);
+      else ptx::tmem_ld16(tm_lane + d_col() + c0, r);
       ptx::tmem_wait_ld();
       const float4* b4 = reinterpret_cast<const float4*>(bias + c0);  // warp-uniform, 16-byte aligned
-      uint32_t ph[16], pl[16];
+      uint32_t ph[W / 2], pl[W / 2];
 #pragma unroll
-      for (int i = 0; i < 8; ++i) {
+      for (int i = 0; i < W / 4; ++i) {
         const float4 b = GLOBAL_BIAS ? __ldg(b4 + i) : b4[i];
 #pragma unroll
         for (int e = 0; e < 2; ++e) {
@@ -325,44 +404,14 @@ struct TcMlp {
           pl[2 * i + e] = ptx::pack_f16x2(l0, l1);
         }
       }
-      ptx::tmem_st16(tm_lane + a_col(0) + c0 / 2, ph);
-      ptx::tmem_st16(tm_lane + a_col(1) + c0 / 2, pl);
-    }
-  }
-
-  // the same for 16 accumulator columns [c0, c0 + 16) (four threads per particle, lrds_rollout_mix_small.cuh)
-  template <bool GLOBAL_BIAS>
-  __device__ __forceinline__ void epilogue_f16_16(const float* __restrict__ bias, int layer, int c0) {
-    const u64 us2 = f2::pk(unscale(layer));
-    uint32_t r[16];
-    ptx::tmem_ld16(tm_lane + d_col() + c0, r);
-    ptx::tmem_wait_ld();
-    const float4* b4 = reinterpret_cast<const float4*>(bias + c0);
-    uint32_t ph[8], pl[8];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const float4 b = GLOBAL_BIAS ? __ldg(b4 + i) : b4[i];
-#pragma unroll
-      for (int e = 0; e < 2; ++e) {
-        const u64 acc = f2::pack(__uint_as_float(r[4 * i + 2 * e]), __uint_as_float(r[4 * i + 2 * e + 1]));
-        const u64 v = f2::fma(acc, us2, e ? f2::pack(b.z, b.w) : f2::pack(b.x, b.y));
-        {
-          float va, vb;
-          f2::unpack(v, va, vb);
-          vmax = max3(vmax, va, vb);
-        }
-        const u64 g = gelu_pair(v, 5.0f, TC_ACT_SCALE);
-        u64 hi, lo;
-        f2::split(g, hi, lo);
-        float h0, h1, l0, l1;
-        f2::unpack(hi, h0, h1);
-        f2::unpack(lo, l0, l1);
-        ph[2 * i + e] = ptx::pack_f16x2(h0, h1);
-        pl[2 * i + e] = ptx::pack_f16x2(l0, l1);
+      if constexpr (W == 32) {
+        ptx::tmem_st16(tm_lane + a_col(0) + c0 / 2, ph);
+        ptx::tmem_st16(tm_lane + a_col(1) + c0 / 2, pl);
+      } else {
+        ptx::tmem_st8(tm_lane + a_col(0) + c0 / 2, ph);
+        ptx::tmem_st8(tm_lane + a_col(1) + c0 / 2, pl);
       }
     }
-    ptx::tmem_st8(tm_lane + a_col(0) + c0 / 2, ph);
-    ptx::tmem_st8(tm_lane + a_col(1) + c0 / 2, pl);
   }
 
   // accumulator (64 columns) [* un-scale] + bias -> GELU -> A operand of the next layer
@@ -370,43 +419,36 @@ struct TcMlp {
   __device__ __forceinline__ void epilogue(const float* __restrict__ bias, int layer) {
     if constexpr (kF16) {
       epilogue_f16<GLOBAL_BIAS>(bias, layer);
-      return;
-    }
-    const float us = kF16 ? unscale(layer) : 1.0f;
-    const float gs = kF16 ? 0.5f * TC_ACT_SCALE : 0.5f;
+    } else {
 #pragma unroll 1
-    for (int c0 = 0; c0 < C; c0 += 32) {
-      uint32_t r[32];
-      ptx::tmem_ld32(tm_lane + d_col() + c0, r);
-      ptx::tmem_wait_ld();
-      float g[32];
-      const float4* b4 = reinterpret_cast<const float4*>(bias + c0);  // warp-uniform, 16-byte aligned
+      for (int c0 = 0; c0 < C; c0 += 32) {
+        uint32_t r[32];
+        ptx::tmem_ld32(tm_lane + d_col() + c0, r);
+        ptx::tmem_wait_ld();
+        float g[32];
+        const float4* b4 = reinterpret_cast<const float4*>(bias + c0);  // warp-uniform, 16-byte aligned
 #pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const float4 b = GLOBAL_BIAS ? __ldg(b4 + i) : b4[i];
-        if (kF16) {
-          gelu_exact2(fmaf(__uint_as_float(r[4 * i + 0]), us, b.x), fmaf(__uint_as_float(r[4 * i + 1]), us, b.y), g[4 * i + 0], g[4 * i + 1], gs);
-          gelu_exact2(fmaf(__uint_as_float(r[4 * i + 2]), us, b.z), fmaf(__uint_as_float(r[4 * i + 3]), us, b.w), g[4 * i + 2], g[4 * i + 3], gs);
-        } else {
+        for (int i = 0; i < 8; ++i) {
+          const float4 b = GLOBAL_BIAS ? __ldg(b4 + i) : b4[i];
           gelu_exact2(__uint_as_float(r[4 * i + 0]) + b.x, __uint_as_float(r[4 * i + 1]) + b.y, g[4 * i + 0], g[4 * i + 1]);
           gelu_exact2(__uint_as_float(r[4 * i + 2]) + b.z, __uint_as_float(r[4 * i + 3]) + b.w, g[4 * i + 2], g[4 * i + 3]);
         }
-      }
-      if (kHalf) {
-        float lo16[16], hi16[16];
+        if (kHalf) {
+          float lo16[16], hi16[16];
 #pragma unroll
-        for (int i = 0; i < 16; ++i) { lo16[i] = g[i]; hi16[i] = g[16 + i]; }
-        store16_half(c0 / 2, lo16);
-        store16_half(c0 / 2 + 8, hi16);
-      } else {
-        uint32_t hi[32];
+          for (int i = 0; i < 16; ++i) { lo16[i] = g[i]; hi16[i] = g[16 + i]; }
+          store16_half(c0 / 2, lo16);
+          store16_half(c0 / 2 + 8, hi16);
+        } else {
+          uint32_t hi[32];
 #pragma unroll
-        for (int i = 0; i < 32; ++i) hi[i] = split_hi(g[i]);
-        ptx::tmem_st32(tm_lane + a_col(0) + c0, hi);
-        if (kX3) {
+          for (int i = 0; i < 32; ++i) hi[i] = split_hi(g[i]);
+          ptx::tmem_st32(tm_lane + a_col(0) + c0, hi);
+          if (kX3) {
 #pragma unroll
-          for (int i = 0; i < 32; ++i) hi[i] = __float_as_uint(g[i] - __uint_as_float(hi[i]));
-          ptx::tmem_st32(tm_lane + a_col(1) + c0, hi);
+            for (int i = 0; i < 32; ++i) hi[i] = __float_as_uint(g[i] - __uint_as_float(hi[i]));
+            ptx::tmem_st32(tm_lane + a_col(1) + c0, hi);
+          }
         }
       }
     }
@@ -475,46 +517,19 @@ rollout_tc_kernel(const RolloutArgs a, const uint8_t* __restrict__ image, const 
   extern __shared__ __align__(128) uint8_t smem_raw[];
   const TcLayout TL = tc_layout(a.s.d, a.s.mlp.num_hidden, PREC);
   const int tid = threadIdx.x, warp = tid >> 5, nwarps = blockDim.x >> 5;
-  uint8_t* img = smem_raw;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + TL.bytes);  // [0] image, [1 + t] tile t
-  uint32_t* slot = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 48);
+  uint32_t* cnts = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 64);  // [t] hand-offs of tile t
   uint8_t* stage = smem_raw + TL.bytes + TC_TAIL_BYTES;
   float* cols = reinterpret_cast<float*>(stage + tc_stage_bytes(a.s, STAGE));
-  if (warp == 0) ptx::tmem_alloc(slot, tmem_cols);
-  if (tid == 0) {
-    for (int i = 0; i < 5; ++i) ptx::mbar_init(bars + i, 1);
-    for (int i = 0; i < 4; ++i) reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 64)[i] = 0u;
-    ptx::fence_mbar_init();
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  if (tid == 0) {  // drift weights staged once per CTA by the TMA engine
-    ptx::mbar_expect_tx(bars, TL.bytes);
-    ptx::bulk_g2s(img, image, TL.bytes, bars);
-  }
-  ptx::mbar_wait(bars, 0);
-  const uint32_t tmem = *slot;
+  const uint32_t tmem = tc_cta_begin(smem_raw, TL, image, tmem_cols, warp, 5, nullptr, 0, cnts, 4, 0u, []() {});
   const int tile = warp >> 2;
   const int tile_warps = min(4, nwarps - 4 * tile);
   TcMlp<PREC> mlp;
-  mlp.L = TL;
-  mlp.img = img;
-  mlp.img_s = ptx::smem_u32(img);
-  mlp.tm_tile = tmem + (uint32_t)(tile * TL.tile_cols);
-  mlp.tm_lane = mlp.tm_tile + ((uint32_t)((warp & 3) * 32) << 16);
-  mlp.bar = bars + 1 + tile;
-  mlp.phase = 0;
-  mlp.bar_id = 1 + tile;
-  mlp.bar_threads = tile_warps * 32;
-  mlp.issuer = (warp & 3) == tile_warps - 1;  // the tile's last warp: its sub-partition carries the fewest warps
-  mlp.hand_cnt = reinterpret_cast<uint32_t*>(smem_raw + TL.bytes + 64) + tile;
-  mlp.hand_warps = (uint32_t)tile_warps;
-  mlp.dp = a.s.mlp.d_pad;
+  // the tile's last warp issues its batches: its sub-partition carries the fewest warps
+  mlp.init(TL, smem_raw, tmem + (uint32_t)(tile * TL.tile_cols), warp, bars + 1 + tile, cnts + tile, (uint32_t)tile_warps,
+           (warp & 3) == tile_warps - 1 ? 3u : 0u, a.s.mlp.d_pad);
   rollout_body<KIND, STAGE, TR>(a, cols, stage, mlp);
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 0) ptx::tmem_dealloc(tmem, tmem_cols);
+  tc_cta_end(warp, tmem, tmem_cols);
 }
 
 // ---- host side -------------------------------------------------------------------------------------------------------
@@ -524,7 +539,38 @@ struct TcPlan {
   size_t smem;
 };
 
-// Warps per CTA: as few waves as possible over the SMs (one CTA per SM), then as few idle lanes as possible.
+// Warps per CTA (one CTA per SM, at most wmax warps) for `need` particle warps: as few waves as possible over the
+// SMs, then as few idle lanes as possible
+inline int plan_warps(int need, int sms, int wmax) {
+  const int waves = (need + sms * wmax - 1) / (sms * wmax);
+  const int w = (need + sms * waves - 1) / (sms * waves);
+  return w < 1 ? 1 : (w > wmax ? wmax : w);
+}
+// TMEM columns to allocate for `cols` used ones: a power of two, at least 32
+inline uint32_t plan_tmem_cols(int cols) {
+  uint32_t c = 32;
+  while ((int)c < cols) c <<= 1;
+  return c;
+}
+
+// Launches a tensor-core rollout kernel (arguments: the rollout, the weight image, then `args`) with the plan's grid and
+// shared memory and `threads` threads per CTA; `what` names the kernel in the error message.
+template <class K, class... A>
+int launch_tc(K kernel, const char* what, const RolloutArgs& a, const TcPlan& p, int threads, cudaStream_t st, char* err, size_t n,
+              A... args) {
+  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
+  if (e == cudaSuccess) {
+    kernel<<<p.grid, threads, p.smem, st>>>(a, static_cast<const uint8_t*>(a.s.mlp.tc_image), args...);
+    e = cudaGetLastError();
+  }
+  if (e != cudaSuccess) {
+    snprintf(err, n, "%s launch (grid %d x %d threads, %zu B smem, %u TMEM cols): %s", what, p.grid, threads, p.smem,
+             p.tmem_cols, cudaGetErrorString(e));
+    return LRDS_ERR_CUDA;
+  }
+  return LRDS_OK;
+}
+
 // Operand staging (LINEAR kind) is used when its shared-memory cost does not reduce the warps per CTA.
 inline int plan_rollout_tc(const lrds_spec& s, int smem_cap, int sms, TcPlan* out, const char** why) {
   const TcLayout TL = tc_layout(s.d, s.mlp.num_hidden, s.precision);
@@ -535,35 +581,28 @@ inline int plan_rollout_tc(const lrds_spec& s, int smem_cap, int sms, TcPlan* ou
   if (fixed + per_warp > (size_t)smem_cap) { *why = "weight image + one warp of particle state exceed shared memory"; return LRDS_ERR_RESOURCES; }
   const int tmax = 512 / TL.tile_cols;
   const int need = (s.B + 31) / 32;
-  auto pick = [&](size_t extra, int* wmax_out) {
-    if (fixed + extra + per_warp > (size_t)smem_cap) { *wmax_out = 0; return 0; }
+  auto pick = [&](size_t extra) {
+    if (fixed + extra + per_warp > (size_t)smem_cap) return 0;
     int wmax = (int)(((size_t)smem_cap - fixed - extra) / per_warp);
     wmax = wmax < tc_max_warps(s.precision) ? wmax : tc_max_warps(s.precision);
     wmax = wmax < 4 * tmax ? wmax : 4 * tmax;
-    *wmax_out = wmax;
-    const int waves = (need + sms * wmax - 1) / (sms * wmax);
-    int w = (need + sms * waves - 1) / (sms * waves);
-    return w < 1 ? 1 : (w > wmax ? wmax : w);
+    return plan_warps(need, sms, wmax);
   };
-  int wm = 0;
-  const int w_plain = pick(0, &wm);
+  const int w_plain = pick(0);
   int level = 0, w = w_plain;
   size_t stage = 0;
   if (s.kind == LRDS_ROLLOUT_LINEAR) {
     for (int lv = 2; lv >= 1; --lv) {  // the deepest staging level that does not cost warps
       const size_t bytes = tc_stage_bytes(s, lv);
-      const int wl = pick(bytes, &wm);
+      const int wl = pick(bytes);
       if (wl >= w_plain) { level = lv; w = wl; stage = bytes; break; }
     }
   }
   const bool staged = level > 0;
-  const int tiles = (w + 3) / 4;
-  uint32_t cols = 32;
-  while ((int)cols < tiles * TL.tile_cols) cols <<= 1;
   out->warps = w;
   out->grid = (need + w - 1) / w;
   out->staged = level;
-  out->tmem_cols = cols;
+  out->tmem_cols = plan_tmem_cols((w + 3) / 4 * TL.tile_cols);
   out->smem = fixed + (staged ? stage : 0) + per_warp * w;
   return LRDS_OK;
 }

@@ -8,43 +8,18 @@
 namespace lrds {
 template int launch_prec<LRDS_PRECISION_F16X3>(const RolloutArgs&, const TcPlan&, cudaStream_t, char*, size_t);
 
-template <bool EM, bool PHI4>
-static int launch_lin_variant(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
-  auto kernel = rollout_lin_kernel<LRDS_PRECISION_F16X3, EM, PHI4>;
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
-  if (e == cudaSuccess) {
-    kernel<<<p.grid, p.warps * 32, p.smem, st>>>(a, static_cast<const uint8_t*>(a.s.mlp.tc_image), p.tmem_cols);
-    e = cudaGetLastError();
-  }
-  if (e != cudaSuccess) {
-    snprintf(err, n, "reference-free tensor-core rollout launch (grid %d x %d threads, %zu B smem, %u TMEM cols): %s", p.grid,
-             p.warps * 32, p.smem, p.tmem_cols, cudaGetErrorString(e));
-    return LRDS_ERR_CUDA;
-  }
-  return LRDS_OK;
-}
-
 int launch_lin_f16x3(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
   const bool em = a.s.update_form == LRDS_UPDATE_EM, phi4 = a.s.target.kind == LRDS_DISTR_PHI4;
-  if (em) return phi4 ? launch_lin_variant<true, true>(a, p, st, err, n) : launch_lin_variant<true, false>(a, p, st, err, n);
-  return phi4 ? launch_lin_variant<false, true>(a, p, st, err, n) : launch_lin_variant<false, false>(a, p, st, err, n);
+  auto kernel = em ? (phi4 ? rollout_lin_kernel<LRDS_PRECISION_F16X3, true, true> : rollout_lin_kernel<LRDS_PRECISION_F16X3, true, false>)
+                   : (phi4 ? rollout_lin_kernel<LRDS_PRECISION_F16X3, false, true> : rollout_lin_kernel<LRDS_PRECISION_F16X3, false, false>);
+  return launch_tc(kernel, "reference-free tensor-core rollout", a, p, p.warps * 32, st, err, n, p.tmem_cols);
 }
 
 int launch_cmcd_tc_f16x3(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
   auto kernel = a.s.kind == LRDS_ROLLOUT_EUBO_CMCD ? rollout_cmcd_tc_kernel<LRDS_PRECISION_F16X3, 1>
                 : a.s.kind == LRDS_ROLLOUT_LINEAR  ? rollout_cmcd_tc_kernel<LRDS_PRECISION_F16X3, 2>
                                                     : rollout_cmcd_tc_kernel<LRDS_PRECISION_F16X3, 0>;
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
-  if (e == cudaSuccess) {
-    kernel<<<p.grid, p.warps * 32, p.smem, st>>>(a, static_cast<const uint8_t*>(a.s.mlp.tc_image), p.tmem_cols);
-    e = cudaGetLastError();
-  }
-  if (e != cudaSuccess) {
-    snprintf(err, n, "CMCD tensor-core rollout launch (grid %d x %d threads, %zu B smem): %s", p.grid, p.warps * 32, p.smem,
-             cudaGetErrorString(e));
-    return LRDS_ERR_CUDA;
-  }
-  return LRDS_OK;
+  return launch_tc(kernel, "CMCD tensor-core rollout", a, p, p.warps * 32, st, err, n, p.tmem_cols);
 }
 
 }  // namespace lrds

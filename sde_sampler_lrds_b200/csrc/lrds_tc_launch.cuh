@@ -1,8 +1,6 @@
 // Launch of the tensor-core rollout for ONE precision (included by lrds_tc_<precision>.cu so that the precisions
 // compile in parallel): kernel selection by loop kind, staging level and compile-time traits.
 #pragma once
-#include <cstdio>
-
 #include "lrds_internal.h"
 #include "lrds_rollout_tc.cuh"
 
@@ -18,18 +16,7 @@ using TraitsDds = LinearTraits<LRDS_UPDATE_AXPY, -1, LRDS_DISTR_PHI4, 1, 0, 0>;
 
 template <int KIND, int PREC, int STAGE, class TR>
 int launch_one(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
-  auto kernel = rollout_tc_kernel<KIND, PREC, STAGE, TR>;
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
-  if (e == cudaSuccess) {
-    kernel<<<p.grid, p.warps * 32, p.smem, st>>>(a, static_cast<const uint8_t*>(a.s.mlp.tc_image), p.tmem_cols);
-    e = cudaGetLastError();
-  }
-  if (e != cudaSuccess) {
-    snprintf(err, n, "tensor-core rollout launch (grid %d x %d threads, %zu B smem, %u TMEM cols): %s", p.grid,
-             p.warps * 32, p.smem, p.tmem_cols, cudaGetErrorString(e));
-    return LRDS_ERR_CUDA;
-  }
-  return LRDS_OK;
+  return launch_tc(rollout_tc_kernel<KIND, PREC, STAGE, TR>, "tensor-core rollout", a, p, p.warps * 32, st, err, n, p.tmem_cols);
 }
 
 template <int PREC, int STAGE>

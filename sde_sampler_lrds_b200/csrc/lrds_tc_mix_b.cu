@@ -1,29 +1,9 @@
 // The mixture tensor-core kernel (lrds_rollout_mix.cuh): lattice target / ClippedCtrl / Euler-Maruyama with a mixture reference (own translation unit: the
 // configurations compile in parallel).
-#include <cstdio>
-
 #include "lrds_internal.h"
 #include "lrds_rollout_mix.cuh"
 
 namespace lrds {
-
-template <class CFG>
-static int launch_mix_cfg(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
-  auto kernel = rollout_mix_kernel<LRDS_PRECISION_F16X3, CFG>;
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
-  if (e == cudaSuccess) {
-    // a partial last tile gets the auxiliary issuer warp (lrds_rollout_mix.cuh) when the CTA has room for it
-    const int aux = (p.warps % 4 != 0 && p.warps < MIX_MAX_WARPS) ? 1 : 0;
-    kernel<<<p.grid, (p.warps + aux) * 32, p.smem, st>>>(a, static_cast<const uint8_t*>(a.s.mlp.tc_image), p.tmem_cols, p.warps);
-    e = cudaGetLastError();
-  }
-  if (e != cudaSuccess) {
-    snprintf(err, n, "mixture tensor-core rollout launch (grid %d x %d threads, %zu B smem, %u TMEM cols): %s", p.grid,
-             p.warps * 32, p.smem, p.tmem_cols, cudaGetErrorString(e));
-    return LRDS_ERR_CUDA;
-  }
-  return LRDS_OK;
-}
 
 int launch_mix_b(int cfg, const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
   switch (cfg) {

@@ -1,6 +1,4 @@
 // The small-batch variant of the mixture tensor-core kernel (lrds_rollout_mix_small.cuh), own translation unit.
-#include <cstdio>
-
 #include "lrds_internal.h"
 #include "lrds_rollout_cmcd_mix.cuh"
 #include "lrds_rollout_mix_small.cuh"
@@ -8,33 +6,11 @@
 namespace lrds {
 
 int launch_mix_small_f16x3(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
-  auto kernel = rollout_mix_small_kernel<LRDS_PRECISION_F16X3>;
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
-  if (e == cudaSuccess) {
-    kernel<<<p.grid, p.warps * 32, p.smem, st>>>(a, static_cast<const uint8_t*>(a.s.mlp.tc_image));
-    e = cudaGetLastError();
-  }
-  if (e != cudaSuccess) {
-    snprintf(err, n, "small-batch mixture rollout launch (grid %d x %d threads, %zu B smem): %s", p.grid, p.warps * 32, p.smem,
-             cudaGetErrorString(e));
-    return LRDS_ERR_CUDA;
-  }
-  return LRDS_OK;
+  return launch_tc(rollout_mix_small_kernel<LRDS_PRECISION_F16X3>, "small-batch mixture rollout", a, p, p.warps * 32, st, err, n);
 }
 
 int launch_cmcd_mix_f16x3(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
-  auto kernel = rollout_cmcd_mix_kernel<LRDS_PRECISION_F16X3>;
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
-  if (e == cudaSuccess) {
-    kernel<<<p.grid, p.warps * 32, p.smem, st>>>(a, static_cast<const uint8_t*>(a.s.mlp.tc_image), p.tmem_cols);
-    e = cudaGetLastError();
-  }
-  if (e != cudaSuccess) {
-    snprintf(err, n, "CMCD mixture rollout launch (grid %d x %d threads, %zu B smem, %u TMEM cols): %s", p.grid, p.warps * 32,
-             p.smem, p.tmem_cols, cudaGetErrorString(e));
-    return LRDS_ERR_CUDA;
-  }
-  return LRDS_OK;
+  return launch_tc(rollout_cmcd_mix_kernel<LRDS_PRECISION_F16X3>, "CMCD mixture rollout", a, p, p.warps * 32, st, err, n, p.tmem_cols);
 }
 }  // namespace lrds
 
