@@ -1,36 +1,62 @@
-// C ABI of liblrds_b200.so (declared in include/lrds_b200.h): argument validation, launch configuration and
-// the small auxiliary kernels (estimator partials, control / distribution evaluation, axpy step, RNG dump).
-#include <cuda_fp16.h>
+// C ABI of liblrds_b200.so (declared in include/lrds_b200.h): argument validation, launch configuration, the error
+// channel and launch counter shared by every translation unit, and the small auxiliary kernels (estimator partials,
+// control / distribution evaluation, MALA chains, score cotangent sums, operand-image packers, axpy step, RNG dump).
 #include <cuda_runtime.h>
 
 #include <atomic>
+#include <cstdarg>
 #include <cstdio>
 #include <cstring>
 
 #include "lrds_internal.h"
 #include "lrds_rollout_simt.cuh"
-#include "lrds_rollout_mix.cuh"  // gmm_pass1_pair: the quadratic forms of two particles per operand load
 
 namespace {
-
 thread_local char g_err[512] = "";
 std::atomic<int64_t> g_launches{0};
+}  // namespace
 
-int fail(int code, const char* fmt, const char* a = "", long v = 0) {
-  snprintf(g_err, sizeof(g_err), fmt, a, v);
+namespace lrds {
+
+int fail(int code, const char* fmt, ...) {
+  va_list ap;
+  va_start(ap, fmt);
+  vsnprintf(g_err, sizeof(g_err), fmt, ap);
+  va_end(ap);
   return code;
 }
 
-int cuda_fail(cudaError_t e, const char* what) {
-  snprintf(g_err, sizeof(g_err), "%s: %s", what, cudaGetErrorString(e));
+int cuda_fail(cudaError_t e, const char* fmt, ...) {
+  va_list ap;
+  va_start(ap, fmt);
+  const int n = vsnprintf(g_err, sizeof(g_err), fmt, ap);
+  va_end(ap);
+  if (n >= 0 && (size_t)n < sizeof(g_err)) snprintf(g_err + n, sizeof(g_err) - n, ": %s", cudaGetErrorString(e));
   return LRDS_ERR_CUDA;
 }
 
-int max_optin_smem() {
-  int dev = 0, v = 0;
+DeviceLimits device_limits() {
+  int dev = 0;
+  DeviceLimits l{0, 0};
   cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-  return v;
+  cudaDeviceGetAttribute(&l.smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+  cudaDeviceGetAttribute(&l.sms, cudaDevAttrMultiProcessorCount, dev);
+  if (l.sms <= 0) l.sms = 148;
+  return l;
+}
+
+}  // namespace lrds
+
+namespace {
+using lrds::cuda_fail;
+using lrds::fail;
+
+// the kernel launch just issued: its error as "<what> launch: ...", else n more launches counted
+int launched(const char* what, int n = 1) {
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return cuda_fail(e, "%s launch", what);
+  g_launches.fetch_add(n);
+  return LRDS_OK;
 }
 
 // threads per CTA for the column layout: as many as fit, preferring >= 2 CTAs per SM
@@ -41,6 +67,27 @@ int pick_threads(int floats_per_particle, int smem_cap) {
   for (int nt = 128; nt >= 32; nt -= 32)
     if (nt * per <= smem_cap) return nt;
   return 0;
+}
+
+// Launch of a kernel with one thread per particle and the spec's shared-memory columns (col_layout): `floats` more
+// shared-memory floats per thread, `bytes` more per CTA, at most `max_nt` threads per CTA, `slices` CTA rows (grid.y);
+// `launches` are counted when the launch succeeds.
+struct ColExtra {
+  int max_nt = 128, floats = 0;
+  uint32_t bytes = 0;
+  int slices = 1, launches = 1;
+};
+template <class K, class... A>
+int launch_cols(K kernel, const char* what, const lrds_spec& s, const ColExtra& x, cudaStream_t st, A... args) {
+  const int floats = lrds::col_layout(s).total + x.floats;
+  int nt = pick_threads(floats, lrds::device_limits().smem_optin - (int)x.bytes);
+  if (nt == 0) return fail(LRDS_ERR_RESOURCES, "per-particle state of %d floats does not fit in shared memory", floats);
+  nt = nt < x.max_nt ? nt : x.max_nt;
+  const size_t smem = (size_t)floats * nt * sizeof(float) + x.bytes;
+  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute");
+  kernel<<<dim3((s.B + nt - 1) / nt, x.slices), nt, smem, st>>>(args...);
+  return launched(what, x.launches);
 }
 
 int validate_gmm(const lrds_gmm& g, const char* name) {
@@ -62,7 +109,7 @@ int refuse_full(const lrds_gmm& g, const char* where) {
 
 int validate_spec(const lrds_spec* s, bool need_steps) {
   if (!s) return fail(LRDS_ERR_INVALID, "spec is NULL");
-  if (s->abi_version != LRDS_ABI_VERSION) return fail(LRDS_ERR_INVALID, "abi_version mismatch (got %s%ld)", "", s->abi_version);
+  if (s->abi_version != LRDS_ABI_VERSION) return fail(LRDS_ERR_INVALID, "abi_version mismatch (got %d)", s->abi_version);
   if (s->B < 1 || s->d < 1 || s->K < 0) return fail(LRDS_ERR_INVALID, "B, d must be positive and K non-negative");
   if (s->mlp.d != s->d || s->mlp.d_pad != ((s->d + 7) / 8) * 8) return fail(LRDS_ERR_INVALID, "mlp.d / d_pad inconsistent with d");
   if (!s->mlp.w_in_t || !s->mlp.w_out_t || !s->mlp.b_out || s->mlp.num_hidden < 0 ||
@@ -97,26 +144,6 @@ int validate_spec(const lrds_spec* s, bool need_steps) {
 constexpr int EST_THREADS = 256;
 constexpr int EST_PER_BLOCK = 8192;
 
-__device__ __forceinline__ double warp_sum(double v) {
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ double warp_max(double v) {
-  for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
-
-template <bool IS_MAX>
-__device__ double block_reduce(double v, double* sh) {
-  v = IS_MAX ? warp_max(v) : warp_sum(v);
-  __syncthreads();
-  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = v;
-  __syncthreads();
-  double r = IS_MAX ? -INFINITY : 0.0;
-  for (int w = 0; w < EST_THREADS / 32; ++w) r = IS_MAX ? fmax(r, sh[w]) : r + sh[w];
-  return r;
-}
-
 // merge of two partial records (max-shifted sums), associative and commutative
 __device__ void merge8(double* acc, const double* p) {
   if (p[5] == 0.0) return;
@@ -138,6 +165,9 @@ __device__ void merge8(double* acc, const double* p) {
 __global__ void __launch_bounds__(EST_THREADS) estimator_kernel(const float* __restrict__ rnd, int B,
                                                                 double* __restrict__ out, double* scratch,
                                                                 unsigned int* counter) {
+  using lrds::block_reduce;
+  const lrds::MaxOp mx_op{};
+  const lrds::SumOp sum{};
   __shared__ double sh[EST_THREADS / 32];
   __shared__ bool is_last;
   const int lo = blockIdx.x * EST_PER_BLOCK, hi = min(B, lo + EST_PER_BLOCK);
@@ -147,19 +177,19 @@ __global__ void __launch_bounds__(EST_THREADS) estimator_kernel(const float* __r
     mx = fmax(mx, -v);
     mn = fmax(mn, v);
   }
-  mx = block_reduce<true>(mx, sh);
-  mn = block_reduce<true>(mn, sh);
+  mx = block_reduce(mx, mx_op, -HUGE_VAL, sh);
+  mn = block_reduce(mn, mx_op, -HUGE_VAL, sh);
   double s1 = 0, s2 = 0, sr = 0, sr2 = 0, sf = 0;
   for (int i = lo + threadIdx.x; i < hi; i += EST_THREADS) {
     const double v = (double)rnd[i];
     const double e = exp(-v - mx);
     s1 += e; s2 += e * e; sr += v; sr2 += v * v; sf += exp(v - mn);
   }
-  s1 = block_reduce<false>(s1, sh);
-  s2 = block_reduce<false>(s2, sh);
-  sr = block_reduce<false>(sr, sh);
-  sr2 = block_reduce<false>(sr2, sh);
-  sf = block_reduce<false>(sf, sh);
+  s1 = block_reduce(s1, sum, 0.0, sh);
+  s2 = block_reduce(s2, sum, 0.0, sh);
+  sr = block_reduce(sr, sum, 0.0, sh);
+  sr2 = block_reduce(sr2, sum, 0.0, sh);
+  sf = block_reduce(sf, sum, 0.0, sh);
   if (threadIdx.x == 0) {
     double* p = scratch + 8 * blockIdx.x;
     p[0] = mx; p[1] = s1; p[2] = s2; p[3] = sr; p[4] = sr2; p[5] = (double)(hi - lo); p[6] = mn; p[7] = sf;
@@ -187,40 +217,10 @@ __global__ void estimator_merge_kernel(const double* __restrict__ parts, int n, 
 }
 
 // ---- packers of the tensor-core operand images (layouts in include/lrds_b200.h) --------------------------------------
-__device__ float block_max_256(float m, float* red) {
-  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-  __syncthreads();
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = m;
-  __syncthreads();
-  float r = 0.f;
-  for (int i = 0; i < (int)(blockDim.x >> 5); ++i) r = fmaxf(r, red[i]);
-  return r;
-}
-__device__ __forceinline__ void put_hi_lo(uint8_t* out, uint32_t part_bytes, uint32_t byte, float vs) {
-  const __half hi = __float2half_rn(vs);
-  *reinterpret_cast<__half*>(out + byte) = hi;
-  *reinterpret_cast<__half*>(out + part_bytes + byte) = __float2half_rn(vs - __half2float(hi));
-}
-__device__ __forceinline__ int pow2_exponent_for(float amax) {  // amax * 2^k in [2^14, 2^15)
-  int k = 0;
-  if (amax > 0.f && amax < INFINITY) k = 14 - ilogbf(amax);
-  return k > 100 ? 100 : (k < -100 ? -100 : k);
-}
-
-__device__ double block_sum_256(double v, double* red) {
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  __syncthreads();
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
-  __syncthreads();
-  double r = 0.0;
-  for (int i = 0; i < (int)(blockDim.x >> 5); ++i) r += red[i];
-  return r;
-}
-
 // one block per step
 __global__ void __launch_bounds__(256) pack_gmm_mix_kernel(const lrds_gmm g, int d, int d_pad, uint8_t* __restrict__ out) {
+  using namespace lrds;
   __shared__ float red[8];
-  __shared__ double redd[8];
   __shared__ float wbar[LRDS_MAX_DIM_PAD];
   __shared__ double cm[64];
   __shared__ float wn[64];
@@ -238,7 +238,7 @@ __global__ void __launch_bounds__(256) pack_gmm_mix_kernel(const lrds_gmm g, int
   };
   float amax = 0.f;
   for (int idx = threadIdx.x; idx < Mp * N2; idx += blockDim.x) amax = fmaxf(amax, fabsf(value(idx / N2, idx % N2)));
-  amax = block_max_256(amax, red);
+  amax = block_reduce(amax, MaxOp{}, 0.f, red);
   const int k = pow2_exponent_for(amax);
   const float sc = ldexpf(1.0f, k);
   for (int idx = threadIdx.x; idx < Mp * N2; idx += blockDim.x) {
@@ -260,14 +260,14 @@ __global__ void __launch_bounds__(256) pack_gmm_mix_kernel(const lrds_gmm g, int
       for (int m = 1; m < g.M; ++m)
         shared_dev = fmaxf(shared_dev, fabsf(iv[(int64_t)m * d_pad + j] - iv[j]) / fabsf(iv[j]));
   }
-  shared_dev = block_max_256(shared_dev, red);  // (contains the __syncthreads that publishes wbar)
+  shared_dev = block_reduce(shared_dev, MaxOp{}, 0.f, red);  // (contains the __syncthreads that publishes wbar)
   auto wc = [&](int m, int j) -> float {
     if (m >= g.M || j >= d) return 0.f;
     return (float)((double)mu[(int64_t)m * d_pad + j] * (double)iv[(int64_t)m * d_pad + j] - (double)wbar[j]);
   };
   float lmax = 0.f;
   for (int idx = threadIdx.x; idx < Mp * Kin; idx += blockDim.x) lmax = fmaxf(lmax, fabsf(wc(idx / Kin, idx % Kin)));
-  lmax = block_max_256(lmax, red);
+  lmax = block_reduce(lmax, MaxOp{}, 0.f, red);
   const int kl = pow2_exponent_for(lmax);
   const float scl = ldexpf(1.0f, kl);
   for (int idx = threadIdx.x; idx < Mp * Kin; idx += blockDim.x) {
@@ -310,10 +310,10 @@ __global__ void __launch_bounds__(256) pack_gmm_mix_kernel(const lrds_gmm g, int
     t2[2] = cmax;
     t2[3] = shared_dev <= 1e-6f ? 1.0f : 0.f;
   }
-  (void)redd;
 }
 
 __global__ void __launch_bounds__(256) pack_logreg_kernel(const lrds_logreg L, int d_pad, uint8_t* __restrict__ out) {
+  using namespace lrds;
   __shared__ float red[8];
   const int N16 = (L.N + 15) / 16 * 16, K16 = (L.p + 1 + 15) / 16 * 16;
   const uint32_t part_bytes = (uint32_t)N16 * (uint32_t)K16 * 2u;
@@ -323,7 +323,7 @@ __global__ void __launch_bounds__(256) pack_logreg_kernel(const lrds_logreg L, i
   };
   float amax = 0.f;
   for (int idx = threadIdx.x; idx < N16 * K16; idx += blockDim.x) amax = fmaxf(amax, fabsf(value(idx / K16, idx % K16)));
-  amax = block_max_256(amax, red);
+  amax = block_reduce(amax, MaxOp{}, 0.f, red);
   const int e = pow2_exponent_for(amax);
   const float sc = ldexpf(1.0f, e);
   for (int idx = threadIdx.x; idx < N16 * K16; idx += blockDim.x) {
@@ -340,14 +340,13 @@ __global__ void __launch_bounds__(128) ctrl_forward_kernel(const lrds_spec s, in
                                                            float* __restrict__ out) {
   using namespace lrds;
   extern __shared__ float smem[];
-  const int NT = blockDim.x, tid = threadIdx.x;
-  const int b_raw = blockIdx.x * NT + tid;
-  const bool live = b_raw < s.B;
-  const int b = live ? b_raw : s.B - 1;
-  const ColLayout L = col_layout(s);
-  const Particle P = make_particle(smem, L, NT, tid);
+  const ParticleThread t = particle_thread(s, smem);
+  const int b = t.b;
+  const bool live = t.live;
+  const Particle& P = t.P;
   const GmmView tv0 = gmm_at(s.target.gmm, 0);
-  SimtMlp mlp{s.mlp, Col{smem + L.act * NT + tid, NT}};
+  const int NT = blockDim.x;
+  SimtMlp mlp{s.mlp, Col{smem + col_layout(s).act * NT + (int)threadIdx.x, NT}};
   const int d = s.d, dp = s.mlp.d_pad;
   for (int j = 0; j < dp; ++j) P.x(j) = (j < d) ? __ldg(x + (int64_t)b * d + j) : 0.f;
   const float* row = s.steps + (int64_t)rowi * LRDS_STEP_STRIDE;
@@ -355,12 +354,9 @@ __global__ void __launch_bounds__(128) ctrl_forward_kernel(const lrds_spec s, in
   const CtrlConst cc = ctrl_const(s);
   if (score_ctrl) target_pass1<false>(s, s.target.kind, tv0, P, false);
   mlp.template hidden<false>(row + LRDS_STEP_BIAS1, P.x);
-  float xm = 0.f;
-  for (int j0 = 0; j0 < dp; j0 += JC) {
-    float xr[JC], ts[JC], u[JC];
-    load_chunk(P.x, j0, xr);
-    const float xp = (j0 + JC < dp) ? P.x(j0 + JC) : 0.f;
-    if (score_ctrl) target_score_chunk<false>(s, s.target.kind, tv0, P, xr, xm, xp, j0, ts);
+  const int kind = score_ctrl ? s.target.kind : LRDS_DISTR_NONE;  // ClippedCtrl reads no score (NONE: zeros)
+  target_score_loop<false>(s, kind, tv0, P, [&](int j0, const float(&xr)[JC], const float(&ts)[JC]) {
+    float u[JC];
     if (s.ctrl_kind >= LRDS_CTRL_CANCEL_DRIFT) {
       float ps[JC] = {};
       if (s.ctrl_kind == LRDS_CTRL_LERP) gmm_score_chunk<false, false>(gmm_at(s.ref_0, 0), d, dp, xr, P.rr, j0, ps);
@@ -368,24 +364,21 @@ __global__ void __launch_bounds__(128) ctrl_forward_kernel(const lrds_spec s, in
     } else {
       ctrl_chunk(cc, mlp, j0, ts, __ldg(row + LRDS_STEP_GAMMA), u);
     }
-    xm = xr[JC - 1];
     if (live)
 #pragma unroll
       for (int c = 0; c < JC; ++c)
         if (j0 + c < d) out[(int64_t)b * d + j0 + c] = u[c];
-  }
+  });
 }
 
 __global__ void __launch_bounds__(128) distr_eval_kernel(const lrds_spec s, const float* __restrict__ x,
                                                          float* __restrict__ logp_out, float* __restrict__ score_out) {
   using namespace lrds;
   extern __shared__ float smem[];
-  const int NT = blockDim.x, tid = threadIdx.x;
-  const int b_raw = blockIdx.x * NT + tid;
-  const bool live = b_raw < s.B;
-  const int b = live ? b_raw : s.B - 1;
-  const ColLayout L = col_layout(s);
-  const Particle P = make_particle(smem, L, NT, tid);
+  const ParticleThread t = particle_thread(s, smem);
+  const int b = t.b;
+  const bool live = t.live;
+  const Particle& P = t.P;
   const GmmView tv0 = gmm_at(s.target.gmm, 0);
   const int d = s.d, dp = s.mlp.d_pad;
   for (int j = 0; j < dp; ++j) P.x(j) = (j < d) ? __ldg(x + (int64_t)b * d + j) : 0.f;
@@ -400,7 +393,7 @@ __global__ void __launch_bounds__(128) distr_eval_kernel(const lrds_spec s, cons
   const float lp = target_pass1<false>(s, s.target.kind, tv0, P, logp_out != nullptr);
   if (live && logp_out) logp_out[b] = lp + s.rnd_offset;
   if (!score_out) return;
-  float xm = 0.f;
+  float xm = 0.f;  // target_score_loop written out: through the helper this kernel's register allocation changes
   for (int j0 = 0; j0 < dp; j0 += JC) {
     float xr[JC], ts[JC];
     load_chunk(P.x, j0, xr);
@@ -419,12 +412,7 @@ __global__ void __launch_bounds__(128) distr_eval_kernel(const lrds_spec s, cons
 // pass of train.py.  One thread per stored state; the products replace the staged cotangents in shared memory and the
 // block's columns are summed from there; every block writes its partial row (part[s][block][dp]) and score_cot_reduce_kernel adds them in a fixed order.
 // bytes of a mixture target staged in shared memory behind the particle columns (0: read from global memory)
-__host__ __device__ inline uint32_t score_cot_stage_bytes(const lrds_spec& s, uint32_t* logc_bytes) {
-  if (s.target.kind != LRDS_DISTR_GMM || s.target.gmm.M < 2) return *logc_bytes = 0u;
-  const int M = s.target.gmm.M;
-  *logc_bytes = (uint32_t)((M + 3) / 4 * 4) * 4u;
-  return *logc_bytes + (uint32_t)((M + 3) / 4) * (uint32_t)s.mlp.d_pad * 32u;
-}
+inline uint32_t score_cot_stage_bytes(const lrds_spec& s) { return lrds::stage_layout(s, 2).tgt_bytes; }
 
 template <bool SH>
 __device__ __forceinline__ void score_cot_body(const lrds_spec& s, const lrds::GmmViewT<SH>& tv, const lrds::Particle& P,
@@ -435,7 +423,7 @@ __device__ __forceinline__ void score_cot_body(const lrds_spec& s, const lrds::G
   const int d = s.d, dp = s.mlp.d_pad;
   float* mine = rows + tid * ld;  // this thread's row of the staged cotangents; the products replace them in place
   if (SH && s.target.kind == LRDS_DISTR_GMM && s.target.gmm.M <= MIX_MAX_M) {
-    // the responsibilities with every (1/sigma, -mu/sigma) vector serving two particles (lrds_rollout_mix.cuh): this
+    // the responsibilities with every (1/sigma, -mu/sigma) vector serving two particles (lrds_rollout_simt.cuh): this
     // kernel is bound by the shared-memory data pipe, not by the FMA pipe
     float r[MIX_MAX_M];
     gmm_pass1_pair(tv, d, dp, P.x, r);
@@ -446,7 +434,7 @@ __device__ __forceinline__ void score_cot_body(const lrds_spec& s, const lrds::G
   } else {
     target_pass1<SH>(s, s.target.kind, tv, P, false);
   }
-  float xm = 0.f;
+  float xm = 0.f;  // target_score_loop written out (particle_thread too): through the helpers this kernel runs longer code
   for (int j0 = 0; j0 < dp; j0 += JC) {
     float xr[JC], ts[JC];
     load_chunk(P.x, j0, xr);
@@ -491,8 +479,8 @@ __global__ void __launch_bounds__(128) score_cot_kernel(const lrds_spec s, const
   const GmmView tv0 = gmm_at(s.target.gmm, 0);
   const int d = s.d, dp = s.mlp.d_pad;
   const int warp = tid >> 5, lane = tid & 31, nw = NT >> 5;
-  uint32_t logc_bytes;
-  const uint32_t stage_bytes = score_cot_stage_bytes(s, &logc_bytes);
+  const StageLayout SL = stage_layout(s, 2);
+  const uint32_t stage_bytes = SL.tgt_bytes, logc_bytes = SL.tgt_logc_bytes;
   // The block's rows are contiguous in global memory: the warps read them row by row (coalesced) into a padded
   // row-major staging area and every thread then takes its own row from there (per-thread global reads of rows
   // 4 d bytes apart cost 32 wavefronts per load).
@@ -575,28 +563,20 @@ struct MalaArgs {
 __global__ void __launch_bounds__(128) mala_kernel(const lrds_spec s, const MalaArgs m) {
   using namespace lrds;
   extern __shared__ float smem[];
-  const int NT = blockDim.x, tid = threadIdx.x;
-  const int b_raw = blockIdx.x * NT + tid;
-  const bool live = b_raw < s.B;
-  const int b = live ? b_raw : s.B - 1;
-  const ColLayout L = col_layout(s);
-  const Particle P = make_particle(smem, L, NT, tid);
+  const ParticleThread t = particle_thread(s, smem);
+  const int b = t.b;
+  const bool live = t.live;
+  const Particle& P = t.P;
   const GmmView tv0 = gmm_at(s.target.gmm, 0);
   const int d = s.d, dp = s.mlp.d_pad, kind = s.target.kind;
   const RolloutArgs na{s, nullptr, m.noise, m.seed, 0, nullptr, nullptr, nullptr};
   // log-density and score at P.x; the score goes to column `out`
   auto eval = [&](const Col& out) -> float {
     const float lp = target_pass1<false>(s, kind, tv0, P, true);
-    float xm = 0.f;
-    for (int j0 = 0; j0 < dp; j0 += JC) {
-      float xr[JC], ts[JC];
-      load_chunk(P.x, j0, xr);
-      const float xp = (j0 + JC < dp) ? P.x(j0 + JC) : 0.f;
-      target_score_chunk<false>(s, kind, tv0, P, xr, xm, xp, j0, ts);
-      xm = xr[JC - 1];
+    target_score_loop<false>(s, kind, tv0, P, [&](int j0, const float(&)[JC], const float(&ts)[JC]) {
 #pragma unroll
       for (int c = 0; c < JC; ++c) out(j0 + c) = (j0 + c < d) ? ts[c] : 0.f;
-    }
+    });
     return lp;
   };
   for (int j = 0; j < dp; ++j) {
@@ -699,55 +679,10 @@ __global__ void normals_kernel(uint64_t seed, uint64_t offset, int stream_id, in
   }
 }
 
-template <typename KernelT>
-int launch_cols(KernelT kernel, const lrds_spec& s, int floats, cudaStream_t st, int* nt_out, size_t* smem_out) {
-  const int cap = max_optin_smem();
-  const int nt = pick_threads(floats, cap);
-  if (nt == 0) return fail(LRDS_ERR_RESOURCES, "per-particle state of %s%ld floats does not fit in shared memory", "", floats);
-  const size_t smem = (size_t)floats * nt * sizeof(float);
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute");
-  *nt_out = nt;
-  *smem_out = smem;
-  (void)st;
-  (void)s;
-  return LRDS_OK;
-}
-
-// shared by lrds_distr_eval and the initial-cost pre-pass of lrds_rollout: logp_out = log-density + offset
-int distr_eval_launch(const lrds_distr* distr, int32_t d, const float* x, int32_t B, float* logp_out, float* score_out,
-                      float offset, cudaStream_t st) {
-  if (!distr || !x || B < 1 || d < 1 || (!logp_out && !score_out)) return fail(LRDS_ERR_INVALID, "distr_eval: bad arguments");
-  lrds_spec s;
-  memset(&s, 0, sizeof(s));
-  s.abi_version = LRDS_ABI_VERSION;
-  s.B = B;
-  s.d = d;
-  s.mlp.d = d;
-  s.mlp.d_pad = ((d + 7) / 8) * 8;
-  s.target = *distr;
-  s.ctrl_kind = LRDS_CTRL_CLIPPED;
-  s.rnd_offset = offset;
-  if (distr->kind == LRDS_DISTR_GMM) {
-    if (int r = validate_gmm(distr->gmm, "distr")) return r;
-  } else if (distr->kind == LRDS_DISTR_LOGREG) {
-    if (distr->logreg.p + 1 != d) return fail(LRDS_ERR_INVALID, "logreg: d must be p + 1");
-  } else if (distr->kind != LRDS_DISTR_PHI4) {
-    return fail(LRDS_ERR_UNSUPPORTED, "distr_eval: unknown distribution kind");
-  }
-  const lrds::ColLayout L = lrds::col_layout(s);
-  int nt = 0;
-  size_t smem = 0;
-  if (int r = launch_cols(distr_eval_kernel, s, L.total, st, &nt, &smem)) return r;
-  distr_eval_kernel<<<(B + nt - 1) / nt, nt, smem, st>>>(s, x, logp_out, score_out);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail(e, "distr_eval launch");
-  g_launches.fetch_add(1);
-  return LRDS_OK;
-}
-
-// spec of a bare distribution evaluation (lrds_distr_eval, lrds_score_cot_sums)
-int distr_spec(const lrds_distr* distr, int32_t d, int32_t B, lrds_spec* out) {
+// Spec of a bare distribution evaluation (lrds_distr_eval, lrds_score_cot_sums, lrds_mala); `who` names the entry
+// point in the messages; full-covariance mixtures are evaluated by lrds_distr_eval only (full_ok).  The caller sets the
+// spec kind / precision that select its column layout.
+int distr_spec(const lrds_distr* distr, int32_t d, int32_t B, const char* who, bool full_ok, lrds_spec* out) {
   lrds_spec& s = *out;
   memset(&s, 0, sizeof(s));
   s.abi_version = LRDS_ABI_VERSION;
@@ -757,21 +692,36 @@ int distr_spec(const lrds_distr* distr, int32_t d, int32_t B, lrds_spec* out) {
   s.mlp.d_pad = ((d + 7) / 8) * 8;
   s.target = *distr;
   s.ctrl_kind = LRDS_CTRL_CLIPPED;
-  s.precision = LRDS_PRECISION_F16X3;  // column layout without the fp32 network's activation columns (no network here)
   if (distr->kind == LRDS_DISTR_GMM) {
-    if (int r = validate_gmm(distr->gmm, "distr")) return r;
-    if (int r = refuse_full(distr->gmm, "score_cot_sums")) return r;
+    if (int r = validate_gmm(distr->gmm, who)) return r;
+    if (!full_ok)
+      if (int r = refuse_full(distr->gmm, who)) return r;
   } else if (distr->kind == LRDS_DISTR_LOGREG) {
-    if (distr->logreg.p + 1 != d) return fail(LRDS_ERR_INVALID, "logreg: d must be p + 1");
+    if (distr->logreg.p + 1 != d) return fail(LRDS_ERR_INVALID, "%s: logreg: d must be p + 1", who);
   } else if (distr->kind != LRDS_DISTR_PHI4) {
-    return fail(LRDS_ERR_UNSUPPORTED, "distr: unknown distribution kind");
+    return fail(LRDS_ERR_UNSUPPORTED, "%s: unknown distribution kind", who);
   }
   return LRDS_OK;
 }
 
+// shared by lrds_distr_eval and the initial-cost pre-pass of lrds_rollout: logp_out = log-density + offset
+int distr_eval_launch(const lrds_distr* distr, int32_t d, const float* x, int32_t B, float* logp_out, float* score_out,
+                      float offset, cudaStream_t st) {
+  if (!distr || !x || B < 1 || d < 1 || (!logp_out && !score_out)) return fail(LRDS_ERR_INVALID, "distr_eval: bad arguments");
+  lrds_spec s;
+  if (int r = distr_spec(distr, d, B, "distr_eval", true, &s)) return r;
+  s.rnd_offset = offset;
+  return launch_cols(distr_eval_kernel, "distr_eval", s, {}, st, s, x, logp_out, score_out);
+}
+
+int score_cot_spec(const lrds_distr* distr, int32_t d, int32_t B, lrds_spec* s) {
+  if (int r = distr_spec(distr, d, B, "score_cot_sums", false, s)) return r;
+  s->precision = LRDS_PRECISION_F16X3;  // column layout without the fp32 network's activation columns (no network here)
+  return LRDS_OK;
+}
+
 int score_cot_threads(const lrds_spec& s) {  // the columns + one padded row of the staging area per thread
-  uint32_t lb;
-  return pick_threads(lrds::col_layout(s).total + s.d + 1, max_optin_smem() - (int)score_cot_stage_bytes(s, &lb));
+  return pick_threads(lrds::col_layout(s).total + s.d + 1, lrds::device_limits().smem_optin - (int)score_cot_stage_bytes(s));
 }
 
 }  // namespace
@@ -781,7 +731,7 @@ extern "C" {
 int64_t lrds_score_cot_scratch_floats(const lrds_distr* distr, int32_t d, int32_t S, int32_t B) {
   lrds_spec s;
   if (!distr || d < 1 || S < 1 || B < 1) return fail(LRDS_ERR_INVALID, "score_cot_sums: bad arguments");
-  if (int r = distr_spec(distr, d, B, &s)) return r;
+  if (int r = score_cot_spec(distr, d, B, &s)) return r;
   const int nt = score_cot_threads(s);
   if (nt == 0) return fail(LRDS_ERR_RESOURCES, "score_cot_sums: per-particle state does not fit in shared memory");
   return (int64_t)S * ((B + nt - 1) / nt) * s.mlp.d_pad;
@@ -793,28 +743,16 @@ int lrds_score_cot_sums(const lrds_distr* distr, int32_t d, const float* x, cons
     return fail(LRDS_ERR_INVALID, "score_cot_sums: bad arguments");
   if (S > 65535) return fail(LRDS_ERR_UNSUPPORTED, "score_cot_sums: at most 65535 time slices per call");
   lrds_spec s;
-  if (int r = distr_spec(distr, d, B, &s)) return r;
-  const lrds::ColLayout L = lrds::col_layout(s);
+  if (int r = score_cot_spec(distr, d, B, &s)) return r;
   cudaStream_t st = (cudaStream_t)stream;
   const int nt = score_cot_threads(s);
   if (nt == 0) return fail(LRDS_ERR_RESOURCES, "score_cot_sums: per-particle state does not fit in shared memory");
-  uint32_t lb;
-  const size_t smem = (size_t)(L.total + d + 1) * nt * sizeof(float) + score_cot_stage_bytes(s, &lb);
-  cudaError_t e0 = cudaFuncSetAttribute(score_cot_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e0 != cudaSuccess) return cuda_fail(e0, "cudaFuncSetAttribute");
-  const int nblk = (B + nt - 1) / nt;
-  score_cot_kernel<<<dim3(nblk, S), nt, smem, st>>>(s, x, cot, step_w, row_w, clip, scratch);
-  cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess) {
-    score_cot_reduce_kernel<<<S, ((d + 31) / 32) * 32, 0, st>>>(scratch, nblk, s.mlp.d_pad, d, out);
-    e = cudaGetLastError();
-  }
-  if (e != cudaSuccess) return cuda_fail(e, "score_cot_sums launch");
-  g_launches.fetch_add(2);
-  return LRDS_OK;
+  // both kernels are counted once the second is issued
+  const ColExtra rows{128, d + 1, score_cot_stage_bytes(s), S, 0};
+  if (int r = launch_cols(score_cot_kernel, "score_cot_sums", s, rows, st, s, x, cot, step_w, row_w, clip, scratch)) return r;
+  score_cot_reduce_kernel<<<S, ((d + 31) / 32) * 32, 0, st>>>(scratch, (B + nt - 1) / nt, s.mlp.d_pad, d, out);
+  return launched("score_cot_sums", 2);
 }
-
-
 
 const char* lrds_last_error(void) { return g_err; }
 int lrds_abi_version(void) { return LRDS_ABI_VERSION; }
@@ -853,28 +791,17 @@ int lrds_rollout(const lrds_spec* spec, const float* x0, const float* noise, uin
   }
 
   if (s.precision != LRDS_PRECISION_FP32_SIMT) {
-    const int r = lrds::launch_rollout_tc(a, st, g_err, sizeof(g_err));
+    const int r = lrds::launch_rollout_tc(a, st);
     if (r == LRDS_OK) g_launches.fetch_add(1);
     return r;
   }
 
-  const lrds::ColLayout L = lrds::col_layout(s);
-  int nt = 0;
-  size_t smem = 0;
-  auto go = [&](auto kernel) -> int {
-    if (int r = launch_cols(kernel, s, L.total, st, &nt, &smem)) return r;
-    const int grid = (s.B + nt - 1) / nt;
-    kernel<<<grid, nt, smem, st>>>(a);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "rollout launch");
-    g_launches.fetch_add(1);
-    return LRDS_OK;
-  };
+  using lrds::rollout_simt_kernel;
   switch (s.kind) {
-    case LRDS_ROLLOUT_LINEAR: return go(lrds::rollout_simt_kernel<LRDS_ROLLOUT_LINEAR>);
-    case LRDS_ROLLOUT_CMCD: return go(lrds::rollout_simt_kernel<LRDS_ROLLOUT_CMCD>);
-    case LRDS_ROLLOUT_EUBO_LINEAR: return go(lrds::rollout_simt_kernel<LRDS_ROLLOUT_EUBO_LINEAR>);
-    case LRDS_ROLLOUT_EUBO_CMCD: return go(lrds::rollout_simt_kernel<LRDS_ROLLOUT_EUBO_CMCD>);
+    case LRDS_ROLLOUT_LINEAR: return launch_cols(rollout_simt_kernel<LRDS_ROLLOUT_LINEAR>, "rollout", s, {}, st, a);
+    case LRDS_ROLLOUT_CMCD: return launch_cols(rollout_simt_kernel<LRDS_ROLLOUT_CMCD>, "rollout", s, {}, st, a);
+    case LRDS_ROLLOUT_EUBO_LINEAR: return launch_cols(rollout_simt_kernel<LRDS_ROLLOUT_EUBO_LINEAR>, "rollout", s, {}, st, a);
+    case LRDS_ROLLOUT_EUBO_CMCD: return launch_cols(rollout_simt_kernel<LRDS_ROLLOUT_EUBO_CMCD>, "rollout", s, {}, st, a);
     default: return fail(LRDS_ERR_INVALID, "unknown rollout kind");
   }
 }
@@ -896,10 +823,7 @@ int lrds_pack_gmm_mix_tc(const lrds_gmm* gmm, int32_t d, int32_t d_pad, int32_t 
       d_pad % 8 != 0 || d_pad > LRDS_MAX_DIM_PAD || steps < 1)
     return fail(LRDS_ERR_INVALID, "pack_gmm_mix_tc: bad arguments");
   pack_gmm_mix_kernel<<<steps, 256, 0, (cudaStream_t)stream>>>(*gmm, d, d_pad, static_cast<uint8_t*>(image_out));
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail(e, "pack_gmm_mix_tc launch");
-  g_launches.fetch_add(1);
-  return LRDS_OK;
+  return launched("pack_gmm_mix_tc");
 }
 
 int64_t lrds_logreg_tc_bytes(int32_t N, int32_t p) {
@@ -912,10 +836,7 @@ int lrds_pack_logreg_tc(const lrds_logreg* logreg, int32_t d_pad, void* image_ou
   if (!logreg || !image_out || !logreg->X || !logreg->y || logreg->N < 1 || logreg->p < 1 || d_pad < logreg->p + 1)
     return fail(LRDS_ERR_INVALID, "pack_logreg_tc: bad arguments");
   pack_logreg_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(*logreg, d_pad, static_cast<uint8_t*>(image_out));
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail(e, "pack_logreg_tc launch");
-  g_launches.fetch_add(1);
-  return LRDS_OK;
+  return launched("pack_logreg_tc");
 }
 
 int lrds_pack_mlp_tc(const lrds_mlp* mlp, int32_t precision, void* image_out, void* stream) {
@@ -925,8 +846,8 @@ int lrds_pack_mlp_tc(const lrds_mlp* mlp, int32_t precision, void* image_out, vo
   if (precision != LRDS_PRECISION_TF32X3 && precision != LRDS_PRECISION_BF16 && precision != LRDS_PRECISION_TF32 &&
       precision != LRDS_PRECISION_F16X3)
     return fail(LRDS_ERR_INVALID, "pack_mlp_tc: not a tensor-core precision");
-  const int r = lrds::pack_tc_image(*mlp, precision, image_out, (cudaStream_t)stream, g_err, sizeof(g_err));
-  if (r == LRDS_OK) g_launches.fetch_add(1);
+  const int r = lrds::pack_tc_image(*mlp, precision, image_out, (cudaStream_t)stream);
+  if (r == LRDS_OK) g_launches.fetch_add(1);  // one, also for the two kernels of F16X3
   return r;
 }
 
@@ -940,19 +861,13 @@ int lrds_estimator_partials(const float* rnd, int32_t B, double* partials, doubl
   cudaError_t e = cudaMemsetAsync(counter, 0, sizeof(double), st);
   if (e != cudaSuccess) return cuda_fail(e, "estimator memset");
   estimator_kernel<<<blocks, EST_THREADS, 0, st>>>(rnd, B, partials, scratch, counter);
-  e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail(e, "estimator launch");
-  g_launches.fetch_add(1);
-  return LRDS_OK;
+  return launched("estimator");
 }
 
 int lrds_estimator_merge(const double* parts, int32_t n, double* out, void* stream) {
   if (!parts || !out || n < 1) return fail(LRDS_ERR_INVALID, "estimator_merge: bad arguments");
   estimator_merge_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(parts, n, out);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail(e, "estimator_merge launch");
-  g_launches.fetch_add(1);
-  return LRDS_OK;
+  return launched("estimator_merge");
 }
 
 int lrds_ctrl_forward(const lrds_spec* spec, int32_t row, const float* x, int32_t B, float* u_out, void* stream) {
@@ -964,16 +879,7 @@ int lrds_ctrl_forward(const lrds_spec* spec, int32_t row, const float* x, int32_
   s.precision = LRDS_PRECISION_FP32_SIMT;  // this entry point evaluates the network with fp32 FFMA
   s.has_ref_ctrl = 0;
   if (s.ctrl_kind != LRDS_CTRL_LERP) s.ref_0.M = 0;  // LerpCtrl reads the prior from ref_0
-  const lrds::ColLayout L = lrds::col_layout(s);
-  int nt = 0;
-  size_t smem = 0;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (int r = launch_cols(ctrl_forward_kernel, s, L.total, st, &nt, &smem)) return r;
-  ctrl_forward_kernel<<<(B + nt - 1) / nt, nt, smem, st>>>(s, row, x, u_out);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail(e, "ctrl_forward launch");
-  g_launches.fetch_add(1);
-  return LRDS_OK;
+  return launch_cols(ctrl_forward_kernel, "ctrl_forward", s, {}, (cudaStream_t)stream, s, row, x, u_out);
 }
 
 int64_t lrds_mlp_grad_floats(int32_t d, int32_t num_hidden) {
@@ -990,7 +896,7 @@ int lrds_mlp_grad(const lrds_mlp* mlp, const float* bias1, const float* x, const
       (!cot_scale_dev && !(cot_scale > 0.f)))
     return fail(LRDS_ERR_INVALID, "mlp_grad: bad arguments");
   const int r = lrds::launch_mlp_grad(*mlp, bias1, x, cot, step_w, row_w, clip, cot_scale, cot_scale_dev, S, B, grads_out, dbias1_out,
-                                      scratch, (cudaStream_t)stream, g_err, sizeof(g_err));
+                                      scratch, (cudaStream_t)stream);
   if (r == LRDS_OK) g_launches.fetch_add(2);
   return r;
 }
@@ -1007,40 +913,13 @@ int lrds_mala(const lrds_distr* target, int32_t d, int32_t C, int32_t n_warmup, 
       (sampler != LRDS_MCMC_MALA && sampler != LRDS_MCMC_RWMH))
     return fail(LRDS_ERR_INVALID, "mala: bad arguments");
   lrds_spec s;
-  memset(&s, 0, sizeof(s));
-  s.abi_version = LRDS_ABI_VERSION;
-  s.B = C;
-  s.d = d;
-  s.mlp.d = d;
-  s.mlp.d_pad = ((d + 7) / 8) * 8;
-  s.target = *target;
-  s.ctrl_kind = LRDS_CTRL_CLIPPED;
+  if (int r = distr_spec(target, d, C, "mala", false, &s)) return r;
   s.kind = LRDS_ROLLOUT_CMCD;  // column layout with the three extra per-chain vectors (current state, two scores)
-  if (target->kind == LRDS_DISTR_GMM) {
-    if (int r = validate_gmm(target->gmm, "target")) return r;
-    if (int r = refuse_full(target->gmm, "mala")) return r;
-  } else if (target->kind == LRDS_DISTR_LOGREG) {
-    if (target->logreg.p + 1 != d) return fail(LRDS_ERR_INVALID, "logreg: d must be p + 1");
-  } else if (target->kind != LRDS_DISTR_PHI4) {
-    return fail(LRDS_ERR_UNSUPPORTED, "mala: unknown distribution kind");
-  }
-  const lrds::ColLayout L = lrds::col_layout(s);
-  int nt = 0;
-  size_t smem = 0;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (int r = launch_cols(mala_kernel, s, L.total, st, &nt, &smem)) return r;
-  if (nt > 32) {  // few chains, long loops: one warp per CTA spreads the chains over the SMs
-    nt = 32;
-    smem = (size_t)L.total * nt * sizeof(float);
-  }
   const float tol = 0.05f, target_acc = 0.75f;
   MalaArgs m{y0, step_size, noise, unif, seed, ys_out, log_acc_out, n_warmup, n_steps, adapt, sampler,
              logf(target_acc), log1pf(tol), -log1pf(-tol), 1.01f};
-  mala_kernel<<<(C + nt - 1) / nt, nt, smem, st>>>(s, m);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail(e, "mala launch");
-  g_launches.fetch_add(1);
-  return LRDS_OK;
+  // few chains, long loops: at most one warp per CTA spreads the chains over the SMs
+  return launch_cols(mala_kernel, "mala", s, {32}, (cudaStream_t)stream, s, m);
 }
 
 int lrds_axpy_step(const float* x, const float* s, const float* z, float a, float b, float c, float* out, int64_t n,
@@ -1050,10 +929,7 @@ int lrds_axpy_step(const float* x, const float* s, const float* z, float a, floa
   const int64_t want = (n + threads - 1) / threads;
   const int grid = (int)(want < 148 * 8 ? want : 148 * 8);
   axpy_step_kernel<<<grid, threads, 0, (cudaStream_t)stream>>>(x, s, z, a, b, c, out, n);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail(e, "axpy_step launch");
-  g_launches.fetch_add(1);
-  return LRDS_OK;
+  return launched("axpy_step");
 }
 
 int lrds_normals(uint64_t seed, uint64_t particle_offset, int32_t stream_id, int32_t K, int32_t B, int32_t d, float* out,
@@ -1064,10 +940,7 @@ int lrds_normals(uint64_t seed, uint64_t particle_offset, int32_t stream_id, int
   const int64_t want = (total + threads - 1) / threads;
   const int grid = (int)(want < 148 * 16 ? want : 148 * 16);
   normals_kernel<<<grid, threads, 0, (cudaStream_t)stream>>>(seed, particle_offset, stream_id, K, B, d, out);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail(e, "normals launch");
-  g_launches.fetch_add(1);
-  return LRDS_OK;
+  return launched("normals");
 }
 
 }  // extern "C"

@@ -8,6 +8,7 @@
 //   PhiFour U / grad_U        distr/phi_four.py:45-96
 //   logistic regression       distr/logistic_regression.py:41-61 (+ autograd score, distr/base.py:146-154)
 #pragma once
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -726,6 +727,40 @@ __device__ __forceinline__ void mlp_out_chunk(const lrds_mlp& w, const Col& act,
     out[3] = fmaf(a.w, ak, out[3]); out[4] = fmaf(b.x, ak, out[4]); out[5] = fmaf(b.y, ak, out[5]);
     out[6] = fmaf(b.z, ak, out[6]); out[7] = fmaf(b.w, ak, out[7]);
   }
+}
+
+// ---- block-wide helpers of the operand-image packers and the estimator ---------------------------------------------
+struct MaxOp {
+  template <class T>
+  __device__ __forceinline__ T operator()(T a, T b) const { return fmax(a, b); }
+};
+struct SumOp {
+  template <class T>
+  __device__ __forceinline__ T operator()(T a, T b) const { return a + b; }
+};
+// op over the block's v (blockDim.x a multiple of 32): shuffles within the warps, then identity op the warp results in
+// warp order 0, 1, ... (so sums are reproducible); `red` holds blockDim.x / 32 values; every thread gets the result
+template <class T, class Op>
+__device__ __forceinline__ T block_reduce(T v, Op op, T identity, T* red) {
+  for (int o = 16; o > 0; o >>= 1) v = op(v, __shfl_xor_sync(0xffffffffu, v, o));
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  T r = identity;
+  for (int w = 0; w < (int)(blockDim.x >> 5); ++w) r = op(r, red[w]);
+  return r;
+}
+// k with amax * 2^k in [2^14, 2^15) (0 for amax = 0 or inf / NaN), clamped to [-100, 100]: the fp16 operand scale
+__device__ __forceinline__ int pow2_exponent_for(float amax) {
+  int k = 0;
+  if (amax > 0.f && amax < INFINITY) k = 14 - ilogbf(amax);
+  return k > 100 ? 100 : (k < -100 ? -100 : k);
+}
+// fp16 hi | lo split of vs: hi at out + byte, the rounding remainder at out + part_bytes + byte
+__device__ __forceinline__ void put_hi_lo(uint8_t* out, uint32_t part_bytes, uint32_t byte, float vs) {
+  const __half hi = __float2half_rn(vs);
+  *reinterpret_cast<__half*>(out + byte) = hi;
+  *reinterpret_cast<__half*>(out + part_bytes + byte) = __float2half_rn(vs - __half2float(hi));
 }
 
 }  // namespace lrds

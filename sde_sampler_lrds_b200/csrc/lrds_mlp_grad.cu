@@ -22,8 +22,6 @@
 // (`cot_scale`, chosen by the caller so that max |cot| cot_scale ~ 4) to sit in fp16's normal range.
 #include <cuda_fp16.h>
 
-#include <cstdio>
-
 #include "lrds_internal.h"
 #include "lrds_rollout_tc.cuh"
 
@@ -524,13 +522,6 @@ __global__ void __launch_bounds__(256) mlp_grad_reduce_kernel(const float* __res
   if (g == 0) dbias1[(int64_t)s * C + c] = (red[0][c] + red[1][c]) + (red[2][c] + red[3][c]);
 }
 
-static int mg_sm_count() {
-  int dev = 0, n = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-  return n > 0 ? n : 148;
-}
-
 int mlp_grad_params(int d, int nh) {
   const int dp = (d + 7) / 8 * 8;
   return d * C + nh * C * C + nh * C + C * dp + dp;
@@ -540,20 +531,16 @@ bool mlp_grad_applicable(int d, int nh) { return d >= 1 && d <= 64 && nh >= 0 &&
 
 int64_t mlp_grad_scratch_floats(int d, int nh, int S, int B) {
   const int64_t tiles = (int64_t)S * ((B + 127) / 128);
-  return (int64_t)mg_sm_count() * mlp_grad_params(d, nh) + tiles * 4 * C;
+  return (int64_t)device_limits().sms * mlp_grad_params(d, nh) + tiles * 4 * C;
 }
 
 int launch_mlp_grad(const lrds_mlp& mlp, const float* bias1, const float* x, const float* cot, const float* step_w,
                     const float* row_w, float clip, float cot_scale, const float* cot_scale_dev, int S, int B,
-                    float* grads, float* dbias1, float* scratch, cudaStream_t st, char* err, size_t n) {
-  if (!mlp_grad_applicable(mlp.d, mlp.num_hidden)) {
-    snprintf(err, n, "mlp_grad: built for d <= 64 and at most 2 hidden layers (got d = %d, %d hidden)", mlp.d, mlp.num_hidden);
-    return LRDS_ERR_UNSUPPORTED;
-  }
-  if (!mlp.tc_image) {
-    snprintf(err, n, "mlp_grad: mlp.tc_image (the F16X3 weight image of lrds_pack_mlp_tc) is required");
-    return LRDS_ERR_INVALID;
-  }
+                    float* grads, float* dbias1, float* scratch, cudaStream_t st) {
+  if (!mlp_grad_applicable(mlp.d, mlp.num_hidden))
+    return fail(LRDS_ERR_UNSUPPORTED, "mlp_grad: built for d <= 64 and at most 2 hidden layers (got d = %d, %d hidden)", mlp.d,
+                mlp.num_hidden);
+  if (!mlp.tc_image) return fail(LRDS_ERR_INVALID, "mlp_grad: mlp.tc_image (the F16X3 weight image of lrds_pack_mlp_tc) is required");
   MlpGradArgs a{};
   a.mlp = mlp;
   a.bias1 = bias1; a.x = x; a.cot = cot; a.step_w = step_w; a.row_w = row_w;
@@ -562,14 +549,12 @@ int launch_mlp_grad(const lrds_mlp& mlp, const float* bias1, const float* x, con
   a.tiles_per_s = (B + 127) / 128;
   a.tiles = (int64_t)S * a.tiles_per_s;
   a.P = mlp_grad_params(mlp.d, mlp.num_hidden);
-  const int grid = mg_sm_count();
+  const DeviceLimits dl = device_limits();
+  const int grid = dl.sms;
   a.part = scratch;
   a.dbias_part = scratch + (int64_t)grid * a.P;
   const TcLayout TL = tc_layout(mlp.d, mlp.num_hidden, LRDS_PRECISION_F16X3);
-  int dev = 0, cap = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&cap, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-  a.staged = mg_layout(TL, mlp.d, true).bytes <= (uint32_t)cap;
+  a.staged = mg_layout(TL, mlp.d, true).bytes <= (uint32_t)dl.smem_optin;
   const MgLayout ML = mg_layout(TL, mlp.d, a.staged != 0);
   cudaError_t e = cudaFuncSetAttribute(mlp_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ML.bytes);
   if (e == cudaSuccess) {
@@ -581,11 +566,7 @@ int launch_mlp_grad(const lrds_mlp& mlp, const float* bias1, const float* x, con
                                                                   4 * a.tiles_per_s, dbias1);
     e = cudaGetLastError();
   }
-  if (e != cudaSuccess) {
-    snprintf(err, n, "mlp_grad launch (grid %d, %u B smem): %s", grid, ML.bytes, cudaGetErrorString(e));
-    return LRDS_ERR_CUDA;
-  }
-  return LRDS_OK;
+  return e == cudaSuccess ? LRDS_OK : cuda_fail(e, "mlp_grad launch (grid %d, %u B smem)", grid, ML.bytes);
 }
 
 }  // namespace lrds

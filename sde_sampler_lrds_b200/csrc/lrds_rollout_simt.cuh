@@ -258,6 +258,129 @@ __device__ __forceinline__ void store_chunk(const Col4& v, int j0, const float (
   v.st4((j0 >> 2) + 1, make_float4(in[4], in[5], in[6], in[7]));
 }
 
+// target score at P.x, chunk by chunk: consume(j0, xr, ts) gets dims [j0, j0 + JC) of x and of the score
+template <bool PIPE, bool SH, class F>
+__device__ __forceinline__ void target_score_loop(const lrds_spec& s, int kind, const GmmViewT<SH>& tv, const Particle& P,
+                                                  F&& consume) {
+  const int dp = s.mlp.d_pad;
+  float xm = 0.f;
+  for (int j0 = 0; j0 < dp; j0 += JC) {
+    float xr[JC], ts[JC];
+    load_chunk(P.x, j0, xr);
+    const float xp = (j0 + JC < dp) ? P.x(j0 + JC) : 0.f;
+    target_score_chunk<PIPE>(s, kind, tv, P, xr, xm, xp, j0, ts);
+    xm = xr[JC - 1];
+    consume(j0, xr, ts);
+  }
+}
+
+// one thread per particle (the column-layout kernels of lrds_capi.cu): b is the thread's particle, clamped to the last
+// one in the idle threads of the last CTA, whose results are not written (live = false)
+struct ParticleThread {
+  int b;
+  bool live;
+  Particle P;
+};
+__device__ __forceinline__ ParticleThread particle_thread(const lrds_spec& s, float* smem) {
+  const int NT = blockDim.x, tid = threadIdx.x;
+  const int b_raw = blockIdx.x * NT + tid;
+  const bool live = b_raw < s.B;
+  return ParticleThread{live ? b_raw : s.B - 1, live, make_particle(smem, col_layout(s), NT, tid)};
+}
+
+constexpr int MIX_MAX_M = 16;  // components of a mixture whose responsibilities live in registers (gmm_pass1_pair)
+
+// Responsibilities r = softmax_m(logc_m - q_m / 2) of a mixture with M <= 16 components in registers (the arithmetic
+// of gmm_pass1, lrds_device.cuh); returns the mixture log-density; modes beyond M get weight zero.  The quadratic forms
+// are bound by the shared-memory pipe, not by the FMA pipe: every (1/sigma, -mu/sigma) pair is used once per particle and a warp-uniform LDS.128
+// (one wavefront) feeds only two FFMA2.  Here the two half-warps split the mode blocks, and every thread evaluates
+// its modes for TWO particles - its own and the one of lane ^ 16 - so that each operand vector feeds four FFMA2;
+// the dims are the outer loop, so that a particle's coordinates are read once per call instead of once per mode
+// block.  The halves swap their partner results with one SHFL per mode.
+template <bool SH>
+__device__ __forceinline__ float gmm_pass1_pair(const GmmViewT<SH>& g, int d, int dp, const Col4& x, float (&r)[MIX_MAX_M]) {
+  const int lane = threadIdx.x & 31, h = lane >> 4;
+  const int nq = (d + 3) >> 2;
+  const int rowq = dp >> 2;
+  const int M4 = (g.M + 3) >> 2;
+  const int nb = (M4 + 1) >> 1;  // mode blocks per half-warp (warp-uniform): 1 or 2
+  const int b0 = h * nb;
+  const Col4 xo{x.p + ((lane ^ 16) - lane) * 4, x.stride};  // the partner's coordinates
+  const int blk0 = min(b0, M4 - 1), blk1 = min(b0 + 1, M4 - 1);  // clamped: results of blocks >= M4 are discarded
+  PPtr<SH> p0 = g.sn + blk0 * rowq * 32, p1 = g.sn + blk1 * rowq * 32;
+  u64 qa[8] = {0, 0, 0, 0, 0, 0, 0, 0}, qb[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // own / partner particle, (even, odd) dims
+  auto block = [&](const PPtr<SH>& p, const ulonglong2& xa, const ulonglong2& xb, int o) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const ulonglong2 sv = p.ld2(2 * i), nv = p.ld2(2 * i + 1);
+      const u64 a0 = f2::fma(xa.x, sv.x, nv.x), a1 = f2::fma(xa.y, sv.y, nv.y);
+      const u64 c0 = f2::fma(xb.x, sv.x, nv.x), c1 = f2::fma(xb.y, sv.y, nv.y);
+      qa[o + i] = f2::fma(a0, a0, qa[o + i]);
+      qb[o + i] = f2::fma(c0, c0, qb[o + i]);
+      qa[o + i] = f2::fma(a1, a1, qa[o + i]);
+      qb[o + i] = f2::fma(c1, c1, qb[o + i]);
+    }
+  };
+  if (nb > 1) {
+    for (int c = 0; c < nq; ++c, p0 = p0 + 32, p1 = p1 + 32) {
+      const ulonglong2 xa = x.ldu(c), xb = xo.ldu(c);
+      block(p0, xa, xb, 0);
+      block(p1, xa, xb, 4);
+    }
+  } else {
+    for (int c = 0; c < nq; ++c, p0 = p0 + 32) {
+      const ulonglong2 xa = x.ldu(c), xb = xo.ldu(c);
+      block(p0, xa, xb, 0);
+    }
+  }
+  float own[8], oth[8];
+  {
+    const float4 l0 = g.logc.ld4(blk0), l1 = g.logc.ld4(blk1);
+    const float lc[8] = {l0.x, l0.y, l0.z, l0.w, l1.x, l1.y, l1.z, l1.w};
+    const bool v0 = b0 < M4, v1 = nb > 1 && b0 + 1 < M4;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      const bool v = k < 4 ? v0 : v1;
+      float ax, ay, bx, by;
+      f2::unpack(qa[k], ax, ay);
+      f2::unpack(qb[k], bx, by);
+      own[k] = v ? lc[k] - 0.5f * (ax + ay) : -INFINITY;
+      oth[k] = v ? lc[k] - 0.5f * (bx + by) : -INFINITY;
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < 8; ++k) oth[k] = __shfl_xor_sync(0xffffffffu, oth[k], 16);  // my particle, the other half's modes
+  if (nb > 1) {
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      r[k] = h ? oth[k] : own[k];
+      r[8 + k] = h ? own[k] : oth[k];
+    }
+  } else {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      r[k] = h ? oth[k] : own[k];
+      r[4 + k] = h ? own[k] : oth[k];
+    }
+#pragma unroll
+    for (int k = 8; k < MIX_MAX_M; ++k) r[k] = -INFINITY;
+  }
+  float mx = r[0];
+#pragma unroll
+  for (int i = 1; i < MIX_MAX_M; ++i) mx = fmaxf(mx, r[i]);
+  float s = 0.f;
+#pragma unroll
+  for (int mb = 0; mb < MIX_MAX_M / 4; ++mb) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) r[4 * mb + i] = __expf(r[4 * mb + i] - mx);
+    s += (r[4 * mb] + r[4 * mb + 1]) + (r[4 * mb + 2] + r[4 * mb + 3]);
+  }
+  const float inv = 1.0f / s;
+#pragma unroll
+  for (int i = 0; i < MIX_MAX_M; ++i) r[i] *= inv;
+  return mx + __logf(s);
+}
+
 // control u = generative_ctrl(tau, x) for dims [j0, j0+JC) after mlp.hidden(), given the raw target score chunk
 // `ts` (ScoreCtrl) and gamma = clip(score_model(tau)).   models/reparam.py:33-43, 112-117
 struct CtrlConst {

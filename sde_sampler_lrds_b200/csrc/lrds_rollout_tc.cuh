@@ -20,8 +20,7 @@
 #pragma once
 #include <cuda_fp16.h>
 
-#include <cstdio>
-
+#include "lrds_internal.h"
 #include "lrds_rollout_simt.cuh"
 #include "lrds_tc_ptx.cuh"
 
@@ -81,15 +80,9 @@ static __global__ void tc_scales_kernel(const lrds_mlp w, const TcLayout L, uint
     const int n = l == 0 ? w.d * C : (l <= L.nh ? C * C : C * w.d_pad);
     float m = 0.f;
     for (int i = threadIdx.x; i < n; i += blockDim.x) m = fmaxf(m, fabsf(p[i]));
-    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = m;
-    __syncthreads();
+    m = block_reduce(m, MaxOp{}, 0.f, red);
     if (threadIdx.x == 0) {
-      for (int i = 1; i < (int)(blockDim.x >> 5); ++i) m = fmaxf(m, red[i]);
-      int k = 0;
-      if (m > 0.f && m < INFINITY) k = 14 - ilogbf(m);
-      k = k > 100 ? 100 : (k < -100 ? -100 : k);
+      const int k = pow2_exponent_for(m);
       sc[l] = ldexpf(1.0f, k);
       sc[8 + l] = ldexpf(1.0f, -k) / (l == 0 ? 1.0f : TC_ACT_SCALE);
     }
@@ -122,10 +115,7 @@ static __global__ void pack_tc_image_kernel(const lrds_mlp w, const TcLayout L, 
     if (L.prec == LRDS_PRECISION_BF16) {
       *reinterpret_cast<uint16_t*>(img + byte) = (uint16_t)(ptx::pack_bf16x2(v, 0.f) & 0xFFFFu);
     } else if (L.prec == LRDS_PRECISION_F16X3) {
-      const float vs = v * sc[layer];  // exact (power of two)
-      const __half hi = __float2half_rn(vs);
-      *reinterpret_cast<__half*>(img + byte) = hi;
-      *reinterpret_cast<__half*>(img + L.part_bytes + byte) = __float2half_rn(vs - __half2float(hi));
+      put_hi_lo(img, L.part_bytes, byte, v * sc[layer]);  // exact scaling (power of two)
     } else {
       const float hi = ptx::to_tf32(v);
       *reinterpret_cast<float*>(img + byte) = hi;
@@ -556,18 +546,14 @@ inline uint32_t plan_tmem_cols(int cols) {
 // Launches a tensor-core rollout kernel (arguments: the rollout, the weight image, then `args`) with the plan's grid and
 // shared memory and `threads` threads per CTA; `what` names the kernel in the error message.
 template <class K, class... A>
-int launch_tc(K kernel, const char* what, const RolloutArgs& a, const TcPlan& p, int threads, cudaStream_t st, char* err, size_t n,
-              A... args) {
+int launch_tc(K kernel, const char* what, const RolloutArgs& a, const TcPlan& p, int threads, cudaStream_t st, A... args) {
   cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);
   if (e == cudaSuccess) {
     kernel<<<p.grid, threads, p.smem, st>>>(a, static_cast<const uint8_t*>(a.s.mlp.tc_image), args...);
     e = cudaGetLastError();
   }
-  if (e != cudaSuccess) {
-    snprintf(err, n, "%s launch (grid %d x %d threads, %zu B smem, %u TMEM cols): %s", what, p.grid, threads, p.smem,
-             p.tmem_cols, cudaGetErrorString(e));
-    return LRDS_ERR_CUDA;
-  }
+  if (e != cudaSuccess)
+    return cuda_fail(e, "%s launch (grid %d x %d threads, %zu B smem, %u TMEM cols)", what, p.grid, threads, p.smem, p.tmem_cols);
   return LRDS_OK;
 }
 

@@ -5,21 +5,20 @@
 
 namespace lrds {
 
-int launch_mix_b(int cfg, const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n);  // lrds_tc_mix_b.cu
-int launch_mix_c(int cfg, const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n);  // lrds_tc_mix_c.cu
+int launch_mix_b(int cfg, const RolloutArgs& a, const TcPlan& p, cudaStream_t st);  // lrds_tc_mix_b.cu
+int launch_mix_c(int cfg, const RolloutArgs& a, const TcPlan& p, cudaStream_t st);  // lrds_tc_mix_c.cu
 
-int launch_mix_f16x3(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
+int launch_mix_f16x3(const RolloutArgs& a, const TcPlan& p, cudaStream_t st) {
   const int cfg = mix_tc_config(a.s);
   switch (cfg) {  // MixCfg<EUBO, TGT, REF, EM>
-    case 0: return launch_mix_cfg<MixBench>(a, p, st, err, n);
-    case 1: return launch_mix_cfg<MixCfg<true, 1, 2, false>>(a, p, st, err, n);
-    case 2: return launch_mix_cfg<MixCfg<false, 1, 1, false>>(a, p, st, err, n);
-    case 3: return launch_mix_cfg<MixCfg<false, 1, 1, true>>(a, p, st, err, n);
-    case 4: case 5: case 6: return launch_mix_b(cfg, a, p, st, err, n);
-    case 7: case 8: case 9: case 10: return launch_mix_c(cfg, a, p, st, err, n);
+    case 0: return launch_mix_cfg<MixBench>(a, p, st);
+    case 1: return launch_mix_cfg<MixCfg<true, 1, 2, false>>(a, p, st);
+    case 2: return launch_mix_cfg<MixCfg<false, 1, 1, false>>(a, p, st);
+    case 3: return launch_mix_cfg<MixCfg<false, 1, 1, true>>(a, p, st);
+    case 4: case 5: case 6: return launch_mix_b(cfg, a, p, st);
+    case 7: case 8: case 9: case 10: return launch_mix_c(cfg, a, p, st);
   }
-  snprintf(err, n, "mixture tensor-core rollout: configuration not built");
-  return LRDS_ERR_UNSUPPORTED;
+  return fail(LRDS_ERR_UNSUPPORTED, "mixture tensor-core rollout: configuration not built");
 }
 }  // namespace lrds
 

@@ -5,11 +5,11 @@
 
 namespace lrds {
 
-int launch_mix_b(int cfg, const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
+int launch_mix_b(int cfg, const RolloutArgs& a, const TcPlan& p, cudaStream_t st) {
   switch (cfg) {
-    case 4: return launch_mix_cfg<MixCfg<false, 2, 2, false>>(a, p, st, err, n);
-    case 5: return launch_mix_cfg<MixCfg<false, 0, 2, false>>(a, p, st, err, n);
-    default: return launch_mix_cfg<MixCfg<false, 1, 2, true>>(a, p, st, err, n);
+    case 4: return launch_mix_cfg<MixCfg<false, 2, 2, false>>(a, p, st);
+    case 5: return launch_mix_cfg<MixCfg<false, 0, 2, false>>(a, p, st);
+    default: return launch_mix_cfg<MixCfg<false, 1, 2, true>>(a, p, st);
   }
 }
 }  // namespace lrds

@@ -5,12 +5,12 @@
 
 namespace lrds {
 
-int launch_mix_c(int cfg, const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
+int launch_mix_c(int cfg, const RolloutArgs& a, const TcPlan& p, cudaStream_t st) {
   switch (cfg) {
-    case 7: return launch_mix_cfg<MixCfg<false, 1, 0, true>>(a, p, st, err, n);
-    case 8: return launch_mix_cfg<MixCfg<false, 1, 0, false>>(a, p, st, err, n);
-    case 10: return launch_mix_cfg<MixCfg<false, 1, 0, true, true>>(a, p, st, err, n);
-    default: return launch_mix_cfg<MixCfg<false, 2, 1, false>>(a, p, st, err, n);
+    case 7: return launch_mix_cfg<MixCfg<false, 1, 0, true>>(a, p, st);
+    case 8: return launch_mix_cfg<MixCfg<false, 1, 0, false>>(a, p, st);
+    case 10: return launch_mix_cfg<MixCfg<false, 1, 0, true, true>>(a, p, st);
+    default: return launch_mix_cfg<MixCfg<false, 2, 1, false>>(a, p, st);
   }
 }
 }  // namespace lrds

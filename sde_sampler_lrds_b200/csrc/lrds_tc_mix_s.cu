@@ -5,12 +5,12 @@
 
 namespace lrds {
 
-int launch_mix_small_f16x3(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
-  return launch_tc(rollout_mix_small_kernel<LRDS_PRECISION_F16X3>, "small-batch mixture rollout", a, p, p.warps * 32, st, err, n);
+int launch_mix_small_f16x3(const RolloutArgs& a, const TcPlan& p, cudaStream_t st) {
+  return launch_tc(rollout_mix_small_kernel<LRDS_PRECISION_F16X3>, "small-batch mixture rollout", a, p, p.warps * 32, st);
 }
 
-int launch_cmcd_mix_f16x3(const RolloutArgs& a, const TcPlan& p, cudaStream_t st, char* err, size_t n) {
-  return launch_tc(rollout_cmcd_mix_kernel<LRDS_PRECISION_F16X3>, "CMCD mixture rollout", a, p, p.warps * 32, st, err, n, p.tmem_cols);
+int launch_cmcd_mix_f16x3(const RolloutArgs& a, const TcPlan& p, cudaStream_t st) {
+  return launch_tc(rollout_cmcd_mix_kernel<LRDS_PRECISION_F16X3>, "CMCD mixture rollout", a, p, p.warps * 32, st, p.tmem_cols);
 }
 }  // namespace lrds
 

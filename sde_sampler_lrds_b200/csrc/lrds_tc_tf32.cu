@@ -2,5 +2,5 @@
 #include "lrds_tc_launch.cuh"
 
 namespace lrds {
-template int launch_prec<LRDS_PRECISION_TF32>(const RolloutArgs&, const TcPlan&, cudaStream_t, char*, size_t);
+template int launch_prec<LRDS_PRECISION_TF32>(const RolloutArgs&, const TcPlan&, cudaStream_t);
 }  // namespace lrds

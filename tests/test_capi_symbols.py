@@ -38,8 +38,39 @@ def test_invalid_arguments_are_rejected_without_a_gpu():
     spec = N.Spec()
     spec.abi_version = 99
     assert lib.lrds_rollout(C.byref(spec), None, None, 0, 0, None, None, None, None) == -1
+    assert b"got 99" in lib.lrds_last_error()
     assert lib.lrds_estimator_blocks(1) == 1 and lib.lrds_estimator_blocks(8193) == 2
     assert lib.lrds_estimator_partials(None, 0, None, None, None) == -1
+
+    # the bare-distribution entry points: arguments, then the distribution (no pointer is dereferenced on these paths)
+    p = 256  # dummy device pointer
+    d = 4
+
+    def distr_eval(distr, B=8, x=p):
+        return lib.lrds_distr_eval(C.byref(distr) if distr else None, d, x, B, p, None, None)
+
+    def mala(distr, C_=8, sampler=N.MCMC_MALA):
+        return lib.lrds_mala(C.byref(distr) if distr else None, d, C_, 0, 4, 0, sampler, p, p, None, None, 0, p, None, None)
+
+    def score_cot(distr, S=2):
+        return lib.lrds_score_cot_scratch_floats(C.byref(distr) if distr else None, d, S, 8)
+
+    good = N.Distr()
+    good.kind = N.DISTR_PHI4
+    for call, who in ((lambda: distr_eval(None), b"distr_eval"), (lambda: distr_eval(good, B=0), b"distr_eval"),
+                      (lambda: distr_eval(good, x=None), b"distr_eval"), (lambda: mala(None), b"mala"),
+                      (lambda: mala(good, C_=0), b"mala"), (lambda: score_cot(None), b"score_cot"),
+                      (lambda: score_cot(good, S=0), b"score_cot")):
+        assert call() == -1 and who in lib.lrds_last_error()
+    none = N.Distr()
+    none.kind = N.DISTR_NONE
+    assert distr_eval(none) == -2 and mala(none) == -2 and score_cot(none) == -2
+    full = N.Distr()
+    full.kind = N.DISTR_GMM
+    full.gmm.M, full.gmm.layout, full.gmm.logc, full.gmm.mu, full.gmm.sn = 2, N.GMM_FULL, p, p, p
+    for call, who in ((lambda: score_cot(full), b"score_cot"), (lambda: mala(full), b"mala")):
+        assert call() == -2 and who in lib.lrds_last_error()
+    assert mala(good, sampler=7) == -1
 
 
 def test_mixture_tensor_core_image_layout():
