@@ -17,7 +17,7 @@
 extern "C" {
 #endif
 
-#define LRDS_ABI_VERSION 9 /* 9: lrds_gmm.layout (full-covariance Gaussian / mixture references) */
+#define LRDS_ABI_VERSION 10 /* 10: lrds_adjoint; 9: lrds_gmm.layout (full-covariance Gaussian / mixture references) */
 #define LRDS_CHANNELS 64 /* FourierMLP / TimeEmbed width, conf/model/base/fouriermlp.yaml:4 */
 #define LRDS_MAX_DIM_PAD 1024 /* largest d_pad the operand packers accept */
 
@@ -243,6 +243,30 @@ typedef struct {
  */
 int lrds_rollout(const lrds_spec* spec, const float* x0, const float* noise, uint64_t seed,
                  uint64_t particle_offset, float* x_out, float* rnd_out, float* traj_out, void* stream);
+
+/* ---- the pathwise (method 'kl' / 'kl_ito') gradient of the LINEAR simulate loop: the reverse-time recursion that
+ * autograd runs through the K steps when the SDE follows the non-detached control (generative_and_sde_ctrl,
+ * oc.py:83-103) and loss = mean(rnd[mask]) (compute_loss, oc.py:105-131).  With g_k = clip(net(t_k, x_k)) and
+ * e_k = the Ito weight of lrds_ito_form times z_k (0 for LRDS_ITO_NONE), the adjoint of particle b is
+ *   lambda_K = w_b (grad ref_0(x_K) - [|target(x_K)| <= clip_target] grad target(x_K))        (init_cost: no ref_0 term)
+ *   gbar_k   = w_b (2 W_COST g_k + e_k) + (d x_{k+1} / d g) lambda_{k+1}                        (B for AXPY, B dt for EM)
+ *   lambda_k = a_k lambda_{k+1} + c_k J_r(x_k) lambda_{k+1} + J_net^T ([|net| <= clip_model] gbar_k)
+ *              (a_k, c_k) = (A, B) for AXPY, (1 - A dt, C dt) for EM; J_r = the Jacobian of the reference score
+ * and d loss / d theta = sum_k <gbar_k, d g_k / d theta>: lrds_mlp_grad with cot = gbar (step_w = row_w = NULL).
+ *   traj    [K+1][B][d] the trajectory lrds_rollout wrote for this spec
+ *   noise   [K][B][d] the increments that rollout consumed, or NULL: the kernel regenerates the production-mode Philox
+ *           increments of (seed, particle_offset)
+ *   row_w   [B] w_b = d loss / d rnd_b
+ *   cot_out [K][B][d] gbar_k = d loss / d g_k
+ * Built for the LRDS_ROLLOUT_LINEAR kind, LRDS_CTRL_CLIPPED, a diagonal reference (or none), every target kind, and the
+ * precisions F16X3 / TF32X3 / FP32_SIMT; LRDS_ERR_UNSUPPORTED for the score-family controls, full-covariance ref_t /
+ * ref_0, the CMCD and EUBO kinds and BF16 / TF32 (their network is not the one the adjoint would linearise).  F16X3 inside
+ * lrds_mlp_grad's envelope (d <= 64, num_hidden <= 2; mlp.tc_image = the F16X3 image) runs the network on tcgen05 with the
+ * rollout's weight image and adds to spec.status like the rollout: [0] += threads (four per particle) whose fp16 operands
+ * saturated (a coordinate or cotangent beyond 65504, a hidden pre-activation beyond 1023), [1] += particles with a
+ * non-finite cotangent.  Every other accepted spec recomputes the network with fp32 FFMA and never touches [0]. */
+int lrds_adjoint(const lrds_spec* spec, const float* traj, const float* noise, uint64_t seed, uint64_t particle_offset,
+                 const float* row_w, float* cot_out, void* stream);
 
 /* ---- tensor-core weight image: the FourierMLP weights in the shared-memory operand layout of tcgen05.mma (plus
  * the fp32 biases), staged once per CTA by a bulk TMA copy.  `image_out` (device, 16-byte aligned) must hold

@@ -19,7 +19,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.environ.get("LRDS_B200_LIB") or os.path.join(CSRC, "liblrds_b200.so")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 CHANNELS = 64
 STEP_STRIDE = 80
 (STEP_A, STEP_B, STEP_C, STEP_DT, STEP_SQRT_DT, STEP_W_COST, STEP_W_ITO, STEP_GAMMA, STEP_FRAC, STEP_SIGU,
@@ -76,7 +76,7 @@ class Spec(C.Structure):
                 ("steps", FP), ("mlp", Mlp), ("target", Distr), ("ref_t", Gmm), ("ref_0", Gmm), ("status", FP)]
 
 
-EXPORTS = ["lrds_rollout", "lrds_tc_image_bytes", "lrds_gmm_mix_tc_bytes", "lrds_pack_gmm_mix_tc", "lrds_logreg_tc_bytes",
+EXPORTS = ["lrds_rollout", "lrds_adjoint", "lrds_tc_image_bytes", "lrds_gmm_mix_tc_bytes", "lrds_pack_gmm_mix_tc", "lrds_logreg_tc_bytes",
            "lrds_pack_logreg_tc", "lrds_pack_mlp_tc", "lrds_estimator_blocks", "lrds_estimator_partials", "lrds_estimator_merge", "lrds_ctrl_forward",
            "lrds_distr_eval", "lrds_axpy_step", "lrds_normals", "lrds_mala", "lrds_mlp_grad", "lrds_mlp_grad_floats",
            "lrds_mlp_grad_scratch_floats", "lrds_score_cot_sums", "lrds_score_cot_scratch_floats",
@@ -140,6 +140,7 @@ def lib():
                 L.lrds_last_error.restype = C.c_char_p
                 L.lrds_launch_count.restype = C.c_int64
                 L.lrds_rollout.argtypes = [C.POINTER(Spec), FP, FP, C.c_uint64, C.c_uint64, FP, FP, FP, FP]
+                L.lrds_adjoint.argtypes = [C.POINTER(Spec), FP, FP, C.c_uint64, C.c_uint64, FP, FP, FP]
                 L.lrds_tc_image_bytes.restype = C.c_int64
                 L.lrds_tc_image_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]
                 L.lrds_pack_mlp_tc.argtypes = [C.POINTER(Mlp), C.c_int32, FP, FP]

@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstring>
 
+#include "lrds_adjoint.cuh"
 #include "lrds_internal.h"
 #include "lrds_rollout_simt.cuh"
 
@@ -71,15 +72,16 @@ int pick_threads(int floats_per_particle, int smem_cap) {
 
 // Launch of a kernel with one thread per particle and the spec's shared-memory columns (col_layout): `floats` more
 // shared-memory floats per thread, `bytes` more per CTA, at most `max_nt` threads per CTA, `slices` CTA rows (grid.y);
-// `launches` are counted when the launch succeeds.
+// `launches` are counted when the launch succeeds; `layout` >= 0 replaces col_layout(s).total (a kernel with its own
+// column layout).
 struct ColExtra {
   int max_nt = 128, floats = 0;
   uint32_t bytes = 0;
-  int slices = 1, launches = 1;
+  int slices = 1, launches = 1, layout = -1;
 };
 template <class K, class... A>
 int launch_cols(K kernel, const char* what, const lrds_spec& s, const ColExtra& x, cudaStream_t st, A... args) {
-  const int floats = lrds::col_layout(s).total + x.floats;
+  const int floats = (x.layout >= 0 ? x.layout : lrds::col_layout(s).total) + x.floats;
   int nt = pick_threads(floats, lrds::device_limits().smem_optin - (int)x.bytes);
   if (nt == 0) return fail(LRDS_ERR_RESOURCES, "per-particle state of %d floats does not fit in shared memory", floats);
   nt = nt < x.max_nt ? nt : x.max_nt;
@@ -138,6 +140,12 @@ int validate_spec(const lrds_spec* s, bool need_steps) {
       return fail(LRDS_ERR_UNSUPPORTED, "unknown target kind");
   }
   return LRDS_OK;
+}
+
+// the fp32 adjoint (lrds_adjoint.cuh): the parity anchor, and every spec outside the tensor-core kernel's envelope
+__global__ void __launch_bounds__(128) adjoint_simt_kernel(const lrds::AdjointArgs a) {
+  extern __shared__ __align__(16) float smem[];
+  lrds::adjoint_body(a, smem);
 }
 
 // ---- estimator partials -----------------------------------------------------------------------------
@@ -804,6 +812,40 @@ int lrds_rollout(const lrds_spec* spec, const float* x0, const float* noise, uin
     case LRDS_ROLLOUT_EUBO_CMCD: return launch_cols(rollout_simt_kernel<LRDS_ROLLOUT_EUBO_CMCD>, "rollout", s, {}, st, a);
     default: return fail(LRDS_ERR_INVALID, "unknown rollout kind");
   }
+}
+
+int lrds_adjoint(const lrds_spec* spec, const float* traj, const float* noise, uint64_t seed, uint64_t particle_offset,
+                 const float* row_w, float* cot_out, void* stream) {
+  if (int r = validate_spec(spec, true)) return r;
+  if (!traj || !row_w || !cot_out) return fail(LRDS_ERR_INVALID, "adjoint: traj, row_w and cot_out are required");
+  const lrds_spec& s = *spec;
+  if (s.K < 1) return fail(LRDS_ERR_INVALID, "adjoint: K must be >= 1");
+  if (s.kind != LRDS_ROLLOUT_LINEAR)
+    return fail(LRDS_ERR_UNSUPPORTED, "adjoint: built for the LINEAR simulate loop (CMCD evaluates the control at both ends of a "
+                                      "step and the EUBO kinds are not trained through it)");
+  if (s.ctrl_kind != LRDS_CTRL_CLIPPED)
+    return fail(LRDS_ERR_UNSUPPORTED, "adjoint: built for ClippedCtrl; the score-family controls also need the target's "
+                                      "Hessian-vector product");
+  if (s.precision == LRDS_PRECISION_BF16 || s.precision == LRDS_PRECISION_TF32)
+    return fail(LRDS_ERR_UNSUPPORTED, "adjoint: the reduced-precision network moved the particles, the adjoint would linearise a "
+                                      "different one (use f16x3, tf32x3 or fp32)");
+  if (s.precision != LRDS_PRECISION_FP32_SIMT && s.precision != LRDS_PRECISION_TF32X3 && s.precision != LRDS_PRECISION_F16X3)
+    return fail(LRDS_ERR_INVALID, "adjoint: unknown precision");
+  if (int r = validate_gmm(s.ref_0, "ref_0")) return r;
+  if (s.has_ref_ctrl)
+    if (int r = validate_gmm(s.ref_t, "ref_t")) return r;
+  if (lrds::ref_t_full(s) || s.ref_0.layout == LRDS_GMM_FULL)
+    return fail(LRDS_ERR_UNSUPPORTED, "adjoint: built for diagonal references (full-covariance ref_t / ref_0 are not)");
+  const lrds::AdjointArgs a{lrds::RolloutArgs{s, nullptr, noise, seed, particle_offset, nullptr, nullptr, nullptr}, traj, row_w,
+                            cot_out};
+  if (lrds::adjoint_tc_applicable(s)) {
+    const int r = lrds::launch_adjoint_tc(a, (cudaStream_t)stream);
+    if (r == LRDS_OK) g_launches.fetch_add(1);
+    return r;
+  }
+  ColExtra cols;
+  cols.layout = lrds::adj_layout(s).total;
+  return launch_cols(adjoint_simt_kernel, "adjoint", s, cols, (cudaStream_t)stream, a);
 }
 
 int64_t lrds_tc_image_bytes(int32_t d, int32_t num_hidden, int32_t precision) {

@@ -681,10 +681,16 @@ __device__ __forceinline__ void fma_row64(float (&acc)[C], const float* __restri
   }
 }
 
+// GELU'(v) = Phi(v) + v phi(v) of the exact GELU
+__device__ __forceinline__ float gelu_grad(float v) {
+  return fmaf(v * 0.3989422804014327f, __expf(-0.5f * v * v), normcdff(v));
+}
+
 // hidden activations GELU(h_L) of the particle -> act(0..63)   (models/mlp.py:136-142)
-template <bool BIAS_SH>
+// TAPE (the adjoint's forward recompute): also GELU'(h_l) of every layer l -> tape(64 l + n)
+template <bool BIAS_SH, bool TAPE = false>
 __device__ __forceinline__ void mlp_hidden(const lrds_mlp& w, const float* __restrict__ bias1, const Col4& x,
-                                           const Col& act) {
+                                           const Col& act, const Col& tape = Col{nullptr, 0}) {
   float acc[C];
 #pragma unroll
   for (int q = 0; q < C / 4; ++q) {
@@ -699,7 +705,10 @@ __device__ __forceinline__ void mlp_hidden(const lrds_mlp& w, const float* __res
       if (4 * kq + e < w.d) fma_row64(acc, w.w_in_t + (int64_t)(4 * kq + e) * C, xs[e]);
   }
 #pragma unroll
-  for (int n = 0; n < C; ++n) act(n) = gelu_exact(acc[n]);
+  for (int n = 0; n < C; ++n) {
+    act(n) = gelu_exact(acc[n]);
+    if constexpr (TAPE) tape(n) = gelu_grad(acc[n]);
+  }
   for (int l = 0; l < w.num_hidden; ++l) {
     const float* wl = w.w_hid_t + (int64_t)l * C * C;
 #pragma unroll
@@ -707,7 +716,10 @@ __device__ __forceinline__ void mlp_hidden(const lrds_mlp& w, const float* __res
 #pragma unroll 2
     for (int k = 0; k < C; ++k) fma_row64(acc, wl + k * C, act(k));
 #pragma unroll
-    for (int n = 0; n < C; ++n) act(n) = gelu_exact(acc[n]);
+    for (int n = 0; n < C; ++n) {
+      act(n) = gelu_exact(acc[n]);
+      if constexpr (TAPE) tape((l + 1) * C + n) = gelu_grad(acc[n]);
+    }
   }
 }
 

@@ -8,6 +8,7 @@
 
 namespace lrds {
 struct RolloutArgs;
+struct AdjointArgs;
 // lrds_capi.cu: the calling thread's message for lrds_last_error; `code` resp. LRDS_ERR_CUDA is returned, and
 // cuda_fail appends ": " and the CUDA error string
 int fail(int code, const char* fmt, ...) __attribute__((format(printf, 2, 3)));
@@ -21,6 +22,9 @@ DeviceLimits device_limits();
 int launch_rollout_tc(const RolloutArgs& a, cudaStream_t st);
 size_t tc_image_bytes(int d, int num_hidden, int precision);
 int pack_tc_image(const lrds_mlp& w, int precision, void* image, cudaStream_t st);
+// lrds_adjoint_tc.cu: the tcgen05 adjoint (F16X3 inside lrds_mlp_grad's envelope, when its shared memory fits)
+bool adjoint_tc_applicable(const lrds_spec& s);
+int launch_adjoint_tc(const AdjointArgs& a, cudaStream_t st);
 // lrds_mlp_grad.cu
 bool mlp_grad_applicable(int d, int num_hidden);
 int mlp_grad_params(int d, int num_hidden);

@@ -14,8 +14,9 @@ Extra keyword arguments (not in the reference, all optional): ``noise`` = record
 to consume instead of in-kernel Philox draws (validation mode), ``seed`` / ``particle_offset`` for the
 counter-based generator (global particle index => results independent of the GPU count).
 Training: ``loss(ts, x, ...)`` with method 'lv' / 'lv_traj' returns a scalar whose ``backward()`` fills the control's
-parameter gradients (train.py: fused rollout + one batched gradient pass), for every loss class below; 'kl' (pathwise
-gradient through the trajectory) raises.
+parameter gradients (train.py: fused rollout + one batched gradient pass), for every loss class below; 'kl' / 'kl_ito'
+(pathwise gradient through the trajectory: fused rollout + the reverse-time adjoint kernel + the same parameter pass) for
+the linear losses with a ClippedCtrl drift.
 """
 from __future__ import annotations
 
@@ -151,25 +152,36 @@ class BaseOCLoss:
             loss = kept.var() if self.method == "lv" else kept.mean()
         return loss, {"train/n_filtered_cumulative": self.n_filtered}
 
-    def _train(self, make_plan, x, noise=None, seed=None, particle_offset: int = 0, group=None):
+    def _train(self, make_plan, x, noise=None, seed=None, particle_offset: int = 0, group=None, initial_log_prob=None):
         """[TRAINING] shared by the ``__call__`` of the linear losses: repeat the initial values, run the fused rollout
-        with the detached control driving the SDE, return (loss, metrics) with the LV gradient attached (train.py)."""
+        and return (loss, metrics) with the gradient attached (train.py): for 'lv' / 'lv_traj' the SDE follows the
+        detached control (lv_objective), for 'kl' / 'kl_ito' the pathwise gradient through the trajectory
+        (kl_objective, ClippedCtrl).  ``initial_log_prob`` (DIS): the prior log-density the rollout starts the log-weight
+        at, which the 'kl' training form leaves out."""
         from .. import train
-        if self.method not in ("lv", "lv_traj"):
-            raise NotImplementedError("method 'kl' / 'kl_ito' differentiates through the trajectory (pathwise gradient): "
-                                      "not built; the shipped solver configs train with loss_type 'lv' or 'kl' "
-                                      "(SURVEY.md 8f item 1)")
         if self.sde_ctrl_noise is not None or self.sde_ctrl_dropout is not None:
             raise NotImplementedError("sde_ctrl_noise / sde_ctrl_dropout are not set by any shipped config")
         if self.traj_per_sample != 1:
             x = x.repeat(self.traj_per_sample, 1, 1).reshape(-1, x.shape[-1])
         info = self._ctrl(False)
-        return train.lv_objective(self, make_plan(x.device), info, x, self._seed(seed), noise=noise,
-                                  particle_offset=particle_offset, group=group)
+        if self.method in ("lv", "lv_traj"):
+            return train.lv_objective(self, make_plan(x.device), info, x, self._seed(seed), noise=noise,
+                                      particle_offset=particle_offset, group=group)
+        if group is not None:
+            raise NotImplementedError("sharded training is built for method 'lv'")
+        if info.kind != N.CTRL_CLIPPED:
+            raise NotImplementedError("method 'kl' / 'kl_ito' is built for ClippedCtrl (base_zero_init): the adjoint of the "
+                                      "score-family controls also needs each target's Hessian-vector product (not built)")
+        if getattr(self, "_init_cost", False):
+            raise NotImplementedError("the discrete-time DIS loss has no 'kl' training rollout here (no shipped config uses it)")
+        # the prior's log_prob runs lrds_distr_eval on the device: the pre-pass's own value, which the kl form removes
+        rnd_start = None if initial_log_prob is None else initial_log_prob(x.detach().to(torch.float32)).reshape(-1)
+        return train.kl_objective(self, make_plan(x.device), info, x, self._seed(seed), noise=noise,
+                                  particle_offset=particle_offset, rnd_start=rnd_start)
 
     def __call__(self, ts, x, *args, **kwargs):
         raise NotImplementedError("training through this loss is not built (SURVEY.md 8f item 1): the linear losses "
-                                  "(EM / EI / DDPM-like reference losses, DDS, DIS) train with method 'lv'")
+                                  "(EM / EI / DDPM-like reference losses, DDS, DIS) train with method 'lv' or 'kl'")
 
     def load_state_dict(self, state_dict: dict):
         self.n_filtered = state_dict["n_filtered"]
@@ -475,7 +487,8 @@ class ExponentialIntegratorSDELoss(BaseOCLoss):
 
     def __call__(self, ts, x, terminal_unnorm_log_prob, reference_log_prob, **kw):
         """[TRAINING] (loss, metrics) of oc.py:1399-1431 (compute_ito_int = method != 'kl')."""
-        return self._train(lambda dev: self._plan(ts, dev, False, terminal_unnorm_log_prob, reference_log_prob, True), x, **kw)
+        ito = self.method != "kl"
+        return self._train(lambda dev: self._plan(ts, dev, False, terminal_unnorm_log_prob, reference_log_prob, ito), x, **kw)
 
     def simulate(self, ts, x, terminal_unnorm_log_prob, reference_log_prob, compute_ito_int: bool = False,
                  change_sde_ctrl: bool = False, return_traj: bool = False, use_ema: bool = False, noise=None,
@@ -554,18 +567,20 @@ class TimeReversalLoss(BaseOCLoss):
 
     def __call__(self, ts, x, terminal_unnorm_log_prob, initial_log_prob=None, **kw):
         """[TRAINING] (loss, metrics) of oc.py:1240-1272 (compute_ito_int = method != 'kl', train=True)."""
-        return self._train(lambda dev: self._plan(ts, dev, False, terminal_unnorm_log_prob, initial_log_prob, True, train=True),
-                           x, **kw)
+        ito = self.method != "kl"
+        return self._train(lambda dev: self._plan(ts, dev, False, terminal_unnorm_log_prob, initial_log_prob, ito, train=True),
+                           x, initial_log_prob=initial_log_prob, **kw)
 
     def simulate(self, ts, x, terminal_unnorm_log_prob, initial_log_prob=None, train: bool = True,
                  compute_ito_int: bool = False, change_sde_ctrl: bool = False, return_traj: bool = False,
                  use_ema: bool = False, noise=None, seed=None, particle_offset: int = 0):
         self._check_plain(change_sde_ctrl)
-        if train and self.method in ["kl", "kl_ito"]:
-            raise NotImplementedError("the kl training rollout starts the log-weight at 0 (oc.py:1164-1165) and is "
-                                      "differentiated through the trajectory: not built (SURVEY.md 8f item 1)")
         plan = self._plan(ts, x.device, use_ema, terminal_unnorm_log_prob, initial_log_prob, compute_ito_int, train=train)
-        return pack.run_rollout(plan, x, noise, self._seed(seed), particle_offset, return_traj)
+        x_T, rnd, xs = pack.run_rollout(plan, x, noise, self._seed(seed), particle_offset, return_traj)
+        if train and self.method in ["kl", "kl_ito"]:  # the kl training form starts the log-weight at 0 (oc.py:1164-1165);
+            # the train plan's pre-pass wrote log p_prior(x_0) with rnd_offset = 0, removed here through lrds_distr_eval
+            rnd = rnd - initial_log_prob(x.detach().to(torch.float32)).reshape(rnd.shape)
+        return x_T, rnd, xs
 
     def eval(self, ts, x, terminal_unnorm_log_prob, initial_log_prob=None, compute_weights: bool = True,
              return_traj: bool = True, use_ema: bool = True, **kw) -> Results:

@@ -23,6 +23,10 @@ by autograd through K sequential steps (~40-150 eager ops each).  Here
      for fp32-grade arithmetic throughout ("tf32x3", "fp32") take the same pass through torch autograd (large library
      GEMMs) - stated, not hidden.
 
+With method 'kl' / 'kl_ito' (kl_objective, ClippedCtrl) the SDE follows the non-detached control and the gradient runs
+through the trajectory: step 3 takes the cotangents d loss / d g_k that the reverse-time adjoint kernel lrds_adjoint
+computes from the stored trajectory (csrc/lrds_adjoint.cuh); everything else is shared with the LV objective.
+
 Nothing here runs on the CPU or imports the oracle.
 """
 from __future__ import annotations
@@ -245,6 +249,62 @@ def lv_weights(rnd: torch.Tensor, mask: torch.Tensor, group=None):
     return var.to(rnd.dtype), w.to(rnd.dtype)
 
 
+def _loss_weights(loss_obj, rnd: torch.Tensor, x_T: torch.Tensor):
+    """(loss, d loss / d rnd_b, metrics) of the reference's loss formula (compute_loss) on the B log-weights."""
+    rnd_leaf = rnd.detach().clone().requires_grad_(True)
+    with torch.enable_grad():
+        value, metrics = loss_obj.compute_loss(rnd_leaf, samples=x_T)
+        (w,) = torch.autograd.grad(value, rnd_leaf)  # zero for filtered particles
+    return value, w, metrics
+
+
+def _param_grads(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, xs: torch.Tensor, cot: torch.Tensor, weights,
+                 max_rows: int, cot_max: float | None = None):
+    """Gradients (aligned with the control's trainable parameters) of  sum_{k,b} <c_kb, g(t_k, x_kb)>  over the K stored
+    states xs [K, B, d], with c = cot, or (step_w_k row_w_b) cot for ``weights`` = (step_w [K], row_w [B]): the
+    weight-gradient kernel (lrds_mlp_grad) where it is built, else autograd over ``control_rows`` in slices of
+    ``max_rows`` rows.  ``cot_max`` >= max |cot| when known (saves a reduction)."""
+    dev = xs.device
+    K, B, d = xs.shape
+    params = [p for p in loss_obj.generative_ctrl.parameters() if p.requires_grad]
+    grads: list = [None] * len(params)
+    taus = pack.on_device(plan, "taus", dev)
+    step_w, row_w = weights if weights is not None else (None, None)
+
+    def dis_rows():  # time-only table columns of the DIS drift models (they do not depend on the parameters)
+        c = torch.zeros(K, N.STEP_BIAS1)
+        pack.dis_ctrl_rows(info, plan.taus, c)
+        return c
+    coef = pack.on_device(plan, "coef", dev, dis_rows)
+    step_rows = max(1, max_rows // B)
+
+    def score_of(k0, k1):  # the constant score factor of the control at the stored states of steps k0 .. k1 - 1
+        flat = xs[k0:k1].reshape(-1, d)
+        score = info.target.score(flat).reshape(k1 - k0, B, d)
+        if info.kind == N.CTRL_LERP:  # clipped_interpolated_score, models/reparam.py:170-183
+            score = torch.lerp(info.prior.score(flat).reshape(k1 - k0, B, d), score, coef[k0:k1, N.STEP_LERP, None, None])
+        return score
+
+    use_kernel = mlp_grad_applicable(info.base) and plan.spec.precision == N.PRECISION_F16X3
+    if use_kernel:  # the backbone's gradient by lrds_mlp_grad: one launch over all K x B stored states
+        grads = control_param_grads(info, params, taus[:K], xs, cot, step_w, None if row_w is None else row_w.reshape(-1),
+                                    coef, score_of, max_rows, cot_max=cot_max)
+    for k0 in range(0, K if not use_kernel else 0, step_rows):
+        k1 = min(K, k0 + step_rows)
+        xs_c = xs[k0:k1]
+        score = None
+        if info.kind != N.CTRL_CLIPPED:
+            score = info.target.score(xs_c.reshape(-1, d)).reshape(k1 - k0, B, d)
+            if info.kind == N.CTRL_LERP:  # clipped_interpolated_score, models/reparam.py:170-183
+                prior = info.prior.score(xs_c.reshape(-1, d)).reshape(k1 - k0, B, d)
+                score = torch.lerp(prior, score, coef[k0:k1, N.STEP_LERP, None, None])
+        c = cot[k0:k1] if weights is None else (step_w[k0:k1, None, None] * row_w.reshape(1, B, 1)) * cot[k0:k1]
+        with torch.enable_grad():
+            surrogate = (c * control_rows(info, taus[k0:k1], xs_c, score, coef[k0:k1])).sum()
+        _accumulate(grads, params, surrogate)
+    return params, grads
+
+
 def lv_objective(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, x: torch.Tensor, seed: int, noise=None,
                  particle_offset: int = 0, max_rows: int = 1 << 20, group=None):
     """(loss, metrics) like ``BaseOCLoss.__call__``: ``loss`` is a scalar whose ``backward()`` leaves the LV gradient in
@@ -268,54 +328,54 @@ def lv_objective(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, x: torch.Tensor
         value, w = lv_weights(rnd, mask, group)
         metrics = {"train/n_filtered_cumulative": loss_obj.n_filtered}
     else:
-        rnd_leaf = rnd.detach().clone().requires_grad_(True)
-        with torch.enable_grad():
-            value, metrics = loss_obj.compute_loss(rnd_leaf, samples=x_T)
-            (w,) = torch.autograd.grad(value, rnd_leaf)  # d loss / d rnd_b, zero for filtered particles
-    params = [p for p in loss_obj.generative_ctrl.parameters() if p.requires_grad]
-    grads: list = [None] * len(params)
-    taus = pack.on_device(plan, "taus", dev)
+        value, w, metrics = _loss_weights(loss_obj, rnd, x_T)
     ito_w = pack.on_device(plan, "ito_w", dev)
-
-    def dis_rows():  # time-only table columns of the DIS drift models (they do not depend on the parameters)
-        c = torch.zeros(K, N.STEP_BIAS1)
-        pack.dis_ctrl_rows(info, plan.taus, c)
-        return c
-    coef = pack.on_device(plan, "coef", dev, dis_rows)
-    step_rows = max(1, max_rows // B)
-
-    def score_of(k0, k1):  # the constant score factor of the control at the stored states of steps k0 .. k1 - 1
-        flat = xs[k0:k1].reshape(-1, d)
-        score = info.target.score(flat).reshape(k1 - k0, B, d)
-        if info.kind == N.CTRL_LERP:  # clipped_interpolated_score, models/reparam.py:170-183
-            score = torch.lerp(info.prior.score(flat).reshape(k1 - k0, B, d), score, coef[k0:k1, N.STEP_LERP, None, None])
-        return score
-
-    use_kernel = mlp_grad_applicable(info.base) and plan.spec.precision == N.PRECISION_F16X3
-    if use_kernel:  # the backbone's gradient by lrds_mlp_grad: one launch over all K x B stored states
-        # the generator's normals are bounded: Box-Muller on at most 32-bit uniforms, |z| <= sqrt(2 * 32 * ln 2) < 6.7
-        grads = control_param_grads(info, params, taus[:K], xs[:K], z, ito_w[:K], w.reshape(-1), coef, score_of, max_rows,
-                                    cot_max=7.0 if noise is None else None)
-    for k0 in range(0, K if not use_kernel else 0, step_rows):
-        k1 = min(K, k0 + step_rows)
-        xs_c = xs[k0:k1]
-        score = None
-        if info.kind != N.CTRL_CLIPPED:
-            score = info.target.score(xs_c.reshape(-1, d)).reshape(k1 - k0, B, d)
-            if info.kind == N.CTRL_LERP:  # clipped_interpolated_score, models/reparam.py:170-183
-                prior = info.prior.score(xs_c.reshape(-1, d)).reshape(k1 - k0, B, d)
-                score = torch.lerp(prior, score, coef[k0:k1, N.STEP_LERP, None, None])
-        cot = (ito_w[k0:k1, None, None] * w[None, :, :]) * z[k0:k1]
-        with torch.enable_grad():
-            surrogate = (cot * control_rows(info, taus[k0:k1], xs_c, score, coef[k0:k1])).sum()
-        for i, g in enumerate(torch.autograd.grad(surrogate, params, allow_unused=True)):
-            if g is not None:
-                grads[i] = g if grads[i] is None else grads[i] + g
+    # the generator's normals are bounded: Box-Muller on at most 32-bit uniforms, |z| <= sqrt(2 * 32 * ln 2) < 6.7
+    params, grads = _param_grads(loss_obj, plan, info, xs[:K], z, (ito_w[:K], w), max_rows,
+                                 cot_max=7.0 if noise is None else None)
     if group is not None:  # one all_reduce over the flattened gradients
         import torch.distributed as dist
         flat = torch.cat([(g if g is not None else torch.zeros_like(p)).reshape(-1) for g, p in zip(grads, params)])
         dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
         grads = [c.reshape(p.shape) for c, p in zip(flat.split([p.numel() for p in params]), params)]
+    return _InjectGrads.apply(value.detach(), grads, *params), metrics
+
+
+def adjoint(plan: pack.Plan, xs: torch.Tensor, w: torch.Tensor, seed: int, noise=None, particle_offset: int = 0):
+    """gbar [K, B, d] = d loss / d g_k of the pathwise ('kl' / 'kl_ito') gradient by the reverse-time kernel lrds_adjoint:
+    ``xs`` [K + 1, B, d] = the trajectory the rollout of ``plan`` wrote, ``w`` [B] = d loss / d rnd_b, ``noise`` = the
+    increments that rollout consumed (None: the kernel regenerates the in-kernel Philox draws of ``seed``)."""
+    dev = xs.device
+    K1, B, d = xs.shape
+    spec = N.Spec.from_buffer_copy(plan.spec)  # the cached plan is shared: never mutated here
+    spec.B = B
+    spec.status = pack.status_counters(dev).data_ptr()
+    cot = torch.empty(K1 - 1, B, d, device=dev, dtype=torch.float32)
+    rw = w.detach().to(dev, torch.float32).reshape(-1).contiguous()
+    z = None if noise is None else noise.detach().to(dev, torch.float32).contiguous()
+    with torch.cuda.device(dev):
+        N.check(N.lib().lrds_adjoint(C.byref(spec), N.ptr(xs.contiguous()), N.ptr(z), C.c_uint64(seed & (2 ** 64 - 1)),
+                                     C.c_uint64(particle_offset), N.ptr(rw), N.ptr(cot), N.stream_ptr(dev)))
+    return cot
+
+
+def kl_objective(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, x: torch.Tensor, seed: int, noise=None,
+                 particle_offset: int = 0, max_rows: int = 1 << 20, rnd_start=None):
+    """(loss, metrics) of method 'kl' / 'kl_ito' (the SDE follows the non-detached control, oc.py:83-103; loss =
+    mean(rnd[mask])): the fused rollout with its trajectory, d loss / d rnd from compute_loss, the reverse-time adjoint
+    (lrds_adjoint) for the cotangents gbar_k = d loss / d g_k, and the same parameter pass as lv_objective with
+    cot = gbar.  ``rnd_start`` [B]: subtracted from the rollout's log-weights (the DIS training form starts at 0, the
+    rollout at the prior log-density)."""
+    if rnd_start is not None and plan.spec.rnd_offset != 0.0:  # the training plans start at log p_prior(x_0) exactly
+        raise ValueError("rnd_start assumes a rollout whose initial cost has no state-independent offset (train=True)")
+    noise = None if noise is None else noise.detach().to(x.device, torch.float32).contiguous()
+    with torch.no_grad():
+        x_T, rnd, xs = pack.run_rollout(plan, x, noise, seed, particle_offset, True)
+        if rnd_start is not None:
+            rnd = rnd - rnd_start.reshape(rnd.shape)
+    value, w, metrics = _loss_weights(loss_obj, rnd, x_T)
+    cot = adjoint(plan, xs, w, seed, noise, particle_offset)
+    params, grads = _param_grads(loss_obj, plan, info, xs[:-1], cot, None, max_rows)
     return _InjectGrads.apply(value.detach(), grads, *params), metrics
 
 
