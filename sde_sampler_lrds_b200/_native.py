@@ -198,6 +198,11 @@ def ptr(t: torch.Tensor | None):
     return C.c_void_p(t.data_ptr())
 
 
+def seed_arg(seed: int):
+    """A Philox seed as the ABI's uint64 (taken modulo 2^64)."""
+    return C.c_uint64(seed & (2 ** 64 - 1))
+
+
 def stream_ptr(device=None):
     return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 

@@ -51,7 +51,7 @@ def mala_chains(target: Distribution, y_init: torch.Tensor, step_size, n_warmup_
     log_acc = torch.empty(S, Cn, device=dev, dtype=torch.float32) if return_log_acc else None
     with torch.cuda.device(dev):
         N.check(N.lib().lrds_mala(C.byref(distr), d, Cn, int(n_warmup_steps), int(n_mcmc_steps), int(bool(adapt_step_size)),
-                                  N.MCMC_RWMH if mcmc_type == "rwmh" else N.MCMC_MALA, N.ptr(y0), N.ptr(h), N.ptr(noise), N.ptr(unif), C.c_uint64(seed & (2 ** 64 - 1)),
+                                  N.MCMC_RWMH if mcmc_type == "rwmh" else N.MCMC_MALA, N.ptr(y0), N.ptr(h), N.ptr(noise), N.ptr(unif), N.seed_arg(seed),
                                   N.ptr(ys), N.ptr(log_acc), N.stream_ptr(dev)))
     del keep
     out = (ys, h.unsqueeze(-1))

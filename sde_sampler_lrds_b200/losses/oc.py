@@ -159,10 +159,7 @@ class BaseOCLoss:
         (kl_objective, ClippedCtrl).  ``initial_log_prob`` (DIS): the prior log-density the rollout starts the log-weight
         at, which the 'kl' training form leaves out."""
         from .. import train
-        if self.sde_ctrl_noise is not None or self.sde_ctrl_dropout is not None:
-            raise NotImplementedError("sde_ctrl_noise / sde_ctrl_dropout are not set by any shipped config")
-        if self.traj_per_sample != 1:
-            x = x.repeat(self.traj_per_sample, 1, 1).reshape(-1, x.shape[-1])
+        x = self._train_batch(x)
         info = self._ctrl(False)
         if self.method in ("lv", "lv_traj"):
             return train.lv_objective(self, make_plan(x.device), info, x, self._seed(seed), noise=noise,
@@ -174,10 +171,17 @@ class BaseOCLoss:
                                       "score-family controls also needs each target's Hessian-vector product (not built)")
         if getattr(self, "_init_cost", False):
             raise NotImplementedError("the discrete-time DIS loss has no 'kl' training rollout here (no shipped config uses it)")
-        # the prior's log_prob runs lrds_distr_eval on the device: the pre-pass's own value, which the kl form removes
-        rnd_start = None if initial_log_prob is None else initial_log_prob(x.detach().to(torch.float32)).reshape(-1)
+        rnd_start = None if initial_log_prob is None else _kl_start(initial_log_prob, x)
         return train.kl_objective(self, make_plan(x.device), info, x, self._seed(seed), noise=noise,
                                   particle_offset=particle_offset, rnd_start=rnd_start)
+
+    def _train_batch(self, x):
+        """The training batch: ``x`` repeated ``traj_per_sample`` times; control noise / dropout are refused."""
+        if self.sde_ctrl_noise is not None or self.sde_ctrl_dropout is not None:
+            raise NotImplementedError("sde_ctrl_noise / sde_ctrl_dropout are not set by any shipped config")
+        if self.traj_per_sample != 1:
+            x = x.repeat(self.traj_per_sample, 1, 1).reshape(-1, x.shape[-1])
+        return x
 
     def __call__(self, ts, x, *args, **kwargs):
         raise NotImplementedError("training through this loss is not built (SURVEY.md 8f item 1): the linear losses "
@@ -236,15 +240,42 @@ class BaseOCLoss:
             hit = self._grids[gkey] = (ts.detach().to("cpu", torch.float32).numpy().tobytes(), ts)  # keeps the storage alive
         return hit[0]
 
-    def _key(self, tag, ts, device, info, extra=(), objs=()):
+    def _key(self, tag, ts, device, info, terminal_unnorm_log_prob, objs=()):
         """(static key, control-parameter versions, keyed objects).  ``objs``: further objects the plan is packed from
-        (references, priors, the owner of the terminal log-density)."""
+        (references, priors, the SDE) besides the terminal target."""
         vers = tuple((p.data_ptr(), p._version) for p in info.base.parameters())
         if info.score_model is not None:
             vers += tuple((p.data_ptr(), p._version) for p in info.score_model.parameters())
-        refs = (info.target, info.sde, info.prior) + tuple(objs)
-        return ((tag, self._grid_bytes(ts), str(device), self.precision or pack.default_precision(), info.kind, extra,
+        refs = (info.target, info.sde, info.prior, _terminal_target(terminal_unnorm_log_prob)) + tuple(objs)
+        fid = (_fid(terminal_unnorm_log_prob), _fid_clip(terminal_unnorm_log_prob))
+        return ((tag, self._grid_bytes(ts), str(device), self.precision or pack.default_precision(), info.kind, fid,
                  tuple(_state(o) for o in refs)), vers, refs)
+
+    def _build_plan(self, tag, ts, device, use_ema, terminal_unnorm_log_prob, ref0, steps, objs=(), prior=None,
+                    single_gaussian=None):
+        """The cached plan of one rollout.  Every loss packs the control, the terminal target, the step table with the
+        control's time-only columns and spec.ref_0 (from ``ref0``: the reference term or the prior) the same way;
+        ``steps(spec, keep, tsc, pairs)`` does the rest: it sets the loss's own spec fields and returns (table, taus),
+        the step rows and the times the control is evaluated at in each row.  ``tag`` and ``objs`` join the cache key;
+        ``prior`` and ``single_gaussian`` go to pack.fill_ctrl and pack.fill_ref0."""
+        info = self._ctrl(use_ema)
+        key = self._key(tag, ts, device, info, terminal_unnorm_log_prob, objs=(ref0,) + tuple(objs))
+
+        def build():
+            tsc, pairs = pack._scalar_rows(ts)
+            spec = pack.new_spec(self.precision)
+            keep: list = []
+            weights = pack.fill_ctrl(spec, info, device, keep, prior=prior)
+            _terminal(spec, keep, device, terminal_unnorm_log_prob, info)
+            spec.K = len(pairs)
+            table, taus = steps(spec, keep, tsc, pairs)
+            spec_table = pack.finish_table(table, info, taus, device)
+            spec.steps = spec_table.data_ptr()
+            pack.fill_ref0(spec, ref0, device, keep, single_gaussian)
+            linear = spec.kind in (N.ROLLOUT_LINEAR, N.ROLLOUT_EUBO_LINEAR)
+            return pack.Plan(spec, keep, weights, spec_table, rows=table.shape[0], noise_steps=spec.K, taus=taus,
+                             ito_w=pack.ito_weights(table, spec.ito_form) if linear else None)
+        return self._cached(key, build, info, device)
 
 
 def _terminal(spec, keep, device, terminal_unnorm_log_prob, info):
@@ -258,6 +289,12 @@ def _terminal(spec, keep, device, terminal_unnorm_log_prob, info):
     spec.target = distr
     keep.append(k)
     spec.clip_target = float(clip_t) if clip_t is not None else 0.0
+
+
+def _kl_start(initial_log_prob, x):
+    """log p_prior(x_0) [B], by lrds_distr_eval: the DIS rollout starts its log-weight there (the pre-pass of its train
+    plan, rnd_offset = 0), the 'kl' training form at 0 (oc.py:1164-1165), so the kl form subtracts it."""
+    return initial_log_prob(x.detach().to(torch.float32)).reshape(-1)
 
 
 class EMReferenceSDELoss(BaseOCLoss):
@@ -290,24 +327,14 @@ class EMReferenceSDELoss(BaseOCLoss):
     def _plan(self, ts, device, use_ema, terminal_unnorm_log_prob, reference_log_prob, eubo):
         if self._variant == "em" and not self.use_rescaling:
             raise NotImplementedError("use_rescaling=False is unreachable from the shipped configs (SURVEY.md App. B.4)")
-        info = self._ctrl(use_ema)
         ref = _resolve_reference(self.reference_ctrl)
-        ref0, _ = pack.resolve_log_prob(reference_log_prob)
-        key = self._key((self._variant, eubo, self._init_cost), ts, device, info, (_fid(terminal_unnorm_log_prob), _fid_clip(terminal_unnorm_log_prob)),
-                        objs=(ref, ref0, _terminal_target(terminal_unnorm_log_prob), self.sde))
+        if eubo and ref is None and not self._init_cost:
+            raise NotImplementedError("compute_eubo needs a reference control (the reference calls it unconditionally)")
 
-        def build():
-            if eubo and ref is None and not self._init_cost:
-                raise NotImplementedError("compute_eubo needs a reference control (the reference calls it unconditionally)")
+        def steps(spec, keep, tsc, pairs):
             sde = self.sde.host()
-            tsc, pairs = pack._scalar_rows(ts)
             T = tsc[-1]
             K = len(pairs)
-            spec = pack.new_spec(self.precision)
-            keep: list = []
-            pack.fill_ctrl(spec, info, device, keep)
-            _terminal(spec, keep, device, terminal_unnorm_log_prob, info)
-            spec.K = K
             spec.kind = N.ROLLOUT_EUBO_LINEAR if eubo else N.ROLLOUT_LINEAR
             # DDPM-like compute_eubo is the EM formula without the 1/sigma rescaling of the control (oc.py:571-582, 343-346)
             em_formulas = self._variant == "em" or (eubo and self._variant == "ddpm")
@@ -338,20 +365,15 @@ class EMReferenceSDELoss(BaseOCLoss):
                     else:  # oc.py:560-564
                         om = sde.omega(s, t)
                         row[N.STEP_W_COST], row[N.STEP_W_ITO] = om, torch.sqrt(om)
-            spec_table = pack.finish_table(table, info, taus, device)
-            spec.steps = spec_table.data_ptr()
-            keep.append(spec_table)
             if ref is not None:
                 if ref.dim != spec.d:
                     raise ValueError("reference dimension differs from the model's")
                 blk = ref.block_at(taus, device)
                 fill_gmm(spec.ref_t, blk, stepped=True)
                 keep.append(blk)
-            blk0 = pack.gauss_block_from(ref0, device)
-            fill_gmm(spec.ref_0, blk0)
-            keep.append(blk0)
-            return pack.Plan(spec, keep, rows=K, noise_steps=K, taus=taus, ito_w=pack.ito_weights(table, spec.ito_form))
-        return self._cached(key, build, info, device)
+            return table, taus
+        return self._build_plan((self._variant, eubo, self._init_cost), ts, device, use_ema, terminal_unnorm_log_prob,
+                                pack.resolve_log_prob(reference_log_prob)[0], steps, objs=(ref, self.sde))
 
     def __call__(self, ts, x, terminal_unnorm_log_prob, reference_log_prob, **kw):
         """[TRAINING] (loss, metrics) of oc.py:364-394."""
@@ -446,24 +468,12 @@ class ExponentialIntegratorSDELoss(BaseOCLoss):
         self.sigma = sigma
 
     def _plan(self, ts, device, use_ema, terminal_unnorm_log_prob, reference_log_prob, compute_ito_int):
-        info = self._ctrl(use_ema)
-        ref0, _ = pack.resolve_log_prob(reference_log_prob)
-        key = self._key(("dds", bool(compute_ito_int), self.alpha, self.sigma), ts, device, info,
-                        (_fid(terminal_unnorm_log_prob), _fid_clip(terminal_unnorm_log_prob)),
-                        objs=(ref0, _terminal_target(terminal_unnorm_log_prob)))
-
-        def build():
-            tsc, pairs = pack._scalar_rows(ts)
-            K = len(pairs)
-            spec = pack.new_spec(self.precision)
-            keep: list = []
-            pack.fill_ctrl(spec, info, device, keep)
-            _terminal(spec, keep, device, terminal_unnorm_log_prob, info)
-            spec.K, spec.kind = K, N.ROLLOUT_LINEAR
+        def steps(spec, keep, tsc, pairs):
+            spec.kind = N.ROLLOUT_LINEAR
             spec.update_form = N.UPDATE_AXPY
             spec.ito_form = N.ITO_DDS if compute_ito_int else N.ITO_NONE
             spec.has_ref_ctrl = 0
-            table = torch.zeros(K, N.STEP_STRIDE)
+            table = torch.zeros(len(pairs), N.STEP_STRIDE)
             for k, (s, t) in enumerate(pairs):  # oc.py:1366-1383
                 row = table[k]
                 dt = t - s
@@ -476,14 +486,9 @@ class ExponentialIntegratorSDELoss(BaseOCLoss):
                 row[N.STEP_W_ITO] = beta_k
                 row[N.STEP_SIGU] = self.sigma
                 row[N.STEP_DT], row[N.STEP_SQRT_DT] = dt, dt.sqrt()
-            spec_table = pack.finish_table(table, info, tsc[:-1], device)
-            spec.steps = spec_table.data_ptr()
-            keep.append(spec_table)
-            blk0 = pack.gauss_block_from(ref0, device)
-            fill_gmm(spec.ref_0, blk0)
-            keep.append(blk0)
-            return pack.Plan(spec, keep, rows=K, noise_steps=K, taus=tsc[:-1], ito_w=pack.ito_weights(table, spec.ito_form))
-        return self._cached(key, build, info, device)
+            return table, tsc[:-1]
+        return self._build_plan(("dds", bool(compute_ito_int), self.alpha, self.sigma), ts, device, use_ema,
+                                terminal_unnorm_log_prob, pack.resolve_log_prob(reference_log_prob)[0], steps)
 
     def __call__(self, ts, x, terminal_unnorm_log_prob, reference_log_prob, **kw):
         """[TRAINING] (loss, metrics) of oc.py:1399-1431 (compute_ito_int = method != 'kl')."""
@@ -523,25 +528,15 @@ class TimeReversalLoss(BaseOCLoss):
         self.use_rescaling = use_rescaling
 
     def _plan(self, ts, device, use_ema, terminal_unnorm_log_prob, initial_log_prob, compute_ito_int, train=False):
-        info = self._ctrl(use_ema)
         prior, _ = pack.resolve_log_prob(initial_log_prob)
-        key = self._key(("dis", bool(compute_ito_int), bool(train)), ts, device, info,
-                        (_fid(terminal_unnorm_log_prob), _fid_clip(terminal_unnorm_log_prob)),
-                        objs=(prior, _terminal_target(terminal_unnorm_log_prob), self.sde))
 
-        def build():
+        def steps(spec, keep, tsc, pairs):
             sde = self.sde.host()
-            tsc, pairs = pack._scalar_rows(ts)
-            K = len(pairs)
-            spec = pack.new_spec(self.precision)
-            keep: list = []
-            pack.fill_ctrl(spec, info, device, keep, prior=prior)
-            _terminal(spec, keep, device, terminal_unnorm_log_prob, info)
-            spec.K, spec.kind = K, N.ROLLOUT_LINEAR
+            spec.kind = N.ROLLOUT_LINEAR
             spec.update_form = N.UPDATE_EM
             spec.ito_form = N.ITO_EM if compute_ito_int else N.ITO_NONE
             spec.has_ref_ctrl = 0
-            table = torch.zeros(K, N.STEP_STRIDE)
+            table = torch.zeros(len(pairs), N.STEP_STRIDE)
             div = torch.zeros(())
             for k, (s, t) in enumerate(pairs):  # oc.py:1171-1230
                 row = table[k]
@@ -552,18 +547,12 @@ class TimeReversalLoss(BaseOCLoss):
                 row[N.STEP_W_COST] = 0.5 * dt
                 row[N.STEP_DT], row[N.STEP_SQRT_DT] = dt, dt.sqrt()
                 div = div - sde.int_drift_coeff_t(s, t) * spec.d  # rnd -= sde.drift_div_int(s, t, x), train=False (1217-1218)
-            spec_table = pack.finish_table(table, info, tsc[:-1], device)
-            spec.steps = spec_table.data_ptr()
-            keep.append(spec_table)
-            blk0 = pack.gauss_block_from(prior, device)
-            if blk0[1].shape[0] != 1:
-                raise NotImplementedError("DIS needs a Gaussian prior (solver/oc.py:207-208)")
-            fill_gmm(spec.ref_0, blk0)
-            keep.append(blk0)
             # the training rollout leaves the divergence integral out (`if not train`, oc.py:1217)
             spec.init_cost, spec.rnd_offset = 1, 0.0 if train else float(div)
-            return pack.Plan(spec, keep, rows=K, noise_steps=K, taus=tsc[:-1], ito_w=pack.ito_weights(table, spec.ito_form))
-        return self._cached(key, build, info, device)
+            return table, tsc[:-1]
+        return self._build_plan(("dis", bool(compute_ito_int), bool(train)), ts, device, use_ema, terminal_unnorm_log_prob,
+                                prior, steps, objs=(self.sde,), prior=prior,
+                                single_gaussian="DIS needs a Gaussian prior (solver/oc.py:207-208)")
 
     def __call__(self, ts, x, terminal_unnorm_log_prob, initial_log_prob=None, **kw):
         """[TRAINING] (loss, metrics) of oc.py:1240-1272 (compute_ito_int = method != 'kl', train=True)."""
@@ -577,9 +566,8 @@ class TimeReversalLoss(BaseOCLoss):
         self._check_plain(change_sde_ctrl)
         plan = self._plan(ts, x.device, use_ema, terminal_unnorm_log_prob, initial_log_prob, compute_ito_int, train=train)
         x_T, rnd, xs = pack.run_rollout(plan, x, noise, self._seed(seed), particle_offset, return_traj)
-        if train and self.method in ["kl", "kl_ito"]:  # the kl training form starts the log-weight at 0 (oc.py:1164-1165);
-            # the train plan's pre-pass wrote log p_prior(x_0) with rnd_offset = 0, removed here through lrds_distr_eval
-            rnd = rnd - initial_log_prob(x.detach().to(torch.float32)).reshape(rnd.shape)
+        if train and self.method in ["kl", "kl_ito"]:
+            rnd = rnd - _kl_start(initial_log_prob, x).reshape(rnd.shape)
         return x_T, rnd, xs
 
     def eval(self, ts, x, terminal_unnorm_log_prob, initial_log_prob=None, compute_weights: bool = True,
@@ -603,26 +591,17 @@ class ControlledLangevinSDELoss(BaseOCLoss):
             raise NotImplementedError("use_rescaling=False is unreachable from the shipped configs (SURVEY.md App. B.4)")
         if not isinstance(self.sde, ControlledLangevinSDE):
             raise NotImplementedError("CMCD needs a ControlledLangevinSDE")
-        info = self._ctrl(use_ema)
         prior, _ = pack.resolve_log_prob(initial_log_prob)
-        key = self._key(("cmcd", eubo), ts, device, info, (_fid(terminal_unnorm_log_prob), _fid_clip(terminal_unnorm_log_prob)),
-                        objs=(prior, _terminal_target(terminal_unnorm_log_prob), self.sde))
 
-        def build():
+        def steps(spec, keep, tsc, pairs):
             sde = self.sde
-            tsc, pairs = pack._scalar_rows(ts)
             K = len(pairs)
-            spec = pack.new_spec(self.precision)
-            keep: list = []
-            pack.fill_ctrl(spec, info, device, keep)
-            _terminal(spec, keep, device, terminal_unnorm_log_prob, info)
             tgt = getattr(sde.target_score, "__self__", None)
             pri = getattr(sde.prior_score, "__self__", None)
             target, _ = pack.resolve_log_prob(terminal_unnorm_log_prob)
             if tgt is not target or pri is not prior:
                 raise NotImplementedError("ControlledLangevinSDE scores must be the bound .score of the rollout's "
                                           "target and prior distributions")
-            spec.K = K
             spec.kind = N.ROLLOUT_EUBO_CMCD if eubo else N.ROLLOUT_CMCD
             spec.cmcd_diff = float(sde.diff_coeff)
             spec.cmcd_clip = float(sde.clip_score) if sde.clip_score is not None else 0.0
@@ -633,16 +612,10 @@ class ControlledLangevinSDELoss(BaseOCLoss):
                 if k < K:
                     dt = tsc[k + 1] - tsc[k]
                     table[k, N.STEP_DT], table[k, N.STEP_SQRT_DT] = dt, dt.sqrt()
-            spec_table = pack.finish_table(table, info, tsc, device)
-            spec.steps = spec_table.data_ptr()
-            keep.append(spec_table)
-            blk0 = pack.gauss_block_from(prior, device)
-            if blk0[1].shape[0] != 1:
-                raise NotImplementedError("CMCD needs a (diagonal) Gaussian prior (solver/oc.py:276-277)")
-            fill_gmm(spec.ref_0, blk0)
-            keep.append(blk0)
-            return pack.Plan(spec, keep, rows=K + 1, noise_steps=K, taus=tsc)
-        return self._cached(key, build, info, device)
+            return table, tsc
+        return self._build_plan(("cmcd", eubo), ts, device, use_ema, terminal_unnorm_log_prob, prior, steps,
+                                objs=(self.sde,),
+                                single_gaussian="CMCD needs a (diagonal) Gaussian prior (solver/oc.py:276-277)")
 
     def __call__(self, ts, x, terminal_unnorm_log_prob, initial_log_prob=None, noise=None, seed=None,
                  particle_offset: int = 0):
@@ -650,10 +623,7 @@ class ControlledLangevinSDELoss(BaseOCLoss):
         from .. import train
         if self.method not in ("lv", "lv_traj"):
             raise NotImplementedError("method 'kl' differentiates through the trajectory: not built (SURVEY.md 8f item 1)")
-        if self.sde_ctrl_noise is not None or self.sde_ctrl_dropout is not None:
-            raise NotImplementedError("sde_ctrl_noise / sde_ctrl_dropout are not set by any shipped config")
-        if self.traj_per_sample != 1:
-            x = x.repeat(self.traj_per_sample, 1, 1).reshape(-1, x.shape[-1])
+        x = self._train_batch(x)
         info = self._ctrl(False)
         if info.kind not in (N.CTRL_CLIPPED, N.CTRL_SCORE):
             raise NotImplementedError("CMCD trains ClippedCtrl / ScoreCtrl drift models")

@@ -96,16 +96,17 @@ def resolve_log_prob(fn):
     raise NotImplementedError("log-density callable must be a bound method of a kernel-backed Distribution")
 
 
-def time_rows(info: CtrlInfo, taus: torch.Tensor, device="cpu"):
-    """Rows (bias1[S][64], gamma[S]) of the time-only parts of the control for times ``taus``, evaluated on ``device``."""
-    bias1 = info.base.bias_rows(taus, device)
+def time_columns(table: torch.Tensor, info: CtrlInfo, taus: torch.Tensor):
+    """Writes the parameter-dependent time-only columns of the control for times ``taus`` into the step table, evaluated
+    on the table's device: bias1 [S][64] = input_embed.bias + TimeEmbed(tau) and gamma [S] = the clipped score-model
+    factor (1 without one)."""
+    dev = table.device
+    table[:, N.STEP_BIAS1:N.STEP_BIAS1 + N.CHANNELS] = info.base.bias_rows(taus, dev)
     if info.kind != N.CTRL_CLIPPED and info.score_model is not None:
-        gamma = info.score_model.rows(taus, device).reshape(-1)
-        if info.clip_model is not None:
-            gamma = gamma.clip(-info.clip_model, info.clip_model)
+        gamma = info.score_model.rows(taus, dev).reshape(-1)
+        table[:, N.STEP_GAMMA] = gamma if info.clip_model is None else gamma.clip(-info.clip_model, info.clip_model)
     else:
-        gamma = torch.ones(taus.numel(), device=device)
-    return bias1, gamma
+        table[:, N.STEP_GAMMA] = 1.0
 
 
 def dis_ctrl_rows(info: CtrlInfo, taus: torch.Tensor, table: torch.Tensor):
@@ -123,7 +124,9 @@ def dis_ctrl_rows(info: CtrlInfo, taus: torch.Tensor, table: torch.Tensor):
 
 
 def fill_ctrl(spec: N.Spec, info: CtrlInfo, device, keep: list, prior: Distribution | None = None):
-    """``prior`` = the distribution that fills spec.ref_0 when it is the rollout's prior (DIS); LerpCtrl needs it."""
+    """Fills the control's fields of the spec and returns the keepalive of the weight block spec.mlp points into
+    (Plan.weights).  ``prior`` = the distribution that fills spec.ref_0 when it is the rollout's prior (DIS); LerpCtrl
+    needs it."""
     if info.kind == N.CTRL_LERP and prior is not info.prior:
         raise NotImplementedError("LerpCtrl runs in the DIS rollout from the prior whose score it interpolates "
                                   "(TimeReversalLoss with initial_log_prob = that prior's log_prob)")
@@ -131,9 +134,8 @@ def fill_ctrl(spec: N.Spec, info: CtrlInfo, device, keep: list, prior: Distribut
     spec.clip_model = float(info.clip_model) if info.clip_model is not None else 0.0
     spec.clip_score = float(info.clip_score) if info.clip_score is not None else 0.0
     spec.scale_score = float(info.scale_score)
-    mlp, k = info.base.lrds_mlp(device, spec.precision)
+    mlp, weights = info.base.lrds_mlp(device, spec.precision)
     spec.mlp = mlp
-    keep.append(k)
     spec.d = info.base.dim
     if info.target is not None:
         if info.target.dim != info.base.dim:
@@ -141,6 +143,7 @@ def fill_ctrl(spec: N.Spec, info: CtrlInfo, device, keep: list, prior: Distribut
         distr, k2 = info.target.lrds_distr(device)
         spec.target = distr
         keep.append(k2)
+    return weights
 
 
 def new_spec(precision: str | None = None) -> N.Spec:
@@ -157,22 +160,15 @@ def ctrl_forward(module, t: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
     info = resolve_ctrl(module)
     keep: list = []
     spec = new_spec("fp32")
-    fill_ctrl(spec, info, x.device, keep, prior=info.prior)
+    keep.append(fill_ctrl(spec, info, x.device, keep, prior=info.prior))
     if info.kind == N.CTRL_LERP:
-        blk0 = gauss_block_from(info.prior, x.device)
-        fill_gmm(spec.ref_0, blk0)
-        keep.append(blk0)
+        fill_ref0(spec, info.prior, x.device, keep)
     t = torch.as_tensor(t)
     if t.numel() != 1:
         if not bool((t.reshape(-1) == t.reshape(-1)[0]).all()):
             raise NotImplementedError("drift models are evaluated at one time per call (as every solver does)")
         t = t.reshape(-1)[0]
-    table = torch.zeros(1, N.STEP_STRIDE)
-    bias1, gamma = time_rows(info, t.reshape(1))
-    table[0, N.STEP_BIAS1:N.STEP_BIAS1 + N.CHANNELS] = bias1[0]
-    table[0, N.STEP_GAMMA] = gamma[0]
-    dis_ctrl_rows(info, t.reshape(1), table)
-    table = table.to(x.device)
+    table = finish_table(torch.zeros(1, N.STEP_STRIDE), info, t.reshape(1), x.device)
     spec.steps = table.data_ptr()
     lead = x.shape[:-1]
     xf = x.detach().reshape(-1, spec.d).to(torch.float32).contiguous()
@@ -189,10 +185,12 @@ def ctrl_forward(module, t: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
 @dataclass
 class Plan:
     spec: N.Spec
-    keep: list = field(default_factory=list)
+    keep: list                          # the further buffers the spec points into (target, reference and prior blocks)
+    weights: object                     # the weight block / tensor-core image spec.mlp points into (fill_ctrl, refresh_ctrl)
+    steps: torch.Tensor                 # [rows, STEP_STRIDE] device: the step table spec.steps points at (finish_table)
     rows: int = 0
     noise_steps: int = 0
-    taus: torch.Tensor | None = None    # [K] host: the time the control is evaluated at in step k (training, train.py)
+    taus: torch.Tensor | None = None    # [rows] host: the time the control is evaluated at in row k (finish_table, train.py)
     ito_w: torch.Tensor | None = None   # [K] host: the weight of <g, z> in the log-weight of step k
     dev_cache: dict = field(default_factory=dict)  # device copies of host-side rows, made once per plan (on_device)
 
@@ -223,43 +221,38 @@ def _scalar_rows(ts: torch.Tensor):
     return ts, list(zip(ts[:-1], ts[1:]))
 
 
-def gauss_block_from(distr: Distribution, device):
-    """(logc, mu, ivar) block of a diagonal Gaussian / mixture Distribution (for ref_0 / the CMCD prior), or the
-    FullBlock of a full-covariance one (GaussFull / GMMFull: the RDS reference term ref_0; the CMCD / DIS priors and
-    LerpCtrl are refused for it by the library)."""
+def fill_ref0(spec: N.Spec, distr: Distribution, device, keep: list, single_gaussian: str | None = None):
+    """Fills spec.ref_0 (the RDS / DDS reference term, the CMCD / DIS prior, LerpCtrl's prior) from the (logc, mu, ivar)
+    block of a diagonal Gaussian / mixture Distribution, or the FullBlock of a full-covariance one (GaussFull / GMMFull:
+    the RDS reference term; the CMCD / DIS priors and LerpCtrl are refused for it by the library).
+    ``single_gaussian``: the refusal raised when ``distr`` has more than one component."""
     if isinstance(distr, GMMFull):
-        return distr.block(device)
-    if not isinstance(distr, GMM):
+        blk = distr.block(device)
+    elif isinstance(distr, GMM):
+        blk = gmm_block(distr.loc, torch.square(distr.scale), distr.mixture_weights, device)
+    else:
         raise NotImplementedError(f"{type(distr).__name__} cannot serve as a Gaussian reference / prior here")
-    return gmm_block(distr.loc, torch.square(distr.scale), distr.mixture_weights, device)
+    if single_gaussian is not None and blk[1].shape[0] != 1:
+        raise NotImplementedError(single_gaussian)
+    fill_gmm(spec.ref_0, blk)
+    keep.append(blk)
 
 
-def finish_table(table: torch.Tensor, info: CtrlInfo, taus: torch.Tensor, device):
-    bias1, gamma = time_rows(info, taus)
-    table[:, N.STEP_BIAS1:N.STEP_BIAS1 + N.CHANNELS] = bias1
-    table[:, N.STEP_GAMMA] = gamma
+def finish_table(table: torch.Tensor, info: CtrlInfo, taus: torch.Tensor, device) -> torch.Tensor:
+    """The host step table with the control's time-only columns for times ``taus`` written in, copied to ``device``."""
+    time_columns(table, info, taus)
     dis_ctrl_rows(info, taus, table)
-    out = table.contiguous().to(device)
-    out._lrds_ctrl_taus = taus.detach().clone()  # refresh_ctrl re-evaluates the parameter-dependent columns at these times
-    return out
+    return table.contiguous().to(device)
 
 
 def refresh_ctrl(plan: "Plan", info: CtrlInfo, device):
-    """Re-packs what depends on the control's parameters into a cached plan: the weight block / tensor-core image
-    (keep[0], set by fill_ctrl) and the TimeEmbed columns of the device table (bias rows, gamma), in place and ordered
-    on the current stream behind earlier launches that read them.  The rows are evaluated on the device here (no
-    parameter round trip through the host in a training step); a freshly built plan evaluates them with the same torch
-    ops on the host, which agrees to float32 rounding."""
-    spec = plan.spec
-    mlp, k = info.base.lrds_mlp(device, spec.precision)
-    spec.mlp = mlp
-    plan.keep[0] = k
-    table = next(t for t in plan.keep if isinstance(t, torch.Tensor) and hasattr(t, "_lrds_ctrl_taus"))
-    if not hasattr(table, "_lrds_ctrl_taus_dev"):  # one copy per plan: a pageable host-to-device copy drains the stream
-        table._lrds_ctrl_taus_dev = table._lrds_ctrl_taus.to(table.device)
-    bias1, gamma = time_rows(info, table._lrds_ctrl_taus_dev, table.device)
-    table[:, N.STEP_BIAS1:N.STEP_BIAS1 + N.CHANNELS] = bias1
-    table[:, N.STEP_GAMMA] = gamma
+    """Re-packs what depends on the control's parameters into a cached plan: the weight block / tensor-core image and
+    the TimeEmbed columns of the device table (bias rows, gamma) at the plan's times, in place and ordered on the
+    current stream behind earlier launches that read them.  The rows are evaluated on the device here (no parameter
+    round trip through the host in a training step); a freshly built plan evaluates them with the same torch ops on the
+    host, which agrees to float32 rounding."""
+    plan.spec.mlp, plan.weights = info.base.lrds_mlp(device, plan.spec.precision)
+    time_columns(plan.steps, info, on_device(plan, "taus", plan.steps.device))
 
 
 _status: dict = {}
@@ -307,7 +300,7 @@ def run_rollout(plan: Plan, x0: torch.Tensor, noise: torch.Tensor | None, seed: 
     rnd = torch.empty(B, device=dev, dtype=torch.float32)
     traj = torch.empty(spec.K + 1, B, d, device=dev, dtype=torch.float32) if return_traj else None
     with torch.cuda.device(dev):
-        N.check(N.lib().lrds_rollout(C.byref(spec), N.ptr(xf), N.ptr(noise), C.c_uint64(seed & (2 ** 64 - 1)),
+        N.check(N.lib().lrds_rollout(C.byref(spec), N.ptr(xf), N.ptr(noise), N.seed_arg(seed),
                                      C.c_uint64(particle_offset), N.ptr(x_out), N.ptr(rnd), N.ptr(traj),
                                      N.stream_ptr(dev)))
     return x_out, rnd.unsqueeze(-1), traj

@@ -77,6 +77,38 @@ def control_rows(info: pack.CtrlInfo, taus: torch.Tensor, xs: torch.Tensor, scor
     return g + sc
 
 
+def control_score(info: pack.CtrlInfo, xs: torch.Tensor, coef: torch.Tensor | None) -> torch.Tensor:
+    """The constant score factor of the control (``score`` of control_rows) at stored states xs [S, B, d]: the target's
+    score, for LerpCtrl interpolated toward the prior's with coef[:, STEP_LERP] (clipped_interpolated_score,
+    models/reparam.py:170-183)."""
+    S, B, d = xs.shape
+    flat = xs.reshape(-1, d)
+    score = info.target.score(flat).reshape(S, B, d)
+    if info.kind == N.CTRL_LERP:
+        score = torch.lerp(info.prior.score(flat).reshape(S, B, d), score, coef[:, N.STEP_LERP, None, None])
+    return score
+
+
+def cotangent_bound(cot: torch.Tensor, step_w=None, row_w=None, cot_max: float | None = None) -> torch.Tensor:
+    """max |cot| max |step_w| max |row_w| >= max |cot * step_w * row_w| (the fp16 operand scale of mlp_grad), a 0-dim
+    device tensor: no host round trip.  ``cot_max`` >= max |cot| when known (saves a reduction)."""
+    dev = cot.device
+    bound = cot.abs().max() if cot_max is None else torch.full((), float(cot_max), device=dev)
+    if step_w is not None:
+        bound = bound * step_w.abs().max().to(dev)
+    if row_w is not None:
+        bound = bound * row_w.abs().max()
+    return bound
+
+
+def _weight_args(dev, step_w, row_w, clip):
+    """(step_w, row_w, clip) as lrds_mlp_grad / lrds_score_cot_sums take them: fp32 device vectors or None (NULL), and
+    the clip bound with 0 for none."""
+    def vec(w):
+        return None if w is None else w.detach().to(dev, torch.float32).reshape(-1).contiguous()
+    return vec(step_w), vec(row_w), float(clip) if clip is not None else 0.0
+
+
 def mlp_grad_applicable(base) -> bool:
     """The weight-gradient kernel (lrds_mlp_grad) is built for the FourierMLP shapes d <= 64, at most 2 hidden layers."""
     return hasattr(base, "lrds_mlp") and N.lib().lrds_mlp_grad_floats(base.dim, len(base.hidden_layer)) > 0
@@ -103,29 +135,22 @@ def mlp_grad(base, bias1: torch.Tensor, xs: torch.Tensor, cot: torch.Tensor, cli
     mlp, keep = base.lrds_mlp(dev, N.PRECISION_F16X3)
     xs, cot = xs.contiguous(), cot.contiguous()
     bias1 = bias1.detach().to(dev, torch.float32).contiguous()
-    if cot_bound is None:
-        cot_bound = cot.abs().max()
-        if step_w is not None:
-            cot_bound = cot_bound * step_w.abs().max().to(dev)
-        if row_w is not None:
-            cot_bound = cot_bound * row_w.abs().max()
+    bound = cotangent_bound(cot, step_w, row_w) if cot_bound is None else cot_bound
     scale, scale_dev = 1.0, None
-    if torch.is_tensor(cot_bound):  # 2^floor(log2(4 / bound)) on the device; 1 for a zero / non-finite bound
-        bnd = cot_bound.detach().to(dev, torch.float32).reshape(())
+    if torch.is_tensor(bound):  # 2^floor(log2(4 / bound)) on the device; 1 for a zero / non-finite bound
+        bnd = bound.detach().to(dev, torch.float32).reshape(())
         scale_dev = torch.exp2(torch.floor(torch.log2(4.0 / bnd)))
         scale_dev = torch.where(torch.isfinite(scale_dev) & (scale_dev > 0), scale_dev, torch.ones_like(scale_dev)).reshape(1)
     else:
-        scale = pow2_scale(float(cot_bound))
+        scale = pow2_scale(float(bound))
     L = N.lib()
     flat = torch.empty(int(L.lrds_mlp_grad_floats(d, nh)), device=dev, dtype=torch.float32)
     dbias1 = torch.empty(S, N.CHANNELS, device=dev, dtype=torch.float32)
     scratch = torch.empty(int(L.lrds_mlp_grad_scratch_floats(d, nh, S, B)), device=dev, dtype=torch.float32)
-    sw = None if step_w is None else step_w.detach().to(dev, torch.float32).contiguous()
-    rw = None if row_w is None else row_w.detach().to(dev, torch.float32).reshape(-1).contiguous()
+    sw, rw, clip = _weight_args(dev, step_w, row_w, clip)
     with torch.cuda.device(dev):
-        N.check(L.lrds_mlp_grad(C.byref(mlp), N.ptr(bias1), N.ptr(xs), N.ptr(cot), N.ptr(sw), N.ptr(rw),
-                                float(clip) if clip is not None else 0.0, scale, N.ptr(scale_dev), S, B, N.ptr(flat),
-                                N.ptr(dbias1), N.ptr(scratch), N.stream_ptr(dev)))
+        N.check(L.lrds_mlp_grad(C.byref(mlp), N.ptr(bias1), N.ptr(xs), N.ptr(cot), N.ptr(sw), N.ptr(rw), clip, scale,
+                                N.ptr(scale_dev), S, B, N.ptr(flat), N.ptr(dbias1), N.ptr(scratch), N.stream_ptr(dev)))
     Cc, dp = N.CHANNELS, mlp.d_pad
     w_in_t, w_hid_t, b_hid, w_out_t, b_out = flat.split([d * Cc, nh * Cc * Cc, nh * Cc, Cc * dp, dp])
     grads = {base.input_embed.weight: w_in_t.view(d, Cc).t(),
@@ -148,12 +173,10 @@ def score_cot_sums(distr, xs: torch.Tensor, cot: torch.Tensor, clip, step_w=None
         N.check(n)
     out = torch.empty(S, d, device=dev, dtype=torch.float32)
     scratch = torch.empty(n, device=dev, dtype=torch.float32)
-    sw = None if step_w is None else step_w.detach().to(dev, torch.float32).contiguous()
-    rw = None if row_w is None else row_w.detach().to(dev, torch.float32).reshape(-1).contiguous()
+    sw, rw, clip = _weight_args(dev, step_w, row_w, clip)
     with torch.cuda.device(dev):
         N.check(L.lrds_score_cot_sums(C.byref(block), d, N.ptr(xs.contiguous()), N.ptr(cot.contiguous()), N.ptr(sw), N.ptr(rw),
-                                      float(clip) if clip is not None else 0.0, S, B, N.ptr(out), N.ptr(scratch),
-                                      N.stream_ptr(dev)))
+                                      clip, S, B, N.ptr(out), N.ptr(scratch), N.stream_ptr(dev)))
     return out
 
 
@@ -169,12 +192,8 @@ def control_param_grads(info: pack.CtrlInfo, params, taus, xs, cot, step_w, row_
     by_param = {}
     with torch.enable_grad():
         bias1 = time_embed_rows(base.timestep_embed, taus) + base.input_embed.bias
-    bound = cot.abs().max() if cot_max is None else torch.full((), float(cot_max), device=xs.device)  # device scalars:
-    if step_w is not None:                                                                            # no host round trip
-        bound = bound * step_w.abs().max()
-    if row_w is not None:
-        bound = bound * row_w.abs().max()
-    kernel_grads, dbias1 = mlp_grad(base, bias1, xs, cot, info.clip_model, step_w, row_w, cot_bound=bound)
+    kernel_grads, dbias1 = mlp_grad(base, bias1, xs, cot, info.clip_model, step_w, row_w,
+                                    cot_bound=cotangent_bound(cot, step_w, row_w, cot_max))
     by_param.update(kernel_grads)
     tp = [p for p in [*base.timestep_embed.parameters(), base.input_embed.bias] if p.requires_grad]
     if tp:
@@ -226,9 +245,14 @@ def normals(seed: int, particle_offset: int, K: int, B: int, d: int, device) -> 
     """The increments z [K, B, d] the production-mode rollout would draw in-kernel (lrds_normals, stream 0)."""
     z = torch.empty(K, B, d, device=device, dtype=torch.float32)
     with torch.cuda.device(device):
-        N.check(N.lib().lrds_normals(C.c_uint64(seed & (2 ** 64 - 1)), C.c_uint64(particle_offset), 0, K, B, d, N.ptr(z),
+        N.check(N.lib().lrds_normals(N.seed_arg(seed), C.c_uint64(particle_offset), 0, K, B, d, N.ptr(z),
                                      N.stream_ptr(device)))
     return z
+
+
+def _increments(seed: int, particle_offset: int, noise, K: int, B: int, d: int, device) -> torch.Tensor:
+    """The increments z [K, B, d] of a training rollout: the recorded ``noise``, else the generator's own (normals)."""
+    return normals(seed, particle_offset, K, B, d, device) if noise is None else noise.detach().to(device, torch.float32).contiguous()
 
 
 def lv_weights(rnd: torch.Tensor, mask: torch.Tensor, group=None):
@@ -259,11 +283,12 @@ def _loss_weights(loss_obj, rnd: torch.Tensor, x_T: torch.Tensor):
 
 
 def _param_grads(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, xs: torch.Tensor, cot: torch.Tensor, weights,
-                 max_rows: int, cot_max: float | None = None):
-    """Gradients (aligned with the control's trainable parameters) of  sum_{k,b} <c_kb, g(t_k, x_kb)>  over the K stored
-    states xs [K, B, d], with c = cot, or (step_w_k row_w_b) cot for ``weights`` = (step_w [K], row_w [B]): the
-    weight-gradient kernel (lrds_mlp_grad) where it is built, else autograd over ``control_rows`` in slices of
-    ``max_rows`` rows.  ``cot_max`` >= max |cot| when known (saves a reduction)."""
+                 max_rows: int, cot_max: float | None = None, scores: torch.Tensor | None = None):
+    """Gradients (aligned with the control's trainable parameters) of  sum_{k,b} <c_kb, g(t_k, x_kb)>  over the stored
+    states xs [K, B, d] at the plan's times, with c = cot, or (step_w_k row_w_b) cot for ``weights`` = (step_w [K],
+    row_w [B]): the weight-gradient kernel (lrds_mlp_grad) where it is built, else autograd over ``control_rows`` in
+    slices of ``max_rows`` rows.  ``cot_max`` >= max |cot| when known (saves a reduction); ``scores`` [K, B, d] = the
+    control's constant score at xs when the caller has it (control_score otherwise)."""
     dev = xs.device
     K, B, d = xs.shape
     params = [p for p in loss_obj.generative_ctrl.parameters() if p.requires_grad]
@@ -279,28 +304,21 @@ def _param_grads(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, xs: torch.Tenso
     step_rows = max(1, max_rows // B)
 
     def score_of(k0, k1):  # the constant score factor of the control at the stored states of steps k0 .. k1 - 1
-        flat = xs[k0:k1].reshape(-1, d)
-        score = info.target.score(flat).reshape(k1 - k0, B, d)
-        if info.kind == N.CTRL_LERP:  # clipped_interpolated_score, models/reparam.py:170-183
-            score = torch.lerp(info.prior.score(flat).reshape(k1 - k0, B, d), score, coef[k0:k1, N.STEP_LERP, None, None])
-        return score
+        if info.kind == N.CTRL_CLIPPED:
+            return None
+        return scores[k0:k1] if scores is not None else control_score(info, xs[k0:k1], coef[k0:k1])
 
-    use_kernel = mlp_grad_applicable(info.base) and plan.spec.precision == N.PRECISION_F16X3
-    if use_kernel:  # the backbone's gradient by lrds_mlp_grad: one launch over all K x B stored states
-        grads = control_param_grads(info, params, taus[:K], xs, cot, step_w, None if row_w is None else row_w.reshape(-1),
-                                    coef, score_of, max_rows, cot_max=cot_max)
-    for k0 in range(0, K if not use_kernel else 0, step_rows):
+    if mlp_grad_applicable(info.base) and plan.spec.precision == N.PRECISION_F16X3:
+        # the backbone's gradient by lrds_mlp_grad: one launch over all K x B stored states
+        return params, control_param_grads(info, params, taus[:K], xs, cot, step_w,
+                                           None if row_w is None else row_w.reshape(-1), coef, score_of, max_rows,
+                                           cot_max=cot_max)
+    for k0 in range(0, K, step_rows):
         k1 = min(K, k0 + step_rows)
-        xs_c = xs[k0:k1]
-        score = None
-        if info.kind != N.CTRL_CLIPPED:
-            score = info.target.score(xs_c.reshape(-1, d)).reshape(k1 - k0, B, d)
-            if info.kind == N.CTRL_LERP:  # clipped_interpolated_score, models/reparam.py:170-183
-                prior = info.prior.score(xs_c.reshape(-1, d)).reshape(k1 - k0, B, d)
-                score = torch.lerp(prior, score, coef[k0:k1, N.STEP_LERP, None, None])
+        score = score_of(k0, k1)
         c = cot[k0:k1] if weights is None else (step_w[k0:k1, None, None] * row_w.reshape(1, B, 1)) * cot[k0:k1]
         with torch.enable_grad():
-            surrogate = (c * control_rows(info, taus[k0:k1], xs_c, score, coef[k0:k1])).sum()
+            surrogate = (c * control_rows(info, taus[k0:k1], xs[k0:k1], score, coef[k0:k1])).sum()
         _accumulate(grads, params, surrogate)
     return params, grads
 
@@ -317,7 +335,7 @@ def lv_objective(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, x: torch.Tensor
     K = plan.noise_steps
     # without recorded increments the rollout draws its own (in-kernel Philox, no read of a [K, B, d] array); lrds_normals
     # reproduces exactly those for the cotangents below
-    z = normals(seed, particle_offset, K, B, d, dev) if noise is None else noise.detach().to(dev, torch.float32).contiguous()
+    z = _increments(seed, particle_offset, noise, K, B, d, dev)
     with torch.no_grad():
         x_T, rnd, xs = pack.run_rollout(plan, x, None if noise is None else z, seed, particle_offset, True)
     if group is not None:
@@ -354,7 +372,7 @@ def adjoint(plan: pack.Plan, xs: torch.Tensor, w: torch.Tensor, seed: int, noise
     rw = w.detach().to(dev, torch.float32).reshape(-1).contiguous()
     z = None if noise is None else noise.detach().to(dev, torch.float32).contiguous()
     with torch.cuda.device(dev):
-        N.check(N.lib().lrds_adjoint(C.byref(spec), N.ptr(xs.contiguous()), N.ptr(z), C.c_uint64(seed & (2 ** 64 - 1)),
+        N.check(N.lib().lrds_adjoint(C.byref(spec), N.ptr(xs.contiguous()), N.ptr(z), N.seed_arg(seed),
                                      C.c_uint64(particle_offset), N.ptr(rw), N.ptr(cot), N.stream_ptr(dev)))
     return cot
 
@@ -399,15 +417,10 @@ def cmcd_lv_objective(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, x: torch.T
     dev = x.device
     B, d = x.shape
     K = plan.noise_steps
-    z = normals(seed, particle_offset, K, B, d, dev) if noise is None else noise.detach().to(dev, torch.float32).contiguous()
+    z = _increments(seed, particle_offset, noise, K, B, d, dev)
     with torch.no_grad():
         x_T, rnd, xs = pack.run_rollout(plan, x, z, seed, particle_offset, True)
-    rnd_leaf = rnd.detach().clone().requires_grad_(True)
-    with torch.enable_grad():
-        value, metrics = loss_obj.compute_loss(rnd_leaf, samples=x_T)
-        (w,) = torch.autograd.grad(value, rnd_leaf)
-    params = [p for p in loss_obj.generative_ctrl.parameters() if p.requires_grad]
-    grads: list = [None] * len(params)
+    value, w, metrics = _loss_weights(loss_obj, rnd, x_T)
     sde = loss_obj.sde
     ts = pack.on_device(plan, "taus", dev)      # [K + 1]
     dt = pack.on_device(plan, "dt", dev, lambda: plan.taus[1:] - plan.taus[:-1])
@@ -433,12 +446,6 @@ def cmcd_lv_objective(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, x: torch.T
         cot[:-1] += db
         cot[1:] -= cost * dt[:, None, None] + db
         cot *= w[None, :, :]
-    use_kernel = mlp_grad_applicable(info.base) and plan.spec.precision == N.PRECISION_F16X3
-    if use_kernel:  # pass 2 by lrds_mlp_grad: one launch over the (K + 1) x B stored states
-        grads = control_param_grads(info, params, ts, xs, cot, None, None, None, lambda j0, j1: tscore[j0:j1], max_rows)
-    for j0 in range(0, K + 1 if not use_kernel else 0, rows):  # pass 2 (shapes the kernel is not built for): autograd
-        j1 = min(K + 1, j0 + rows)
-        with torch.enable_grad():
-            g = control_rows(info, ts[j0:j1], xs[j0:j1], tscore[j0:j1] if info.kind != N.CTRL_CLIPPED else None)
-            _accumulate(grads, params, (cot[j0:j1] * g).sum())
+    # pass 2: the parameter pass of the linear objectives over the K + 1 stored states (ScoreCtrl: the target scores of pass 1)
+    params, grads = _param_grads(loss_obj, plan, info, xs, cot, None, max_rows, scores=tscore)
     return _InjectGrads.apply(value.detach(), grads, *params), metrics
