@@ -17,7 +17,7 @@
 extern "C" {
 #endif
 
-#define LRDS_ABI_VERSION 10 /* 10: lrds_adjoint; 9: lrds_gmm.layout (full-covariance Gaussian / mixture references) */
+#define LRDS_ABI_VERSION 11 /* 11: lrds_adjoint_cmcd; 10: lrds_adjoint; 9: lrds_gmm.layout (full-covariance Gaussian / mixture references) */
 #define LRDS_CHANNELS 64 /* FourierMLP / TimeEmbed width, conf/model/base/fouriermlp.yaml:4 */
 #define LRDS_MAX_DIM_PAD 1024 /* largest d_pad the operand packers accept */
 
@@ -267,6 +267,33 @@ int lrds_rollout(const lrds_spec* spec, const float* x0, const float* noise, uin
  * non-finite cotangent.  Every other accepted spec recomputes the network with fp32 FFMA and never touches [0]. */
 int lrds_adjoint(const lrds_spec* spec, const float* traj, const float* noise, uint64_t seed, uint64_t particle_offset,
                  const float* row_w, float* cot_out, void* stream);
+
+/* ---- the pathwise (method 'kl' / 'kl_ito') gradient of the CMCD simulate loop (ControlledLangevinSDELoss.simulate,
+ * oc.py:666-755, in its training form: rnd starts at 0, oc.py:695-696; the Ito term is always there, so 'kl_ito' = 'kl').
+ * Every trajectory point x_j (j = 0..K) carries the control u_j = clip(net(t_j, x_j)) and the tempered drift
+ * D_j = clip(sig^2/2 (f_j grad log pi(x_j) + (1 - f_j) grad log p_0(x_j)), cmcd_clip), sig = cmcd_diff, f_j = LRDS_STEP_FRAC of
+ * row j, p_0 = ref_0.  With c_k = (D_k + D_{k+1}) / sig + u_k - u_{k+1} and e_k = w_b (c_k dt_k + sqrt(dt_k) z_k):
+ *   ubar_j   = [j<K] (e_j + sig dt_j lambda_{j+1}) - [j>=1] e_{j-1}                              = d loss / d u_j
+ *   Dbar_j   = [j<K] (e_j / sig + dt_j lambda_{j+1}) + [j>=1] e_{j-1} / sig
+ *   lambda_j = [j<K] lambda_{j+1} + J_net^T ([|net_j| <= clip_model] ubar_j)
+ *              + sig^2/2 (f_j H_pi(x_j) + (1 - f_j) H_0) ([|D_j before the clip| <= cmcd_clip] Dbar_j)
+ *              + [j=K] (-w_b [|log pi(x_K)| <= clip_target] grad log pi(x_K))
+ * with H_pi the Hessian of log pi (exact for the diagonal mixture; the lattice stencil for PhiFour) and H_0 = -diag(1/var_0).
+ * d loss / d theta = sum_j <ubar_j, d u_j / d theta> over the K + 1 points: lrds_mlp_grad with cot = ubar.
+ *   traj    [K+1][B][d] the trajectory lrds_rollout wrote for this spec
+ *   noise   [K][B][d] the increments that rollout consumed, or NULL: the kernel regenerates the production-mode Philox
+ *           increments of (seed, particle_offset)
+ *   row_w   [B] w_b = d loss / d rnd_b
+ *   cot_out [K+1][B][d] ubar_j (written without atomics: deterministic)
+ * Built for the LRDS_ROLLOUT_CMCD kind, LRDS_CTRL_CLIPPED, a diagonal Gaussian prior in ref_0, diagonal mixture (M >= 1)
+ * and PhiFour targets, and the precisions F16X3 / TF32X3 / FP32_SIMT; LRDS_ERR_UNSUPPORTED for the other controls, the
+ * logistic-regression target, full-covariance blocks, BF16 / TF32 and every other kind.  F16X3 inside lrds_mlp_grad's
+ * envelope (d <= 64, num_hidden <= 2; mlp.tc_image = the F16X3 image), when its shared-memory columns fit, runs the network
+ * on tcgen05 with the rollout's weight image and adds to spec.status[0] like lrds_adjoint; every other accepted spec
+ * recomputes the network with fp32 FFMA and never touches [0].  Both add to [1] the particles with a non-finite
+ * cotangent. */
+int lrds_adjoint_cmcd(const lrds_spec* spec, const float* traj, const float* noise, uint64_t seed, uint64_t particle_offset,
+                      const float* row_w, float* cot_out, void* stream);
 
 /* ---- tensor-core weight image: the FourierMLP weights in the shared-memory operand layout of tcgen05.mma (plus
  * the fp32 biases), staged once per CTA by a bulk TMA copy.  `image_out` (device, 16-byte aligned) must hold

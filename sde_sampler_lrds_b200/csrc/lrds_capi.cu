@@ -9,6 +9,7 @@
 #include <cstring>
 
 #include "lrds_adjoint.cuh"
+#include "lrds_adjoint_cmcd.cuh"
 #include "lrds_internal.h"
 #include "lrds_rollout_simt.cuh"
 
@@ -146,6 +147,11 @@ int validate_spec(const lrds_spec* s, bool need_steps) {
 __global__ void __launch_bounds__(128) adjoint_simt_kernel(const lrds::AdjointArgs a) {
   extern __shared__ __align__(16) float smem[];
   lrds::adjoint_body(a, smem);
+}
+// the fp32 adjoint of the CMCD loop (lrds_adjoint_cmcd.cuh)
+__global__ void __launch_bounds__(128) adjoint_cmcd_simt_kernel(const lrds::AdjointArgs a) {
+  extern __shared__ __align__(16) float smem[];
+  lrds::adjoint_cmcd_body(a, smem);
 }
 
 // ---- estimator partials -----------------------------------------------------------------------------
@@ -822,7 +828,7 @@ int lrds_adjoint(const lrds_spec* spec, const float* traj, const float* noise, u
   if (s.K < 1) return fail(LRDS_ERR_INVALID, "adjoint: K must be >= 1");
   if (s.kind != LRDS_ROLLOUT_LINEAR)
     return fail(LRDS_ERR_UNSUPPORTED, "adjoint: built for the LINEAR simulate loop (CMCD evaluates the control at both ends of a "
-                                      "step and the EUBO kinds are not trained through it)");
+                                      "step: lrds_adjoint_cmcd; the EUBO kinds are not trained through it)");
   if (s.ctrl_kind != LRDS_CTRL_CLIPPED)
     return fail(LRDS_ERR_UNSUPPORTED, "adjoint: built for ClippedCtrl; the score-family controls also need the target's "
                                       "Hessian-vector product");
@@ -846,6 +852,42 @@ int lrds_adjoint(const lrds_spec* spec, const float* traj, const float* noise, u
   ColExtra cols;
   cols.layout = lrds::adj_layout(s).total;
   return launch_cols(adjoint_simt_kernel, "adjoint", s, cols, (cudaStream_t)stream, a);
+}
+
+int lrds_adjoint_cmcd(const lrds_spec* spec, const float* traj, const float* noise, uint64_t seed, uint64_t particle_offset,
+                      const float* row_w, float* cot_out, void* stream) {
+  if (int r = validate_spec(spec, true)) return r;
+  if (!traj || !row_w || !cot_out) return fail(LRDS_ERR_INVALID, "adjoint_cmcd: traj, row_w and cot_out are required");
+  const lrds_spec& s = *spec;
+  if (s.K < 1) return fail(LRDS_ERR_INVALID, "adjoint_cmcd: K must be >= 1");
+  if (s.kind != LRDS_ROLLOUT_CMCD)
+    return fail(LRDS_ERR_UNSUPPORTED, "adjoint_cmcd: built for the CMCD simulate loop (LINEAR: lrds_adjoint; the EUBO kinds are "
+                                      "not trained through it)");
+  if (s.ctrl_kind != LRDS_CTRL_CLIPPED)
+    return fail(LRDS_ERR_UNSUPPORTED, "adjoint_cmcd: built for ClippedCtrl; the score-family controls also need the Hessian-vector "
+                                      "product inside the control");
+  if (s.precision == LRDS_PRECISION_BF16 || s.precision == LRDS_PRECISION_TF32)
+    return fail(LRDS_ERR_UNSUPPORTED, "adjoint_cmcd: the reduced-precision network moved the particles, the adjoint would "
+                                      "linearise a different one (use f16x3, tf32x3 or fp32)");
+  if (s.precision != LRDS_PRECISION_FP32_SIMT && s.precision != LRDS_PRECISION_TF32X3 && s.precision != LRDS_PRECISION_F16X3)
+    return fail(LRDS_ERR_INVALID, "adjoint_cmcd: unknown precision");
+  if (s.target.kind == LRDS_DISTR_NONE) return fail(LRDS_ERR_INVALID, "adjoint_cmcd: CMCD needs a target");
+  if (s.target.kind != LRDS_DISTR_GMM && s.target.kind != LRDS_DISTR_PHI4)
+    return fail(LRDS_ERR_UNSUPPORTED, "adjoint_cmcd: built for mixture and PhiFour targets (the logistic-regression target has "
+                                      "no Hessian-vector product here)");
+  if (int r = validate_gmm(s.ref_0, "ref_0")) return r;
+  if (s.ref_0.layout == LRDS_GMM_FULL || s.ref_0.M != 1)
+    return fail(LRDS_ERR_UNSUPPORTED, "adjoint_cmcd: built for a diagonal Gaussian prior in ref_0 (full-covariance priors are not)");
+  const lrds::AdjointArgs a{lrds::RolloutArgs{s, nullptr, noise, seed, particle_offset, nullptr, nullptr, nullptr}, traj, row_w,
+                            cot_out};
+  if (lrds::adjoint_cmcd_tc_applicable(s)) {
+    const int r = lrds::launch_adjoint_cmcd_tc(a, (cudaStream_t)stream);
+    if (r == LRDS_OK) g_launches.fetch_add(1);
+    return r;
+  }
+  ColExtra cols;
+  cols.layout = lrds::adj_cmcd_layout(s).total;
+  return launch_cols(adjoint_cmcd_simt_kernel, "adjoint_cmcd", s, cols, (cudaStream_t)stream, a);
 }
 
 int64_t lrds_tc_image_bytes(int32_t d, int32_t num_hidden, int32_t precision) {

@@ -25,6 +25,9 @@ int pack_tc_image(const lrds_mlp& w, int precision, void* image, cudaStream_t st
 // lrds_adjoint_tc.cu: the tcgen05 adjoint (F16X3 inside lrds_mlp_grad's envelope, when its shared memory fits)
 bool adjoint_tc_applicable(const lrds_spec& s);
 int launch_adjoint_tc(const AdjointArgs& a, cudaStream_t st);
+// lrds_adjoint_cmcd_tc.cu: the tcgen05 adjoint of the CMCD loop (same envelope)
+bool adjoint_cmcd_tc_applicable(const lrds_spec& s);
+int launch_adjoint_cmcd_tc(const AdjointArgs& a, cudaStream_t st);
 // lrds_mlp_grad.cu
 bool mlp_grad_applicable(int d, int num_hidden);
 int mlp_grad_params(int d, int num_hidden);

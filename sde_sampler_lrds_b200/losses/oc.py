@@ -16,7 +16,7 @@ counter-based generator (global particle index => results independent of the GPU
 Training: ``loss(ts, x, ...)`` with method 'lv' / 'lv_traj' returns a scalar whose ``backward()`` fills the control's
 parameter gradients (train.py: fused rollout + one batched gradient pass), for every loss class below; 'kl' / 'kl_ito'
 (pathwise gradient through the trajectory: fused rollout + the reverse-time adjoint kernel + the same parameter pass) for
-the linear losses with a ClippedCtrl drift.
+the linear losses and CMCD with a ClippedCtrl drift.
 """
 from __future__ import annotations
 
@@ -166,9 +166,7 @@ class BaseOCLoss:
                                       particle_offset=particle_offset, group=group)
         if group is not None:
             raise NotImplementedError("sharded training is built for method 'lv'")
-        if info.kind != N.CTRL_CLIPPED:
-            raise NotImplementedError("method 'kl' / 'kl_ito' is built for ClippedCtrl (base_zero_init): the adjoint of the "
-                                      "score-family controls also needs each target's Hessian-vector product (not built)")
+        _kl_ctrl_check(info)
         if getattr(self, "_init_cost", False):
             raise NotImplementedError("the discrete-time DIS loss has no 'kl' training rollout here (no shipped config uses it)")
         rnd_start = None if initial_log_prob is None else _kl_start(initial_log_prob, x)
@@ -289,6 +287,13 @@ def _terminal(spec, keep, device, terminal_unnorm_log_prob, info):
     spec.target = distr
     keep.append(k)
     spec.clip_target = float(clip_t) if clip_t is not None else 0.0
+
+
+def _kl_ctrl_check(info):
+    """'kl' / 'kl_ito' train ClippedCtrl drifts only."""
+    if info.kind != N.CTRL_CLIPPED:
+        raise NotImplementedError("method 'kl' / 'kl_ito' is built for ClippedCtrl (base_zero_init): the adjoint of the "
+                                  "score-family controls also needs each target's Hessian-vector product (not built)")
 
 
 def _kl_start(initial_log_prob, x):
@@ -619,25 +624,31 @@ class ControlledLangevinSDELoss(BaseOCLoss):
 
     def __call__(self, ts, x, terminal_unnorm_log_prob, initial_log_prob=None, noise=None, seed=None,
                  particle_offset: int = 0):
-        """[TRAINING] (loss, metrics) of oc.py:830-860 for method 'lv' / 'lv_traj' (train.cmcd_lv_objective)."""
+        """[TRAINING] (loss, metrics) of oc.py:830-860: method 'lv' / 'lv_traj' (train.cmcd_lv_objective), or 'kl' /
+        'kl_ito' for a ClippedCtrl drift (train.cmcd_kl_objective: the pathwise gradient through the trajectory; the Ito
+        term is always part of the CMCD log-weight, so the two are the same objective)."""
         from .. import train
-        if self.method not in ("lv", "lv_traj"):
-            raise NotImplementedError("method 'kl' differentiates through the trajectory: not built (SURVEY.md 8f item 1)")
         x = self._train_batch(x)
         info = self._ctrl(False)
         if info.kind not in (N.CTRL_CLIPPED, N.CTRL_SCORE):
             raise NotImplementedError("CMCD trains ClippedCtrl / ScoreCtrl drift models")
+        if self.method in ("kl", "kl_ito"):
+            _kl_ctrl_check(info)
         plan = self._plan(ts, x.device, False, terminal_unnorm_log_prob, initial_log_prob, eubo=False)
+        if self.method in ("kl", "kl_ito"):
+            return train.cmcd_kl_objective(self, plan, info, x, self._seed(seed), _kl_start(initial_log_prob, x), noise=noise,
+                                           particle_offset=particle_offset)
         return train.cmcd_lv_objective(self, plan, info, x, self._seed(seed), noise=noise, particle_offset=particle_offset)
 
     def simulate(self, ts, x, terminal_unnorm_log_prob, initial_log_prob=None, train: bool = True,
                  change_sde_ctrl: bool = False, return_traj: bool = False, use_ema: bool = False, noise=None,
                  seed=None, particle_offset: int = 0):
         self._check_plain(change_sde_ctrl)
-        if train and self.method in ["kl", "kl_ito"]:
-            raise NotImplementedError("the training variant (rnd starts at 0, oc.py:695-696) is part of SURVEY.md 8f item 1")
         plan = self._plan(ts, x.device, use_ema, terminal_unnorm_log_prob, initial_log_prob, eubo=False)
-        return pack.run_rollout(plan, x, noise, self._seed(seed), particle_offset, return_traj)
+        x_T, rnd, xs = pack.run_rollout(plan, x, noise, self._seed(seed), particle_offset, return_traj)
+        if train and self.method in ["kl", "kl_ito"]:  # the training form starts the log-weight at 0 (oc.py:695-696)
+            rnd = rnd - _kl_start(initial_log_prob, x).reshape(rnd.shape)
+        return x_T, rnd, xs
 
     def compute_eubo(self, ts, x, terminal_unnorm_log_prob, initial_log_prob=None, use_ema: bool = False, noise=None,
                      seed=None, particle_offset: int = 0):

@@ -25,7 +25,9 @@ by autograd through K sequential steps (~40-150 eager ops each).  Here
 
 With method 'kl' / 'kl_ito' (kl_objective, ClippedCtrl) the SDE follows the non-detached control and the gradient runs
 through the trajectory: step 3 takes the cotangents d loss / d g_k that the reverse-time adjoint kernel lrds_adjoint
-computes from the stored trajectory (csrc/lrds_adjoint.cuh); everything else is shared with the LV objective.
+computes from the stored trajectory (csrc/lrds_adjoint.cuh); everything else is shared with the LV objective.  CMCD
+(cmcd_kl_objective) does the same with lrds_adjoint_cmcd (csrc/lrds_adjoint_cmcd.cuh), whose cotangents cover the K + 1
+trajectory points and whose recursion also runs through the Hessian of the target in the tempered Langevin drift.
 
 Nothing here runs on the CPU or imports the oracle.
 """
@@ -448,4 +450,40 @@ def cmcd_lv_objective(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, x: torch.T
         cot *= w[None, :, :]
     # pass 2: the parameter pass of the linear objectives over the K + 1 stored states (ScoreCtrl: the target scores of pass 1)
     params, grads = _param_grads(loss_obj, plan, info, xs, cot, None, max_rows, scores=tscore)
+    return _InjectGrads.apply(value.detach(), grads, *params), metrics
+
+
+def adjoint_cmcd(plan: pack.Plan, xs: torch.Tensor, w: torch.Tensor, seed: int, noise=None, particle_offset: int = 0):
+    """ubar [K + 1, B, d] = d loss / d u_j of the pathwise CMCD gradient by the reverse-time kernel lrds_adjoint_cmcd:
+    ``xs`` [K + 1, B, d] = the trajectory the CMCD rollout of ``plan`` wrote, ``w`` [B] = d loss / d rnd_b, ``noise`` =
+    the increments that rollout consumed (None: the kernel regenerates the in-kernel Philox draws of ``seed``)."""
+    dev = xs.device
+    K1, B, d = xs.shape
+    spec = N.Spec.from_buffer_copy(plan.spec)  # the cached plan is shared: never mutated here
+    spec.B = B
+    spec.status = pack.status_counters(dev).data_ptr()
+    cot = torch.empty(K1, B, d, device=dev, dtype=torch.float32)
+    rw = w.detach().to(dev, torch.float32).reshape(-1).contiguous()
+    z = None if noise is None else noise.detach().to(dev, torch.float32).contiguous()
+    with torch.cuda.device(dev):
+        N.check(N.lib().lrds_adjoint_cmcd(C.byref(spec), N.ptr(xs.contiguous()), N.ptr(z), N.seed_arg(seed),
+                                          C.c_uint64(particle_offset), N.ptr(rw), N.ptr(cot), N.stream_ptr(dev)))
+    return cot
+
+
+def cmcd_kl_objective(loss_obj, plan: pack.Plan, info: pack.CtrlInfo, x: torch.Tensor, seed: int, rnd_start: torch.Tensor,
+                      noise=None, particle_offset: int = 0, max_rows: int = 1 << 20):
+    """(loss, metrics) of ControlledLangevinSDELoss with method 'kl' / 'kl_ito' (ClippedCtrl; the SDE follows the
+    non-detached control, loss = mean(rnd[mask])): the fused rollout with its trajectory, its log-weights in the training
+    form (``rnd_start`` [B] = log p_prior(x_0) subtracted: that form starts at 0, oc.py:695-696), d loss / d rnd from
+    compute_loss, the reverse-time adjoint (lrds_adjoint_cmcd) for ubar_j = d loss / d u_j at the K + 1 points, and the
+    parameter pass of the other objectives with cot = ubar.  With ``noise`` None the rollout draws its increments in the
+    kernel and the adjoint regenerates them."""
+    noise = None if noise is None else noise.detach().to(x.device, torch.float32).contiguous()
+    with torch.no_grad():
+        x_T, rnd, xs = pack.run_rollout(plan, x, noise, seed, particle_offset, True)
+        rnd = rnd - rnd_start.reshape(rnd.shape)
+    value, w, metrics = _loss_weights(loss_obj, rnd, x_T)
+    cot = adjoint_cmcd(plan, xs, w, seed, noise, particle_offset)
+    params, grads = _param_grads(loss_obj, plan, info, xs, cot, None, max_rows)
     return _InjectGrads.apply(value.detach(), grads, *params), metrics
